@@ -8,6 +8,8 @@ One "step" = one sweep through the whole per-frame chain (MAIN.cpp:143-144, 186-
   python bench.py [--gpus N] [--steps K] [--warmup W]          this repo's CUDA path
   python bench.py --impl reference [...]                       the CPU restatement of the reference
                                                                (oracle/, KD-tree mode) on the host cores
+  python bench.py [...] --dump-outputs DIR                     also write what the last timed sweep computed
+                                                               as DIR/<name>.npy (see dump_outputs)
 
 The K-step window is measured R times (--repeats, default min(25, 700 // K)), every window on a fresh context
 with the same W + 1 warm-up sweeps, with a barrier + synchronize on both sides; `value` / `e2e` are the medians
@@ -442,6 +444,25 @@ def _stats(x):
     return {"median": float(np.median(x)), "min": float(x.min()), "max": float(x.max()), "windows": int(len(x))}
 
 
+DUMP_MAX_MAP_POINTS = 1_900_000  # per map: two maps of float32[n, 4] stay under 64 MB with the pose and the cube counts
+
+
+def dump_outputs(out_dir, pose, maps):
+    """What a caller of the timed path receives for the last timed sweep, as out_dir/<name>.npy: the pose
+    process_frame returned (float64[14]: odometry q, t, mapped q, t) and the corner / surf maps after that
+    sweep (`lm.*Map` blobs split into the per-cube point counts, float64[4851], and the points, float32[n, 4]).
+    A map of more than DUMP_MAX_MAP_POINTS points is written as a fixed seeded sample of its rows, in order."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pose.npy"), np.asarray(pose, np.float64))
+    for name, blob in zip(("corner_map", "surf_map"), maps):
+        counts = np.frombuffer(blob[:4851 * 4], np.int32)
+        pts = np.frombuffer(blob[4851 * 4:], np.float32).reshape(-1, 4)
+        if len(pts) > DUMP_MAX_MAP_POINTS:
+            pts = pts[np.sort(np.random.default_rng(0).choice(len(pts), DUMP_MAX_MAP_POINTS, replace=False))]
+        np.save(os.path.join(out_dir, name + "_counts.npy"), counts.astype(np.float64))
+        np.save(os.path.join(out_dir, name + "_points.npy"), pts)
+
+
 def run_ours(args, rank, world_size, local_rank):
     import torch
     pkg = importlib.import_module("vloam-noted_b200")
@@ -482,7 +503,7 @@ def run_ours(args, rank, world_size, local_rank):
     # Every window: fresh context, W + 1 warm-up sweeps, barrier + synchronize, K timed sweeps, synchronize.
     dev_ms, e2e_ms, launches, lat = [], [], [], []
     poses = np.zeros((K, 14))
-    last_ctx = None
+    last_ctx = last_maps = None
     for r in range(R):
         ctx = fresh()
         ext = torch.cuda.ExternalStream(ctx.stream, device=local_rank)
@@ -527,6 +548,8 @@ def run_ours(args, rank, world_size, local_rank):
         ctx.synchronize()  # like the device-timed leg: the last sweep's map update belongs to the window
         e2e_ms.append((time.perf_counter() - t0) * 1e3)
         sampler.active = False
+        if args.dump_outputs and rank == 0 and r == R - 1:
+            last_maps = (ctx.get("lm.cornerMap"), ctx.get("lm.surfMap"))
         ctx.close()
     clocks = sampler.stop() if rank == 0 else None
     h2d = float(np.mean([s.shape[0] * 16 for s in scans[first:first + K]]))
@@ -631,6 +654,8 @@ def run_ours(args, rank, world_size, local_rank):
     if ktable: line["kernels"] = ktable
     if cpu: line["cpu_baseline"] = cpu
     if parity: line["parity"] = parity
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, poses[-1], last_maps)
     print(json.dumps(line), flush=True)
     if dist: dist.destroy_process_group()
 
@@ -717,7 +742,7 @@ def run_c5(args, rank, world_size, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed sweeps per window (see --repeats)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--repeats", type=int, default=0, help="timed windows of --steps sweeps each (0 = min(25, 700 // steps), at least 3)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
@@ -729,7 +754,13 @@ def main():
     ap.add_argument("--no-pin", action="store_true", help="do not pin this rank's threads to its slice of the host cores (N > 1)")
     ap.add_argument("--workload", default="c3", choices=["c3", "c5"], help="c3: the headline (default); c5: 8 sequences batched across the GPUs")
     ap.add_argument("--frames", type=int, default=110, help="sweeps per sequence for --workload c5")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the pose of the last timed sweep and the maps after it as DIR/<name>.npy "
+                    "(last end-to-end window, rank 0); the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c3"):
+        ap.error("--dump-outputs writes the outputs of the c3 workload of this repo's CUDA path")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
