@@ -28,6 +28,10 @@
  * and inside every getter.  A frame on which mapping is skipped
  * (mapping_skip_frame > 1) with NULL output pointers returns without S2; the
  * device-side ordering between frames never depends on those host waits.
+ * vloam_b200_publish_map() queues the assembly of the global map on a stream of
+ * its own, behind the last map update, and returns; the next sweeps' map edits
+ * wait for it on the device, so publishing neither blocks the caller nor
+ * changes any result.  vloam_b200_get_map() is the only call that waits for it.
  * vloam_b200_synchronize() drains everything, including the helper thread.
  */
 #ifndef VLOAM_B200_H_
@@ -132,6 +136,16 @@ int vloam_b200_laser_mapping(vloam_b200_ctx* c, double* q_w_curr, double* t_w_cu
  * to query the size).  Returns the number of points or a negative error. */
 int vloam_b200_register_full_cloud(vloam_b200_ctx* c, float* out_xyzi, int cap_points);
 
+/* LaserMapping::publish, LM.cpp:884-899: queue the assembly of laserCloudMap (all 4851 cubes, corner then surf per cube)
+ * from the map as of the last mapped frame.  Returns at once; the device orders every later map edit behind it.  (A call
+ * that has to grow the context's publication buffers -- the first one, or when the map outgrew them -- first waits for the
+ * previous publication.) */
+int vloam_b200_publish_map(vloam_b200_ctx* c);
+/* Wait for the last publish_map and copy its cloud to host memory (out NULL: size query).  Returns the number of points,
+ * VLOAM_E_CAPACITY when cap_points is too small, VLOAM_E_INVALID when nothing was published since create.  A second
+ * publish_map before get_map replaces the first. */
+int vloam_b200_get_map(vloam_b200_ctx* c, float* out_xyzi, int cap_points);
+
 /* MAIN.cpp:143-144, 186-190 in one call: begin_frame, scan_registration,
  * laser_odometry, laser_mapping.  pose_out (may be NULL): 14 doubles
  * {odom q[4], odom t[3], mapped q[4], mapped t[3]}.  On a mapped frame the call
@@ -168,7 +182,8 @@ int vloam_b200_profile_timeline(vloam_b200_ctx* c, char* buf, int cap);
  * sr.label sr.scanStartInd sr.scanEndInd lo.cornerLast lo.surfLast lo.pose
  * lo.assoc.corner{0,1} lo.assoc.surf{0,1} lm.pose lm.state lm.cornerStack
  * lm.surfStack lm.cornerFromMap lm.surfFromMap lm.validInd lm.cornerMap
- * lm.surfMap lm.knn.{cidx,sidx,cd2,sd2,cok,sok}{0,1} lm.costs lo.costs;
+ * lm.surfMap lm.knn.{cidx,sidx,cd2,sd2,cok,sok}{0,1} lm.costs lo.costs
+ * lm.paths (int64 {in-place, pool-path} mapped sweeps since create);
  * set: lo.last lo.pose lm.pose lm.state lm.cornerMap lm.surfMap. */
 long vloam_b200_debug_get(vloam_b200_ctx* c, const char* name, void* out, long cap_bytes);
 int vloam_b200_debug_set(vloam_b200_ctx* c, const char* name, const void* data, long bytes);

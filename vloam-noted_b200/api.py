@@ -16,6 +16,7 @@ EXPORTS = [
     "vloam_b200_laser_mapping", "vloam_b200_process_frame", "vloam_b200_process_frame_device", "vloam_b200_synchronize",
     "vloam_b200_stream", "vloam_b200_kernel_launches", "vloam_b200_set_timing", "vloam_b200_stage_ms", "vloam_b200_debug_get",
     "vloam_b200_debug_set", "vloam_b200_profile_kernel", "vloam_b200_profile_result", "vloam_b200_profile_table", "vloam_b200_profile_timeline", "vloam_b200_register_full_cloud", "vloam_b200_lo_associate", "vloam_b200_voxel_grid", "vloam_b200_evaluate", "vloam_b200_solve", "vloam_b200_fit", "vloam_b200_evaluate_deskew", "vloam_b200_solve_deskew", "vloam_b200_exact_math",
+    "vloam_b200_publish_map", "vloam_b200_get_map",
 ]
 
 
@@ -77,6 +78,8 @@ def load_lib(build=False):
     L.vloam_b200_register_full_cloud.argtypes = [vp, vp, ci]
     L.vloam_b200_fit.argtypes = [vp, vp, ci, ci, vp, vp]
     L.vloam_b200_exact_math.argtypes = [vp, vp, vp, ci, vp, vp]
+    L.vloam_b200_publish_map.argtypes = [vp]
+    L.vloam_b200_get_map.argtypes = [vp, vp, ci]
     _lib = L
     return L
 
@@ -86,7 +89,7 @@ def _decode(name, raw):
         return raw
     dt = {"sr.curvature": np.float32, "sr.label": np.int32, "sr.scanStartInd": np.int32, "sr.scanEndInd": np.int32,
           "lo.pose": np.float64, "lm.pose": np.float64, "lm.state": np.int32, "lm.validInd": np.int32,
-          "lo.costs": np.float64, "lm.costs": np.float64, "alloc.count": np.int64}
+          "lo.costs": np.float64, "lm.costs": np.float64, "alloc.count": np.int64, "lm.paths": np.int64}
     if name in dt:
         return np.frombuffer(raw, dt[name]).copy()
     if name.startswith("lo.assoc.corner"):
@@ -160,6 +163,18 @@ class Context:
         if n:
             self._chk(self.L.vloam_b200_register_full_cloud(self.h, out.ctypes.data, n))
         return out
+
+    def publish_map(self):
+        """LaserMapping::publish's laserCloudMap (LM.cpp:884-899): queue its assembly from the map of the last mapped frame."""
+        self._chk(self.L.vloam_b200_publish_map(self.h))
+
+    def get_map(self):
+        """The cloud of the last publish_map: float32[n, 4], for each of the 4851 cubes its corner then its surf points."""
+        n = self._chk(self.L.vloam_b200_get_map(self.h, None, 0))
+        out = np.empty((n, 4), np.float32)
+        if n:
+            n = self._chk(self.L.vloam_b200_get_map(self.h, out.ctypes.data, n))
+        return out[:n]
 
     def laser_odometry(self, prior_q=None, prior_t=None, want_pose=True):
         qw, tw, ql, tl = np.zeros(4), np.zeros(3), np.zeros(4), np.zeros(3)
@@ -327,8 +342,12 @@ class LaserOdometry:
 class LaserMapping:
     """vloam::LaserMapping (laser_mapping.h:72-100)."""
 
-    def __init__(self, ctx):
+    def __init__(self, ctx, map_pub_number=20):
         self.ctx, self.pose = ctx, None
+        self.map_pub_number = map_pub_number  # ROS parameter map_pub_number (LM.cpp:44-45)
+        self.frameCount = 0                   # mapped frames (incremented at the end of solveMapping)
+        self.skip_frame = False               # input(): the odometry skipped mapping on this frame (LM.cpp:197-201)
+        self._published_at = 0
 
     def init(self):
         pass
@@ -336,18 +355,37 @@ class LaserMapping:
     def reset(self):
         pass
 
+    def input(self, skip_frame):
+        self.skip_frame = bool(skip_frame)
+
     def solveMapping(self):
+        """On a skipped frame this only propagates the high-frequency pose (the reference does not call solveMapping then), so the
+        mapped-frame count is left alone, as in vloam_adapter.hpp."""
         self.pose = self.ctx.laser_mapping()
+        if not self.skip_frame:
+            self.frameCount += 1
+
+    def publish(self):
+        """LM.cpp:884-899: every map_pub_number mapped frames the global map is published (parity unpinned: the reference is
+        not in this checkout); the rule of vloam_adapter.hpp's LaserMapping::publish: nothing before the first mapped frame, and
+        a map already published is not queued again on the skipped frames after it.  Returns True when a publication was queued;
+        Context.get_map() reads it."""
+        n = self.frameCount
+        if self.map_pub_number > 0 and n > 0 and n % self.map_pub_number == 0 and n != self._published_at:
+            self.ctx.publish_map()
+            self._published_at = n
+            return True
+        return False
 
 
 class LidarOdometryMapping:
     """vloam::LidarOdometryMapping (lidar_odometry_mapping.h:45-86): the per-frame call sequence."""
 
-    def __init__(self, **params):
+    def __init__(self, map_pub_number=20, **params):
         self.ctx = Context(**params)
         self.scan_registration = ScanRegistration(self.ctx)
         self.laser_odometry = LaserOdometry(self.ctx)
-        self.laser_mapping = LaserMapping(self.ctx)
+        self.laser_mapping = LaserMapping(self.ctx, map_pub_number)
 
     def init(self):
         pass
@@ -362,4 +400,7 @@ class LidarOdometryMapping:
         self.laser_odometry.solveLO()
 
     def laserMappingIO(self):  # lidar_odometry_mapping.cpp:144-176
+        last = self.laser_odometry.last
+        self.laser_mapping.input(last["skip_frame"] if last else False)
         self.laser_mapping.solveMapping()
+        self.laser_mapping.publish()

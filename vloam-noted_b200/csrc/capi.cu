@@ -451,7 +451,18 @@ int vloam_b200_synchronize(vloam_b200_ctx* c) {
   VL_CUDA(cudaStreamSynchronize(c->streamAux));
   VL_CUDA(cudaStreamSynchronize(c->stream)); VL_CUDA(cudaStreamSynchronize(c->stream2)); VL_CUDA(cudaStreamSynchronize(c->stream3));
   VL_CUDA(cudaStreamSynchronize(c->stream4));
+  VL_TRY(vl_lm_pub_sync(c));
   return VLOAM_OK;
+}
+
+int vloam_b200_publish_map(vloam_b200_ctx* c) {
+  if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
+  return vl_lm_publish_map(c);
+}
+int vloam_b200_get_map(vloam_b200_ctx* c, float* out_xyzi, int cap_points) {
+  if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
+  if (cap_points < 0) return VLOAM_E_INVALID;
+  return vl_lm_get_map(c, out_xyzi, cap_points);
 }
 void* vloam_b200_stream(vloam_b200_ctx* c) { if (!c) return nullptr; return (void*)c->stream; }
 long long vloam_b200_kernel_launches(const vloam_b200_ctx* c) { if (!c) return 0; return c->launches; }
@@ -637,6 +648,7 @@ long vloam_b200_debug_get(vloam_b200_ctx* c, const char* name, void* out, long c
     return put_host(v, sizeof v, out, cap);
   }
   if (n == "alloc.count") { const long long v = c->regrows; return put_host(&v, sizeof v, out, cap); }  // device buffer (re)allocations so far
+  if (n == "lm.paths") { long long v[2]; vl_lm_paths(c, v); return put_host(v, sizeof v, out, cap); }  // mapped sweeps since create: {in-place, pool path}
   if (n == "lo.costs") return put_host(c->dbgLoCost, sizeof c->dbgLoCost, out, cap);
   if (n == "lm.costs") return put_host(c->dbgLmCost, sizeof c->dbgLmCost, out, cap);
   if (n == "lm.pose" || n == "lm.state" || n == "lm.validInd") {

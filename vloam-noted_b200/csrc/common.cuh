@@ -397,6 +397,10 @@ int vl_lm_run(vloam_b200_ctx* c);
 int vl_lm_enqueue_stacks(vloam_b200_ctx* c, const float4* corner, int nc, const float4* surf, int ns, bool early = false);
 int vl_lm_enqueue_stacks_next(vloam_b200_ctx* c, const float4* corner, int nc, const float4* surf, int ns);  // into the spare stack buffers (helper thread)
 int vl_lm_adopt_stacks_next(vloam_b200_ctx* c);  // make the spare stack buffers current
+int vl_lm_publish_map(vloam_b200_ctx* c);         // queue the assembly of laserCloudMap (LM.cpp:884-899) on the publication stream
+int vl_lm_get_map(vloam_b200_ctx* c, float* out, int cap_points);  // wait for it and copy it out
+int vl_lm_pub_sync(vloam_b200_ctx* c);            // host wait for the last publication
+void vl_lm_paths(vloam_b200_ctx* c, long long out[2]);  // mapped sweeps on the in-place / pool path since create
 int vl_lm_init(vloam_b200_ctx* c);
 void vl_lm_free(vloam_b200_ctx* c);
 extern "C" int vl_launch_lookahead(vloam_b200_ctx* c);  // capi.cu: queue the registered look-ahead scan registration (no-op without one)

@@ -1637,6 +1637,143 @@ __global__ void lm_set_counts(LmScalars* s, RfWork* w, const int* qc, const int*
   w->nq = s->optimized ? *qc + *qs : 0;  // factor slots the solver looks at
 }
 
+// ---- LaserMapping::publish: laserCloudMap (LM.cpp:884-899) assembled on the device, without touching the map -------------------
+// Output: for cube i = 0 .. 4850 in table order, corner cube i then surf cube i -- segment q = 2 i + kind -- each cube's points in
+// the order the pools hold them after a pool-path sweep (pcl::VoxelGrid's order, raw appends after it).  Where a segment's points
+// are taken from:
+//   * the pools, for every cube when they are current, and for the cubes outside the grid's window otherwise;
+//   * the grid, for the grid window's valid cubes after in-place updates (the pools are stale there).  The live entries of such a
+//     segment, in ascending voxel key, are what lm_materialize would write: an entry from the build keeps its rank in the stale
+//     (key-ordered) pool prefix, shifted by the voxels created since with a smaller key; a voxel created since goes to the number
+//     of prefix points with a smaller key (binary search, as rf_match) plus its rank among the new voxels of its segment (sorted
+//     per segment with rf_seg_scatter / rf_seg_sort).  One scatter then writes every point to its final slot.
+// Nothing here writes pools, cube tables, the grid or LmScalars; the merge scratch is the assembly's own.
+#define MP_NSEG (2 * VL_CUBE_NUM)
+#define MP_INTS (2 * MP_NSEG + 2)
+#define MP_CNT (MP_NSEG + 1)   // pubInt[MP_CNT]: voxels created since the grid was built (collected)
+#define MP_SRC (MP_NSEG + 2)   // pubInt[MP_SRC + q]: pool start of segment q, -1 = from the grid
+
+// every live grid entry created since the build (posOf < 0) -> (segment | voxel key | j) and its entry index
+__global__ void __launch_bounds__(256) mp_collect(LgGrid g, RfWork* __restrict__ w, unsigned long long* __restrict__ keys, int* __restrict__ ent,
+                                                  int* __restrict__ counter, int cap) {
+  VL_PDL_WAIT();
+  for (int cell = blockIdx.x * blockDim.x + threadIdx.x; cell < 2 * LM_NCELL; cell += gridDim.x * blockDim.x) {
+    const int2 d = g.dir[cell];
+    const int kind = cell >= LM_NCELL;
+    int chunk = d.y;
+    for (int left = d.x; left > 0; left -= LG_C, chunk = left > 0 ? g.next[chunk] : -1) {
+      const int m = min(left, LG_C);
+      for (int i = 0; i < m; ++i) {
+        const int e = chunk * LG_C + i;
+        const unsigned long long key = g.key[e];
+        if (key == LG_DEAD || g.posOf[e] >= 0) continue;
+        const int j = atomicAdd(counter, 1);
+        if (j >= cap) continue;  // (the host bounds the voxels created since the build; vl_lm_get_map reports a violation)
+        const int sg = kind * VL_MAX_VALID + (int)(key >> 32);
+        keys[j] = ((unsigned long long)sg << 56) | ((unsigned long long)((unsigned)key & 0x3fffffffu) << 26) | (unsigned long long)j;
+        ent[j] = e;
+        atomicAdd(&w->segCount[sg], 1);
+      }
+    }
+  }
+}
+
+// points per output segment -> exclusive offsets (pubInt[0 .. MP_NSEG]) and where each segment comes from (pubInt[MP_SRC + q])
+__global__ void __launch_bounds__(1024) mp_layout(const LgHeader* __restrict__ gh, const RfWork* __restrict__ w, const MapCubeTable* __restrict__ tc,
+                                                  const MapCubeTable* __restrict__ ts, int fromGrid, int* __restrict__ pub) {
+  VL_PDL_WAIT();
+  __shared__ int slotOf[VL_CUBE_NUM];
+  __shared__ int ws[32];
+  for (int i = threadIdx.x; i < VL_CUBE_NUM; i += 1024) slotOf[i] = -1;
+  __syncthreads();
+  if (fromGrid && (int)threadIdx.x < gh->validNum) slotOf[gh->validInd[threadIdx.x]] = threadIdx.x;
+  __syncthreads();
+  constexpr int PER = (MP_NSEG + 1023) / 1024;
+  const int q0 = threadIdx.x * PER;
+  int cnt[PER], own = 0;
+#pragma unroll
+  for (int k = 0; k < PER; ++k) {
+    const int q = q0 + k;
+    cnt[k] = 0;
+    if (q >= MP_NSEG) continue;
+    const int cb = q >> 1, kind = q & 1;
+    const MapCubeTable* tb = kind ? ts : tc;
+    const int slot = slotOf[cb];
+    cnt[k] = tb->count[cb] + (slot >= 0 ? w->segCount[kind * VL_MAX_VALID + slot] : 0);
+    pub[MP_SRC + q] = slot >= 0 ? -1 : tb->start[cb];
+    own += cnt[k];
+  }
+  int tot = 0;
+  int run = vl_block_excl_scan<1024>(own, ws, &tot);
+#pragma unroll
+  for (int k = 0; k < PER; ++k) if (q0 + k < MP_NSEG) { pub[q0 + k] = run; run += cnt[k]; }
+  if (threadIdx.x == 0) pub[MP_NSEG] = tot;
+}
+
+// segments taken from the pools: one thread per output point
+__global__ void __launch_bounds__(256) mp_copy_pools(const int* __restrict__ pub, const float4* __restrict__ poolC, const float4* __restrict__ poolS,
+                                                     float4* __restrict__ out, int outCap) {
+  VL_PDL_WAIT();
+  const int total = min(pub[MP_NSEG], outCap);
+  for (int g = blockIdx.x * blockDim.x + threadIdx.x; g < total; g += gridDim.x * blockDim.x) {
+    int lo = 0, hi = MP_NSEG;
+    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (pub[mid] <= g) lo = mid; else hi = mid; }
+    const int src = pub[MP_SRC + lo];
+    if (src >= 0) out[g] = ((lo & 1) ? poolS : poolC)[src + g - pub[lo]];
+  }
+}
+
+// segments taken from the grid, entries that existed when it was built: stale pool rank + new voxels of the segment with a smaller key
+__global__ void __launch_bounds__(256) mp_grid_old(LgGrid g, const RfWork* __restrict__ w, const unsigned long long* __restrict__ sorted,
+                                                   const int* __restrict__ pub, float4* __restrict__ out, int outCap) {
+  VL_PDL_WAIT();
+  for (int cell = blockIdx.x * blockDim.x + threadIdx.x; cell < 2 * LM_NCELL; cell += gridDim.x * blockDim.x) {
+    const int2 d = g.dir[cell];
+    const int kind = cell >= LM_NCELL;
+    int chunk = d.y;
+    for (int left = d.x; left > 0; left -= LG_C, chunk = left > 0 ? g.next[chunk] : -1) {
+      const int m = min(left, LG_C);
+      for (int i = 0; i < m; ++i) {
+        const int e = chunk * LG_C + i;
+        const unsigned long long key = g.key[e];
+        const int pos = g.posOf[e];
+        if (key == LG_DEAD || pos < 0) continue;
+        const int slot = (int)(key >> 32), sg = kind * VL_MAX_VALID + slot;
+        const unsigned vk = (unsigned)key & 0x3fffffffu;
+        int a = w->tailBegin[sg], b = w->tailBegin[sg + 1];
+        const int segBegin = a;
+        while (a < b) { const int mid = (a + b) >> 1; if (RF_VOX(sorted[mid]) < vk) a = mid + 1; else b = mid; }
+        const int o = pub[2 * g.hdr->validInd[slot] + kind] + pos + (a - segBegin);
+        if (o < outCap) out[o] = g.pts[e];
+      }
+    }
+  }
+}
+
+// segments taken from the grid, voxels created since the build (sorted per segment): prefix points with a smaller key + rank
+__global__ void __launch_bounds__(256) mp_grid_new(LgGrid g, const RfWork* __restrict__ w, const unsigned long long* __restrict__ sorted,
+                                                   const int* __restrict__ ent, vloam_b200_params prm, const MapCubeTable* __restrict__ tc,
+                                                   const MapCubeTable* __restrict__ ts, const float4* __restrict__ poolC,
+                                                   const float4* __restrict__ poolS, const int* __restrict__ pub, float4* __restrict__ out, int outCap) {
+  VL_PDL_WAIT();
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= w->nKeysValid) return;
+  const unsigned long long key = sorted[t];
+  const int sg = (int)(key >> 56);
+  const int kind = sg / VL_MAX_VALID, slot = sg % VL_MAX_VALID;
+  const unsigned vk = RF_VOX(key);
+  const LgHeader* h = g.hdr;
+  const int cb = h->validInd[slot];
+  const int ci = cb % VL_CUBE_W, cj = (cb / VL_CUBE_W) % VL_CUBE_H, ck = cb / (VL_CUBE_W * VL_CUBE_H);
+  const MapCubeTable* tb = kind ? ts : tc;
+  const float4* pool = (kind ? poolS : poolC) + tb->start[cb];
+  const float inv = lm_leaf_inv(prm, kind);
+  int lo = 0, hi = tb->count[cb];  // (every point of a grid-window cube is in its filtered prefix: a tail would have kept the grid dirty)
+  while (lo < hi) { const int mid = (lo + hi) >> 1; if (lm_vox_key(pool[mid], inv, ci, cj, ck, h->cenW, h->cenH, h->cenD) < vk) lo = mid + 1; else hi = mid; }
+  const int o = pub[2 * cb + kind] + lo + (t - w->tailBegin[sg]);
+  if (o < outCap) out[o] = g.pts[ent[(int)(key & 0x3ffffffull)]];
+}
+
 // -----------------------------------------------------------------------------------------------
 #define LM_POOL_C (16 << 20)
 #define LM_POOL_S (48 << 20)
@@ -1661,6 +1798,16 @@ struct LmDevice {  // extra device state owned by this file
   long long builtCountC;             // ... of them corner points
   long long baseC, baseS;            // bound on the map size (all cubes) when the grid was built, and the raw appends outside the window
   long long outBaseC, outBaseS;      // counted until then: the bound of every later sweep follows the DEVICE counts from there (no drift)
+  long long paths[2];                // mapped sweeps since create that took the in-place path / the pool path ("lm.paths")
+  // ---- map publication (LaserMapping::publish's laserCloudMap, vl_lm_publish_map)
+  cudaStream_t pubStream;            // the assembly runs here, behind the last map update; every later map edit waits for evPub
+  cudaEvent_t evPub;
+  RfWork* pubWork;                   // the assembly's own merge scratch (the update's `work` may be in use by the next sweep)
+  int* pubInt;                       // [MP_NSEG + 1] output offsets (last: points) | new-voxel counter | [MP_NSEG] pool start or -1 (grid)
+  DBuf<unsigned long long> pubKeys; DBuf<int> pubEnt;  // new voxels: sort keys (unsorted | sorted | scratch) and their grid entries
+  DBuf<float4> pubOut;               // the published cloud
+  bool pubDone;                      // something was published since create
+  long long pubNewCap, pubOutCap;    // bounds the last assembly was sized for (checked by vl_lm_get_map)
 };
 static LmDevice* lmdev(vloam_b200_ctx* c) { return reinterpret_cast<LmDevice*>(c->gridPrm); }
 
@@ -1672,6 +1819,7 @@ static int lg_reserve(vloam_b200_ctx* c, LmDevice* d, long long chunks) {
   long long ncap = d->grid.cap ? d->grid.cap : (1LL << 20);
   while (ncap < chunks) ncap *= 2;
   VL_CUDA(cudaStreamSynchronize(VL_STREAM(c)));  // (only ever called right before a full rebuild: the old contents are dead)
+  if (d->pubStream) VL_CUDA(cudaEventSynchronize(d->evPub));  // ... but a map publication may still be reading them
   if (d->grid.pts) { cudaFree(d->grid.pts); cudaFree(d->grid.key); cudaFree(d->grid.next); cudaFree(d->grid.posOf); }
   __atomic_fetch_add(&c->regrows, 1LL, __ATOMIC_RELAXED);
   VL_CUDA(cudaMalloc(&d->grid.pts, (size_t)ncap * LG_C * sizeof(float4)));
@@ -1698,6 +1846,11 @@ int vl_lm_init(vloam_b200_ctx* c) {
   VL_CUDA(cudaMalloc(&d->grid.hdr, sizeof(LgHeader)));
   VL_CUDA(cudaMemset(d->grid.hdr, 0, sizeof(LgHeader)));
   VL_TRY(lg_reserve(c, d, 1 << 21));  // 2 Mi chunks (~0.8 GB of the 180 GB): a ~30M-point sub-map before the first regrow
+  VL_CUDA(cudaStreamCreateWithFlags(&d->pubStream, cudaStreamNonBlocking));  // (default = lowest priority: the assembly is never on the pose chain)
+  VL_CUDA(cudaEventCreateWithFlags(&d->evPub, cudaEventDisableTiming));
+  VL_CUDA(cudaMalloc(&d->pubWork, sizeof(RfWork)));
+  VL_CUDA(cudaMalloc(&d->pubInt, sizeof(int) * MP_INTS));
+  VL_CUDA(cudaMemset(d->pubInt, 0, sizeof(int) * MP_INTS));
   d->gridEnabled = getenv("VLOAM_NO_SPECULATION") == nullptr && getenv("VLOAM_NO_GRID") == nullptr;
   d->gridValid = false; d->poolsStale = false; d->gridTopUpper = 0; d->newVoxUpper = 0; d->builtCount = 0;
   VL_CUDA(cudaFuncSetAttribute(rf_seg_sort, cudaFuncAttributeMaxDynamicSharedMemorySize, RF_SEG_CAP * 8));
@@ -1728,8 +1881,11 @@ int vl_lm_init(vloam_b200_ctx* c) {
 void vl_lm_free(vloam_b200_ctx* c) {  // everything vl_lm_init and this file's reserves own (the pools are freed by capi.cu)
   LmDevice* d = lmdev(c);
   if (!d) return;
+  if (d->pubStream) { cudaStreamSynchronize(d->pubStream); cudaStreamDestroy(d->pubStream); }
+  if (d->evPub) cudaEventDestroy(d->evPub);
   void* dev[] = {d->work, d->dQ, d->subReal, d->subSpec, d->newPts.p, d->newCube.p, d->unmatched.p, d->grid.dir, d->grid.top, d->grid.hdr,
-                 d->grid.pts, d->grid.key, d->grid.next, d->grid.posOf, d->muKey.p, d->muInt.p, d->knnIds.p};
+                 d->grid.pts, d->grid.key, d->grid.next, d->grid.posOf, d->muKey.p, d->muInt.p, d->knnIds.p,
+                 d->pubWork, d->pubInt, d->pubKeys.p, d->pubEnt.p, d->pubOut.p};
   for (void* p : dev) vl_dev_free(c, p);
   delete d;
   c->gridPrm = nullptr;
@@ -1817,6 +1973,8 @@ static int lg_rebuild_launch(vloam_b200_ctx* c, LmDevice* d, const LmSub* sub, l
 static int lm_pool_headroom(vloam_b200_ctx* c, long long totalC, long long totalS, int Qc, int Qs) {
   const size_t needC = 2 * ((size_t)totalC + Qc) + 256 * (size_t)(VL_MAX_VALID + min(Qc, VL_CUBE_NUM));
   const size_t needS = 2 * ((size_t)totalS + Qs) + 256 * (size_t)(VL_MAX_VALID + min(Qs, VL_CUBE_NUM));
+  const bool growC = (size_t)c->h_lmm->poolTopC + needC > c->poolC.cap, growS = (size_t)c->h_lmm->poolTopS + needS > c->poolS.cap;
+  if (growC || growS) VL_CUDA(cudaEventSynchronize(lmdev(c)->evPub));  // a map publication in flight reads the pool that is replaced
   if ((size_t)c->h_lmm->poolTopC + needC > c->poolC.cap) VL_TRY(vl_reserve(c, c->poolC, 2 * ((size_t)c->h_lmm->poolTopC + needC), true));
   if ((size_t)c->h_lmm->poolTopS + needS > c->poolS.cap) VL_TRY(vl_reserve(c, c->poolS, 2 * ((size_t)c->h_lmm->poolTopS + needS), true));
   return VLOAM_OK;
@@ -1848,6 +2006,7 @@ static int lm_materialize(vloam_b200_ctx* c, LmDevice* d) {
   VL_TRY(vl_reserve(c, d->unmatched, (size_t)P + 2, false, (size_t)P + (1 << 16)));
   VL_TRY(vl_reserve(c, c->staging, (size_t)total + P + 1, false, (size_t)total / 2 + (1 << 20)));
   const int gsGrid = c->num_sms * 8;
+  VL_CUDA(cudaStreamWaitEvent(VL_STREAM(c), d->evPub, 0));  // a map publication may still read the stale pools and the grid
   VL_CUDA(cudaMemsetAsync(keysIn, 0xff, N * sizeof(unsigned long long), VL_STREAM(c)));  // unused key slots read as "no key"
   VL_LAUNCH(mz_layout_for_grid, 1, 256, 0, c->lmm, d->work, d->grid.hdr, c->cubeC, c->cubeS);
   VL_BYTES(32.0 * (double)total);
@@ -2065,6 +2224,8 @@ int vl_lm_run(vloam_b200_ctx* c) {
       mw.foundCell = mw.found + nq; mw.members = mw.foundCell + nq;
       // (the scratch is cleared behind the previous update, on its stream, BEFORE the wait for this sweep's pose: off the chain)
       VL_CUDA(cudaStreamWaitEvent(c->stream3, c->evAux, 0));                // (anyOutside is read by the previous sweep's append on streamAux)
+      // a map publication queued since the last update reads the grid and the pools that mu_apply and rf_append_outside (behind evUpd) edit
+      VL_CUDA(cudaStreamWaitEvent(c->stream3, d->evPub, 0));
       VL_CUDA(cudaMemsetAsync(mw.hkey, 0xff, (size_t)H * 8, c->stream3));   // empty slots
       VL_CUDA(cudaMemsetAsync(mw.cnt, 0, (size_t)(H + 4) * 4, c->stream3));  // group sizes and the anyOutside flag behind them
       VL_CUDA(cudaStreamWaitEvent(c->stream3, c->evPose, 0));
@@ -2103,6 +2264,7 @@ int vl_lm_run(vloam_b200_ctx* c) {
       d->hMapUpperS = d->baseS + ((c->h_lmm->gridCount - c->h_lmm->gridCountC) - (d->builtCount - d->builtCountC)) + (c->h_lmm->outsideS - d->outBaseS) + Qs;
       d->newVoxUpper = (long long)c->h_lmm->gridCount - d->builtCount + nq;  // voxels created so far (device count at S2) + at most nq by this update
       if (nq > 0) d->poolsStale = true;
+      d->paths[0]++;
       c->lm_frameCount++;
       VL_HOST_MARK(7);
       VL_CUDA(cudaGetLastError());
@@ -2113,7 +2275,11 @@ int vl_lm_run(vloam_b200_ctx* c) {
 
   // ---- pool path (round 1's): cube tables, sorted pools; the grid is rebuilt for the window lm_prepare finds
   VL_CUDA(cudaStreamWaitEvent(c->stream, c->evAux, 0));  // (the previous sweep's raw appends outside the window edit the cube tables)
+  // a map publication queued since the last update: lm_prepare rolls the cube tables it reads, and this stream's evPose orders the
+  // update, the speculative rebuild and the appends (stream3, streamAux) behind it as well
+  VL_CUDA(cudaStreamWaitEvent(c->stream, d->evPub, 0));
   if (d->poolsStale) VL_TRY(lm_materialize(c, d));  // the in-place updates since the last pool-path sweep, written back first (main stream)
+  d->paths[1]++;
   VL_LAUNCH(lm_prepare, 1, 1024, 0, c->lmm, c->los, c->cubeC, c->cubeS, d->work, 0, resetValid, d->subReal);
   const long long totalBound = d->hMapUpperC + d->hMapUpperS;
   if (d->gridEnabled) VL_TRY(lm_reserve_merge(c, d, totalBound));
@@ -2295,6 +2461,88 @@ int vl_lm_import_map(vloam_b200_ctx* c, int which, const void* data, long bytes)
   return VLOAM_OK;
 }
 
+// LaserMapping::publish (LM.cpp:884-899): queue the assembly of laserCloudMap on the publication stream, behind the last map
+// update (evMap) and its raw appends (evAux).  The host does not wait; every later edit of the map waits for evPub on the device
+// (vl_lm_run, lm_materialize), and the host waits for it before it replaces a buffer the assembly reads (lm_pool_headroom,
+// lg_reserve, vl_lm_pub_sync before imports and destroy).
+int vl_lm_publish_map(vloam_b200_ctx* c) {
+  LmDevice* d = lmdev(c);
+  VL_TRY(vl_lm_join(c));  // the helper thread has issued the last update (evMap, evAux recorded; poolsStale / newVoxUpper / hMapUpper* current)
+  struct Restore { cudaStream_t prev; ~Restore() { vl_tls_stream = prev; } } restore{vl_tls_stream};
+  vl_tls_stream = d->pubStream;
+  const bool fromGrid = d->poolsStale;
+  const long long bound = d->hMapUpperC + d->hMapUpperS;
+  // buffers first, while this stream holds nothing but earlier publications: a regrow syncs the stream, and behind the waits
+  // below that would make the host wait for the map update in flight
+  VL_TRY(vl_reserve(c, d->pubOut, (size_t)max(bound, 1LL), false, (size_t)bound / 2 + (1 << 20)));
+  if (fromGrid) {
+    VL_TRY(vl_reserve(c, d->pubKeys, (size_t)4 * LG_NEWVOX_MAX));  // sized once for the largest bound: [0, N) unsorted | [N, 2N) sorted | [2N, 4N) scratch
+    VL_TRY(vl_reserve(c, d->pubEnt, (size_t)LG_NEWVOX_MAX));
+  }
+  VL_CUDA(cudaStreamWaitEvent(d->pubStream, c->evMap, 0));
+  VL_CUDA(cudaStreamWaitEvent(d->pubStream, c->evAux, 0));
+  d->pubOutCap = (long long)d->pubOut.cap;
+  const int gsGrid = c->num_sms * 8;
+  const int outCap = (int)min(d->pubOutCap, (long long)INT_MAX);
+  int* pub = d->pubInt;
+  VL_CUDA(cudaMemsetAsync(d->pubWork, 0, sizeof(RfWork), d->pubStream));
+  VL_CUDA(cudaMemsetAsync(pub + MP_CNT, 0, sizeof(int), d->pubStream));
+  const int P = fromGrid ? (int)max(min(d->newVoxUpper, (long long)LG_NEWVOX_MAX), 1LL) : 0;
+  const size_t N = ((size_t)P + 255) & ~(size_t)255;
+  unsigned long long* keysIn = nullptr; unsigned long long* keysSorted = nullptr;
+  if (fromGrid) {
+    keysIn = d->pubKeys.p; keysSorted = d->pubKeys.p + N;
+    VL_CUDA(cudaMemsetAsync(keysIn, 0xff, N * sizeof(unsigned long long), d->pubStream));
+    VL_BYTES(16.0 * LM_NCELL + 12.0 * bound);
+    VL_LAUNCH(mp_collect, gsGrid, 256, 0, d->grid, d->pubWork, keysIn, d->pubEnt.p, pub + MP_CNT, P);
+    VL_LAUNCH(rf_seg_scatter, vl_div_up(P, 256), 256, 0, keysIn, P, d->pubWork, keysSorted);
+    VL_LAUNCH(rf_seg_sort, LM_NSEG, RF_SEG_THREADS, (size_t)RF_SEG_CAP * 8, keysSorted, d->pubWork, d->pubKeys.p + 2 * N, RF_SEG_CAP);
+  }
+  d->pubNewCap = P;
+  VL_LAUNCH(mp_layout, 1, 1024, 0, (const LgHeader*)d->grid.hdr, (const RfWork*)d->pubWork, (const MapCubeTable*)c->cubeC, (const MapCubeTable*)c->cubeS,
+            fromGrid ? 1 : 0, pub);
+  VL_BYTES(32.0 * bound);  // every point read once and written once (upper bound: the grid's share is moved by the kernels below)
+  VL_LAUNCH(mp_copy_pools, gsGrid, 256, 0, (const int*)pub, (const float4*)c->poolC.p, (const float4*)c->poolS.p, d->pubOut.p, outCap);
+  if (fromGrid) {
+    VL_LAUNCH(mp_grid_old, gsGrid, 256, 0, d->grid, (const RfWork*)d->pubWork, (const unsigned long long*)keysSorted, (const int*)pub, d->pubOut.p, outCap);
+    VL_LAUNCH(mp_grid_new, vl_div_up(P, 256), 256, 0, d->grid, (const RfWork*)d->pubWork, (const unsigned long long*)keysSorted, (const int*)d->pubEnt.p,
+              c->prm, (const MapCubeTable*)c->cubeC, (const MapCubeTable*)c->cubeS, (const float4*)c->poolC.p, (const float4*)c->poolS.p, (const int*)pub,
+              d->pubOut.p, outCap);
+  }
+  VL_CUDA(cudaEventRecord(d->evPub, d->pubStream));
+  VL_CUDA(cudaGetLastError());
+  d->pubDone = true;
+  return VLOAM_OK;
+}
+
+// wait for the last publication and copy its cloud out (out == NULL: size query)
+int vl_lm_get_map(vloam_b200_ctx* c, float* out, int cap_points) {
+  LmDevice* d = lmdev(c);
+  if (!d->pubDone) { snprintf(c->err, sizeof c->err, "get_map: nothing was published"); return VLOAM_E_INVALID; }
+  VL_CUDA(cudaStreamWaitEvent(c->stream, d->evPub, 0));
+  int h[2] = {0, 0};  // {points, voxels created since the grid was built}
+  VL_CUDA(cudaMemcpyAsync(h, d->pubInt + MP_NSEG, sizeof h, cudaMemcpyDeviceToHost, c->stream));
+  VL_CUDA(cudaStreamSynchronize(c->stream));
+  if (h[1] > d->pubNewCap || h[0] > d->pubOutCap) {
+    snprintf(c->err, sizeof c->err, "get_map: the published map exceeded its bounds (%d points / %lld, %d new voxels / %lld)", h[0], d->pubOutCap, h[1], d->pubNewCap);
+    return VLOAM_E_CAPACITY;
+  }
+  if (!out || h[0] == 0) return h[0];
+  if (cap_points < h[0]) { snprintf(c->err, sizeof c->err, "map buffer too small (%d < %d)", cap_points, h[0]); return VLOAM_E_CAPACITY; }
+  VL_CUDA(cudaMemcpyAsync(out, d->pubOut.p, (size_t)h[0] * 16, cudaMemcpyDeviceToHost, c->stream));
+  VL_CUDA(cudaStreamSynchronize(c->stream));
+  return h[0];
+}
+
+// host wait for the last publication (before the map is replaced from the host, and in vloam_b200_synchronize)
+int vl_lm_pub_sync(vloam_b200_ctx* c) {
+  LmDevice* d = lmdev(c);
+  if (d && d->pubStream) VL_CUDA(cudaStreamSynchronize(d->pubStream));
+  return VLOAM_OK;
+}
+
+void vl_lm_paths(vloam_b200_ctx* c, long long out[2]) { const LmDevice* d = lmdev(c); out[0] = d->paths[0]; out[1] = d->paths[1]; }
+
 int vl_chain_trace_arm_lm(void* dev) { return cudaMemcpyToSymbol(g_chain_trace, &dev, sizeof(void*)) == cudaSuccess ? VLOAM_OK : VLOAM_E_CUDA; }
 int vl_lm_preload(vloam_b200_ctx* c) {  // see vl_sr_set_attrs: load every kernel of this file when a context is created
   cudaFuncAttributes fa_;
@@ -2321,5 +2569,7 @@ int vl_lm_preload(vloam_b200_ctx* c) {  // see vl_sr_set_attrs: load every kerne
   VL_CUDA(cudaFuncGetAttributes(&fa_, lm_scan_sorted));
   VL_CUDA(cudaFuncGetAttributes(&fa_, lm_set_counts));
   VL_CUDA(cudaFuncGetAttributes(&fa_, lm_register_full));
+  VL_CUDA(cudaFuncGetAttributes(&fa_, mp_collect)); VL_CUDA(cudaFuncGetAttributes(&fa_, mp_layout)); VL_CUDA(cudaFuncGetAttributes(&fa_, mp_copy_pools));
+  VL_CUDA(cudaFuncGetAttributes(&fa_, mp_grid_old)); VL_CUDA(cudaFuncGetAttributes(&fa_, mp_grid_new));
   return VLOAM_OK;
 }
