@@ -56,7 +56,7 @@ typedef struct vloam_b200_params {
   float line_res;         /* mapping_line_resolution */
   float plane_res;        /* mapping_plane_resolution */
   int mapping_skip_frame; /* mapping_skip_frame */
-  int reserved;           /* flags: VLOAM_FLAG_DISTORTION or 0 */
+  int reserved;           /* flags: VLOAM_FLAG_DISTORTION | VLOAM_FLAG_TRANSFORM_TO_END, or 0 */
 } vloam_b200_params;
 
 /* LaserOdometry::DISTORTION (laser_odometry.h:90; a compile-time `false` in the reference): with this flag set in
@@ -64,6 +64,15 @@ typedef struct vloam_b200_params {
  * int(intensity)) / SCAN_PERIOD: TransformToStart uses Identity.slerp(s, q_last_curr) and s * t_last_curr
  * (laser_odometry.cpp:152-173) and the two odometry functors interpolate the same way (lidarFactor.hpp:29-33, 86-90). */
 #define VLOAM_FLAG_DISTORTION 1
+/* TransformToEnd (laser_odometry.cpp:176-193) applied as the block at laser_odometry.cpp:537-556 does (under `if (0)` in
+ * the reference, whose KITTI sweeps come motion-compensated): after every odometry solve -- on the first frame too, with
+ * identity -- every point of cornerPointsLessSharp, surfPointsLessFlat and laserCloudFullRes is moved into the frame of the
+ * sweep's END: un = TransformToStart(p) (float; s from the intensity under VLOAM_FLAG_DISTORTION, s = 1 otherwise), then
+ * q_last_curr.inverse() * (un - t_last_curr) in double, stored as float, intensity truncated to int(intensity).  Those clouds
+ * become the "last" clouds of the next odometry solve and the mapping stage's input, and vloam_b200_register_full_cloud
+ * registers the end-frame full-resolution cloud.  Set it together with VLOAM_FLAG_DISTORTION to de-skew sweeps that are not
+ * motion-compensated; accepted with or without it. */
+#define VLOAM_FLAG_TRANSFORM_TO_END 2
 
 typedef struct vloam_b200_ctx vloam_b200_ctx;
 
@@ -75,8 +84,10 @@ enum {
   VLOAM_CLOUD_LESS_SHARP = 2,  /* cornerPointsLessSharp */
   VLOAM_CLOUD_FLAT = 3,        /* surfPointsFlat */
   VLOAM_CLOUD_LESS_FLAT = 4,   /* surfPointsLessFlat */
-  VLOAM_CLOUD_CORNER_LAST = 5, /* laserCloudCornerLast (after solveLO's swap) */
-  VLOAM_CLOUD_SURF_LAST = 6    /* laserCloudSurfLast */
+  VLOAM_CLOUD_CORNER_LAST = 5, /* laserCloudCornerLast (after solveLO's swap; end frame under VLOAM_FLAG_TRANSFORM_TO_END) */
+  VLOAM_CLOUD_SURF_LAST = 6,   /* laserCloudSurfLast (same) */
+  VLOAM_CLOUD_FULL_RES = 7     /* laserCloudFullRes as LaserOdometry::output hands it over: VLOAM_CLOUD_FULL, in the sweep-end
+                                  frame under VLOAM_FLAG_TRANSFORM_TO_END (byte-equal to VLOAM_CLOUD_FULL without the flag) */
 };
 
 void vloam_b200_default_params(vloam_b200_params* p);
@@ -132,7 +143,8 @@ int vloam_b200_laser_mapping(vloam_b200_ctx* c, double* q_w_curr, double* t_w_cu
 
 /* The full-resolution cloud of this sweep registered into the map frame: LaserMapping::publish's loop
  * over laserCloudFullRes with pointAssociateToMap (LM.cpp:901-905; q_w_curr / t_w_curr after
- * solveMapping, the propagated pose on skipped frames).  out_xyzi: HOST buffer of cap_points points (NULL
+ * solveMapping, the propagated pose on skipped frames).  Under VLOAM_FLAG_TRANSFORM_TO_END each point is
+ * pointAssociateToMap(TransformToEnd(p)) with a float intermediate, the cloud LaserOdometry hands over.  out_xyzi: HOST buffer of cap_points points (NULL
  * to query the size).  Returns the number of points or a negative error. */
 int vloam_b200_register_full_cloud(vloam_b200_ctx* c, float* out_xyzi, int cap_points);
 

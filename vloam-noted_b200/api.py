@@ -8,7 +8,8 @@ import os
 import numpy as np
 from . import _build
 
-CLOUD_FULL, CLOUD_SHARP, CLOUD_LESS_SHARP, CLOUD_FLAT, CLOUD_LESS_FLAT, CLOUD_CORNER_LAST, CLOUD_SURF_LAST = range(7)
+CLOUD_FULL, CLOUD_SHARP, CLOUD_LESS_SHARP, CLOUD_FLAT, CLOUD_LESS_FLAT, CLOUD_CORNER_LAST, CLOUD_SURF_LAST, CLOUD_FULL_RES = range(8)
+FLAG_DISTORTION, FLAG_TRANSFORM_TO_END = 1, 2  # vloam_b200_params.reserved
 
 EXPORTS = [
     "vloam_b200_default_params", "vloam_b200_create", "vloam_b200_destroy", "vloam_b200_last_error", "vloam_b200_begin_frame",
@@ -109,9 +110,13 @@ def _decode(name, raw):
 class Context:
     """One vloam_b200_ctx: one sequence (several CUDA streams and a helper thread inside, include/vloam_b200.h)."""
 
-    def __init__(self, n_scans=64, minimum_range=5.0, line_res=0.4, plane_res=0.8, mapping_skip_frame=1, device=0, distortion=0):
+    def __init__(self, n_scans=64, minimum_range=5.0, line_res=0.4, plane_res=0.8, mapping_skip_frame=1, device=0, distortion=0,
+                 transform_to_end=False):
+        """distortion: VLOAM_FLAG_DISTORTION (per-point de-skew in the odometry); transform_to_end: VLOAM_FLAG_TRANSFORM_TO_END (every
+        sweep's less-sharp / less-flat / full-resolution clouds moved to the sweep end, LO.cpp:537-556)."""
         self.L = load_lib()
-        self.params = Params(n_scans, minimum_range, line_res, plane_res, mapping_skip_frame, 1 if distortion else 0)  # reserved: VLOAM_FLAG_DISTORTION
+        flags = (FLAG_DISTORTION if distortion else 0) | (FLAG_TRANSFORM_TO_END if transform_to_end else 0)
+        self.params = Params(n_scans, minimum_range, line_res, plane_res, mapping_skip_frame, flags)
         h = ctypes.c_void_p()
         r = self.L.vloam_b200_create(ctypes.byref(self.params), device, ctypes.byref(h))
         if r != 0:
@@ -336,7 +341,7 @@ class LaserOdometry:
     def output(self):
         g = self.ctx.get_cloud
         r = self.last
-        return r["q_w_curr"], r["t_w_curr"], g(CLOUD_CORNER_LAST), g(CLOUD_SURF_LAST), g(CLOUD_FULL), r["skip_frame"]
+        return r["q_w_curr"], r["t_w_curr"], g(CLOUD_CORNER_LAST), g(CLOUD_SURF_LAST), g(CLOUD_FULL_RES), r["skip_frame"]
 
 
 class LaserMapping:

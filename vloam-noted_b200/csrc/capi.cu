@@ -67,7 +67,7 @@ int vloam_b200_create(const vloam_b200_params* p, int device, vloam_b200_ctx** o
   // SR.cpp:58-61, 255-259: only 16 / 32 / 64 beams (128 = builder extension)
   if (p->n_scans != 16 && p->n_scans != 32 && p->n_scans != 64 && p->n_scans != 128) return VLOAM_E_INVALID;
   if (!(p->line_res >= 0.05f) || !(p->plane_res >= 0.05f) || p->mapping_skip_frame < 1) return VLOAM_E_INVALID;
-  if (p->reserved & ~VLOAM_FLAG_DISTORTION) return VLOAM_E_INVALID;
+  if (p->reserved & ~(VLOAM_FLAG_DISTORTION | VLOAM_FLAG_TRANSFORM_TO_END)) return VLOAM_E_INVALID;
   VL_CUDA_CREATE(cudaSetDevice(device));
   vloam_b200_ctx* c = new vloam_b200_ctx();  // value-initialised: every pointer / handle starts out null
   const int r = create_impl(c, p, device);
@@ -141,6 +141,7 @@ static int create_impl(vloam_b200_ctx* c, const vloam_b200_params* p, int device
   VL_CUDA_CREATE(cudaMallocHost(&c->h_s2flag, 64)); *c->h_s2flag = 0; c->s2seq = 0;
   VL_CUDA_CREATE(cudaEventCreateWithFlags(&c->evLoSolve, cudaEventDisableTiming));
   VL_CUDA_CREATE(cudaEventCreateWithFlags(&c->evLoNext, cudaEventDisableTiming));
+  VL_CUDA_CREATE(cudaEventCreateWithFlags(&c->evEnd, cudaEventDisableTiming));
   VL_CUDA_CREATE(cudaStreamCreateWithPriority(&c->streamLO, cudaStreamNonBlocking, pr[4]));
   c->loNextValid = c->loNextQueued = c->srAdopted = c->s2Done = false; c->loAssumeMonotone = c->inProcessFrame = c->loDeferred = false; c->srDeferred = c->sideSubmitted = false; c->preDeferred = c->loPreValid = c->sideWaitsIssued = c->earlyLoArmed = c->stacksAdopted = false; c->loNextSet = 0; c->stackSel = 0; c->stacksNextReady = false;
   VL_CUDA_CREATE(cudaMallocHost(&c->h_los, sizeof(LoScalars)));
@@ -188,14 +189,14 @@ void vloam_b200_destroy(vloam_b200_ctx* c) {
   vl_lm_free(c);
   vl_scan_free(&c->loScan[0]); vl_scan_free(&c->loScan[1]);
   if (c->streamLO) { cudaStreamSynchronize(c->streamLO); cudaStreamDestroy(c->streamLO); }
-  cudaEventDestroy(c->evS2); cudaEventDestroy(c->evLoSolve); cudaEventDestroy(c->evLoNext);
+  cudaEventDestroy(c->evS2); cudaEventDestroy(c->evLoSolve); cudaEventDestroy(c->evLoNext); if (c->evEnd) cudaEventDestroy(c->evEnd);
   void* singles[] = {c->los, c->losNext, c->evalOut, c->lms, c->lmm, c->cubeC, c->cubeS, c->vScalars, c->loRingTbl, c->loGridCells[0].p, c->loGridCells[1].p,
                      c->loGridCellOf.p, c->loGridSorted[0].p, c->loGridSorted[1].p, c->dbgLoCorner[0].p, c->dbgLoCorner[1].p, c->dbgLoSurf[0].p,
                      c->dbgLoSurf[1].p, c->dbgKnnIdx[0][0].p, c->dbgKnnIdx[0][1].p, c->dbgKnnIdx[1][0].p, c->dbgKnnIdx[1][1].p, c->dbgKnnD2[0][0].p,
                      c->dbgKnnD2[0][1].p, c->dbgKnnD2[1][0].p, c->dbgKnnD2[1][1].p, c->dbgKnnOk[0][0].p, c->dbgKnnOk[0][1].p, c->dbgKnnOk[1][0].p,
                      c->dbgKnnOk[1][1].p};
   for (void* p : singles) vl_dev_free(c, p);
-  void* bufs[] = {c->lessSharp[0].p, c->lessSharp[1].p, c->lessSharp[2].p, c->lessFlat[0].p, c->lessFlat[1].p, c->lessFlat[2].p, c->loCornerIdx.p, c->loSurfIdx.p, c->factors.p, c->factorS.p, c->factorValid.p, c->loFactors.p, c->loFactorValid.p, c->evalPartials.p,
+  void* bufs[] = {c->lessSharp[0].p, c->lessSharp[1].p, c->lessSharp[2].p, c->lessFlat[0].p, c->lessFlat[1].p, c->lessFlat[2].p, c->endSharp[0].p, c->endSharp[1].p, c->endSharp[2].p, c->endFlat[0].p, c->endFlat[1].p, c->endFlat[2].p, c->loCornerIdx.p, c->loSurfIdx.p, c->factors.p, c->factorS.p, c->factorValid.p, c->loFactors.p, c->loFactorValid.p, c->evalPartials.p,
                   c->poolC.p, c->poolS.p, c->stackC.p, c->stackS.p, c->stackCN.p, c->stackSN.p, c->fromMapC.p, c->fromMapS.p, c->knnIdx.p, c->knnD2.p, c->knnOk.p,
                   c->vKeys.p, c->vKeys2.p, c->vHead.p, c->vScan.p, c->vScan2.p, c->vOut.p, c->vIn.p, c->regOut.p, c->tailKeys.p, c->staging.p};
   for (void* p : bufs) vl_dev_free(c, p);
@@ -346,6 +347,14 @@ int vloam_b200_get_cloud(vloam_b200_ctx* c, int which, float* out, int cap_point
     case VLOAM_CLOUD_LESS_FLAT: src = c->lessFlat[c->cur].p; n = c->nLessFlat; break;
     case VLOAM_CLOUD_CORNER_LAST: src = c->cornerLastPtr; n = c->nCornerLast; break;
     case VLOAM_CLOUD_SURF_LAST: src = c->surfLastPtr; n = c->nSurfLast; break;
+    case VLOAM_CLOUD_FULL_RES:  // LaserOdometry::output's laserCloudFullRes: the end-frame cloud under VLOAM_FLAG_TRANSFORM_TO_END
+      src = c->cloud.p; n = c->nKept;
+      if (vl_to_end(c) && out && n > 0 && cap_points >= n) {
+        VL_TRY(vl_reserve(c, c->regOut, (size_t)n));
+        VL_TRY(vl_lo_to_end_cloud(c, c->cloud.p, n, c->regOut.p));
+        src = c->regOut.p;
+      }
+      break;
     default: snprintf(c->err, sizeof c->err, "unknown cloud id %d", which); return VLOAM_E_INVALID;
   }
   if (out && n > 0) {

@@ -160,7 +160,9 @@ struct vloam_b200_ctx {
   DBuf<int> selIdx;           // per-ring compacted selection (original indices)
   DBuf<float4> sharp, flat;
   DBuf<float4> lessSharp[3], lessFlat[3];  // three generations: the "last" clouds, this frame's ([cur]) and the look-ahead's
-  int cur;                    // index of this frame's lessSharp / lessFlat buffer
+  DBuf<float4> endSharp[3], endFlat[3];    // VLOAM_FLAG_TRANSFORM_TO_END: generation g's clouds in the sweep-end frame (lo_transform_to_end)
+  cudaEvent_t evEnd;                       // ... this sweep's end clouds are written (recorded by vl_lo_run; the stack filters wait on it)
+  int cur;                   // index of this frame's lessSharp / lessFlat buffer
   int nKept, nSharp, nLessSharp, nFlat, nLessFlat;  // host copies (valid after the SR sync point)
   bool sr_counts_valid;
   // look-ahead scan registration (vloam_b200_prefetch_scan[_device]): a second set of every field above (VL_SR_FIELDS)
@@ -447,6 +449,8 @@ int vl_solve_buf(vloam_b200_ctx* c, const double* d_factors, const int* d_valid,
                  const double* d_s, int ncta = 16);  // same on explicit factor buffers; ncta: CTAs of the solver's cluster (8 or 16: it fixes the summation order), on the calling thread's current stream (VL_STREAM)
 int vl_evaluate_once(vloam_b200_ctx* c, int nslots, const double* d_x, EvalOut* d_out, const double* d_s = nullptr);
 static inline bool vl_distortion(const vloam_b200_ctx* c) { return (c->prm.reserved & 1) != 0; }  // LaserOdometry::DISTORTION (LO.h:90)
+static inline bool vl_to_end(const vloam_b200_ctx* c) { return (c->prm.reserved & VLOAM_FLAG_TRANSFORM_TO_END) != 0; }  // LO.cpp:537-556 enabled
+int vl_lo_to_end_cloud(vloam_b200_ctx* c, const float4* d_in, int n, float4* d_out);  // TransformToEnd of n points with this sweep's q/t_last_curr
 
 // ---- shared device helpers -----------------------------------------------------
 #ifdef __CUDACC__
@@ -504,6 +508,18 @@ __device__ __forceinline__ void vl_transform_to_start(const double* pose, const 
     vl_qrot(pose, (double)p.x, (double)p.y, (double)p.z, r);
     sx = (float)(r[0] + pose[4]); sy = (float)(r[1] + pose[5]); sz = (float)(r[2] + pose[6]);
   }
+}
+// TransformToEnd (LO.cpp:176-193): un = TransformToStart(p) stored as float, then q_last_curr.inverse() * (un - t_last_curr) in
+// double, stored as float; intensity = int(intensity).  inverse() is Eigen's conjugate / squaredNorm (q is not exactly unit after
+// the solver's update), `*` Eigen's _transformVector (vl_qrot).
+__device__ __forceinline__ float4 vl_transform_to_end(const double* pose, const float4 p, int deskew) {
+  float ux, uy, uz;
+  vl_transform_to_start(pose, p, deskew, ux, uy, uz);
+  const double n2 = pose[0] * pose[0] + pose[1] * pose[1] + pose[2] * pose[2] + pose[3] * pose[3];
+  const double qi[4] = {-pose[0] / n2, -pose[1] / n2, -pose[2] / n2, pose[3] / n2};
+  double r[3];
+  vl_qrot(qi, (double)ux - pose[4], (double)uy - pose[5], (double)uz - pose[6], r);
+  return make_float4((float)r[0], (float)r[1], (float)r[2], (float)(int)p.w);
 }
 
 // Visit every element of up to 32 index ranges of ARRAY (float4) with all lanes busy, 128 elements per step.

@@ -556,6 +556,43 @@ __global__ void lo_accumulate(LoScalars* s) {
   for (int k = 0; k < 4; ++k) s->q_w[k] = qn[k];
 }
 
+// LO.cpp:537-556 (VLOAM_FLAG_TRANSFORM_TO_END): every point of a[0, na) followed by b[0, nb) through TransformToEnd with
+// pose = {q_last_curr, t_last_curr}, out of place.  na / nb are device counts (a look-ahead solve is queued before the host knows
+// them); na == nullptr takes the host count naHost.
+__global__ void __launch_bounds__(256) lo_transform_to_end(const float4* __restrict__ a, const int* __restrict__ na, int naHost, float4* __restrict__ ea,
+                                                           const float4* __restrict__ b, const int* __restrict__ nb, float4* __restrict__ eb,
+                                                           const double* __restrict__ pose, int deskew) {
+  VL_PDL_WAIT();
+  const int n0 = na ? *na : naHost, n1 = nb ? *nb : 0;
+  const double P[7] = {pose[0], pose[1], pose[2], pose[3], pose[4], pose[5], pose[6]};
+  for (int g = blockIdx.x * blockDim.x + threadIdx.x; g < n0 + n1; g += gridDim.x * blockDim.x) {
+    if (g < n0) ea[g] = vl_transform_to_end(P, a[g], deskew);
+    else eb[g - n0] = vl_transform_to_end(P, b[g - n0], deskew);
+  }
+}
+
+// This sweep's less-sharp / less-flat clouds (generation c->cur of the scan-registration set swapped in) into the end buffers of
+// the same generation, with the odometry state c->los, on the current stream.  Raw clouds stay readable; a discarded look-ahead
+// result only ever wrote the end buffers of its own generation.
+static int lo_queue_to_end(vloam_b200_ctx* c) {
+  const int g = c->cur;
+  VL_TRY(vl_reserve(c, c->endSharp[g], max(c->lessSharp[g].cap, (size_t)1)));
+  VL_TRY(vl_reserve(c, c->endFlat[g], max(c->lessFlat[g].cap, (size_t)1)));
+  VL_BYTES(32.0 * ((double)c->nLessSharp + c->nLessFlat));  // (last known counts)
+  VL_LAUNCH(lo_transform_to_end, c->num_sms * 4, 256, 0, (const float4*)c->lessSharp[g].p, (const int*)&c->srs->nLessSharp, 0, c->endSharp[g].p,
+            (const float4*)c->lessFlat[g].p, (const int*)&c->srs->nLessFlat, c->endFlat[g].p, (const double*)c->los->para_q, vl_distortion(c) ? 1 : 0);
+  VL_CUDA(cudaGetLastError());
+  return VLOAM_OK;
+}
+// the full-resolution cloud (n points, host count) through the same TransformToEnd, on the context's main stream
+int vl_lo_to_end_cloud(vloam_b200_ctx* c, const float4* d_in, int n, float4* d_out) {
+  VL_BYTES(32.0 * n);
+  VL_LAUNCH(lo_transform_to_end, c->num_sms * 4, 256, 0, d_in, (const int*)nullptr, n, d_out, (const float4*)nullptr, (const int*)nullptr,
+            (float4*)nullptr, (const double*)c->los->para_q, vl_distortion(c) ? 1 : 0);
+  VL_CUDA(cudaGetLastError());
+  return VLOAM_OK;
+}
+
 __global__ void lo_set_prior(LoScalars* s, const double* __restrict__ prior) {
   VL_PDL_WAIT();
   // LO.cpp:237-250
@@ -653,7 +690,7 @@ int vl_lo_preload(vloam_b200_ctx* c) {  // see vl_sr_set_attrs: load every kerne
   VL_CUDA(cudaFuncGetAttributes(&fa_, lo_grid_count)); VL_CUDA(cudaFuncGetAttributes(&fa_, lo_grid_alloc)); VL_CUDA(cudaFuncGetAttributes(&fa_, lo_grid_fill));
   VL_CUDA(cudaFuncGetAttributes(&fa_, lo_assoc_grid<false>)); VL_CUDA(cudaFuncGetAttributes(&fa_, lo_assoc_grid<true>));
   VL_CUDA(cudaFuncGetAttributes(&fa_, lo_assoc_grid_both)); VL_CUDA(cudaFuncGetAttributes(&fa_, lo_accumulate));
-  VL_CUDA(cudaFuncGetAttributes(&fa_, lo_set_prior));
+  VL_CUDA(cudaFuncGetAttributes(&fa_, lo_set_prior)); VL_CUDA(cudaFuncGetAttributes(&fa_, lo_transform_to_end));
   return VLOAM_OK;
 }
 
@@ -698,6 +735,7 @@ static int lo_queue_solve(vloam_b200_ctx* c, const double* prior_q, const double
                           c->nSharp + c->nFlat, vl_distortion(c) ? c->factorS.p : nullptr, 8));
     }
     VL_LAUNCH(lo_accumulate, 1, 32, 0, c->los);
+    if (vl_to_end(c)) VL_TRY(lo_queue_to_end(c));  // LO.cpp:537-556, before the swap: evLoSolve / evLoNext cover it
   VL_CUDA(cudaEventRecord(c->evLoSolve, VL_STREAM(c)));
   return VLOAM_OK;
 }
@@ -718,7 +756,8 @@ static bool lo_lookahead_possible(const vloam_b200_ctx* c) {
 static int lo_lookahead_waits(vloam_b200_ctx* c) {
   VL_CUDA(cudaStreamWaitEvent(c->streamLO, c->evLoSolve, 0));
   VL_CUDA(cudaStreamWaitEvent(c->streamLO, c->evLast, 0));
-  VL_CUDA(cudaStreamWaitEvent(c->streamLO, c->srNext->evSRfeat, 0));  // (sharp + flat of the next sweep: not its per-ring voxel filter)
+  // (sharp + flat of the next sweep: not its per-ring voxel filter -- unless its TransformToEnd reads the less-flat cloud as well)
+  VL_CUDA(cudaStreamWaitEvent(c->streamLO, vl_to_end(c) ? c->srNext->evSR : c->srNext->evSRfeat, 0));
   return VLOAM_OK;
 }
 int vl_lo_lookahead_solve(vloam_b200_ctx* c, bool flush, bool waitsIssued) {
@@ -758,7 +797,9 @@ int vl_lo_lookahead_stacks(vloam_b200_ctx* c) {
   static const bool noStacksNext = getenv("VLOAM_NO_STACKS_LOOKAHEAD") != nullptr;
   bool srDone = false;
   int r = VLOAM_OK;
-  if (mapNext && !noStacksNext) {
+  // Under VLOAM_FLAG_TRANSFORM_TO_END the next sweep's stacks come from its end clouds, i.e. from the look-ahead solve queued just
+  // now, which may still be discarded: they are filtered in the plain order, after that solve is adopted (vl_lo_run).
+  if (mapNext && !noStacksNext && !vl_to_end(c)) {
     for (;;) {
       cudaError_t e = cudaEventQuery(c->srNext->evSR);
       if (e == cudaSuccess) { srDone = true; break; }
@@ -825,7 +866,9 @@ int vl_lo_side_work(vloam_b200_ctx* c) {
 int vl_lo_plan_prebuild(vloam_b200_ctx* c) {
   c->preDeferred = false;
   static const bool off = getenv("VLOAM_NO_PREBUILD") != nullptr;
-  if (off || !c->srNextValid || c->loPreValid || cudaEventQuery(c->srNext->evSR) != cudaSuccess) { (void)cudaGetLastError(); return VLOAM_OK; }
+  // (under VLOAM_FLAG_TRANSFORM_TO_END the next sweep's "last" clouds are its end clouds, which do not exist before its own
+  // odometry solve: nothing to pre-build, its structures are built in the plain order)
+  if (off || vl_to_end(c) || !c->srNextValid || c->loPreValid || cudaEventQuery(c->srNext->evSR) != cudaSuccess) { (void)cudaGetLastError(); return VLOAM_OK; }
   vl_sr_swap(c, *c->srNext);
   const int r = vl_sr_sync_counts(c);
   c->preCorner = c->lessSharp[c->cur].p; c->preNc = c->nLessSharp; c->preSurf = c->lessFlat[c->cur].p; c->preNs = c->nLessFlat;
@@ -881,7 +924,9 @@ int vl_lo_run(vloam_b200_ctx* c, const double* prior_q, const double* prior_t, i
     c->stacksNextReady = false;
     if (c->srAdopted && mapThisFrame) { VL_TRY(vl_sr_sync_counts(c)); VL_TRY(vl_lm_adopt_stacks_next(c)); stacksQueued = true; c->stacksAdopted = true; }
   }
-  if (!stacksQueued && early && mapThisFrame && cudaEventQuery(c->evSR) == cudaSuccess) {
+  const bool toEnd = vl_to_end(c);
+  // (under VLOAM_FLAG_TRANSFORM_TO_END the stacks are filtered from the end clouds: queued below, once this sweep's solve is)
+  if (!toEnd && !stacksQueued && early && mapThisFrame && cudaEventQuery(c->evSR) == cudaSuccess) {
     VL_TRY(vl_sr_sync_counts(c));
     VL_TRY(vl_lm_enqueue_stacks(c, c->lessSharp[c->cur].p, c->nLessSharp, c->lessFlat[c->cur].p, c->nLessFlat, true));
     stacksQueued = true;
@@ -892,6 +937,22 @@ int vl_lo_run(vloam_b200_ctx* c, const double* prior_q, const double* prior_t, i
   c->loNextValid = false;
   if (adoptLO) { LoScalars* t_ = c->los; c->los = c->losNext; c->losNext = t_; }
   else if (c->lo_inited) VL_TRY(lo_queue_solve(c, prior_q, prior_t, use_prior));  // LO.cpp:209-217: the first frame only initialises
+  else if (toEnd) {  // ... but LO.cpp:537-556 runs on it too, with q_last_curr = identity, t_last_curr = 0
+    VL_TRY(lo_queue_to_end(c));
+    VL_CUDA(cudaEventRecord(c->evLoSolve, VL_STREAM(c)));
+  }
+  // this sweep's clouds as LaserOdometry hands them on: in the sweep-end frame under the flag (the main stream is behind the
+  // transform here: queued above, or waited for through evLoNext when the look-ahead solve was adopted)
+  const float4* outCorner = toEnd ? c->endSharp[c->cur].p : c->lessSharp[c->cur].p;
+  const float4* outSurf = toEnd ? c->endFlat[c->cur].p : c->lessFlat[c->cur].p;
+  if (toEnd) {
+    VL_CUDA(cudaEventRecord(c->evEnd, c->stream));
+    if (early && mapThisFrame && cudaEventQuery(c->evSR) == cudaSuccess) {
+      VL_TRY(vl_sr_sync_counts(c));
+      VL_TRY(vl_lm_enqueue_stacks(c, outCorner, c->nLessSharp, outSurf, c->nLessFlat, true));
+      stacksQueued = true;
+    }
+  }
   // With the solve adopted, the stacks queued and the mapping stage following in the same call, nothing on the pose
   // chain depends on the search structures of the next "last" clouds: they are queued by the mapping stage right after
   // its own launches (vl_lo_flush_deferred).
@@ -905,7 +966,7 @@ int vl_lo_run(vloam_b200_ctx* c, const double* prior_q, const double* prior_t, i
   VL_HOST_MARK(2);
   VL_TRY(vl_sr_sync_counts(c));  // sync point S1 (event after scan registration; the odometry above is already queued)
   if (mapThisFrame && !stacksQueued)
-    VL_TRY(vl_lm_enqueue_stacks(c, c->lessSharp[c->cur].p, c->nLessSharp, c->lessFlat[c->cur].p, c->nLessFlat));
+    VL_TRY(vl_lm_enqueue_stacks(c, outCorner, c->nLessSharp, outSurf, c->nLessFlat));
   // built during the previous sweep (two sweeps registered ahead)?
   const bool preHit = c->loPreValid && c->srAdopted && c->preSet == (c->lastSet ^ 1) && c->preCorner == c->lessSharp[c->cur].p && c->preNc == c->nLessSharp &&
                       c->preSurf == c->lessFlat[c->cur].p && c->preNs == c->nLessFlat && c->loGridValid[c->lastSet ^ 1];
@@ -914,12 +975,12 @@ int vl_lo_run(vloam_b200_ctx* c, const double* prior_q, const double* prior_t, i
     // nothing to build: evLast was recorded behind that build
   } else if (defer) {
     c->loDeferred = true; c->defSet = c->lastSet ^ 1;
-    c->defCorner = c->lessSharp[c->cur].p; c->defNc = c->nLessSharp; c->defSurf = c->lessFlat[c->cur].p; c->defNs = c->nLessFlat;
+    c->defCorner = outCorner; c->defNc = c->nLessSharp; c->defSurf = outSurf; c->defNs = c->nLessFlat;
   } else {  // LO.cpp:573-574 (setInputCloud on both KD-trees) for the clouds that become "last" after this solve:
      // they are this frame's less-sharp / less-flat clouds, final since scan registration, so the side
-     // stream builds them while the odometry still searches the previous set
+     // stream builds them while the odometry still searches the previous set (end clouds: behind this solve, evLoSolve)
     vl_tls_stream = c->stream2;
-    const int r = vl_lo_build_last(c, c->lastSet ^ 1, c->lessSharp[c->cur].p, c->nLessSharp, c->lessFlat[c->cur].p, c->nLessFlat);
+    const int r = vl_lo_build_last(c, c->lastSet ^ 1, outCorner, c->nLessSharp, outSurf, c->nLessFlat);
     vl_tls_stream = nullptr;
     if (r != VLOAM_OK) return r;
     VL_CUDA(cudaEventRecord(c->evLast, c->stream2));
@@ -927,7 +988,7 @@ int vl_lo_run(vloam_b200_ctx* c, const double* prior_q, const double* prior_t, i
   }
   c->lo_inited = true;
   // LO.cpp:558-574: this frame's less-sharp / less-flat clouds become the "last" clouds
-  c->cornerLastPtr = c->lessSharp[c->cur].p; c->surfLastPtr = c->lessFlat[c->cur].p;
+  c->cornerLastPtr = const_cast<float4*>(outCorner); c->surfLastPtr = const_cast<float4*>(outSurf);
   c->nCornerLast = c->nLessSharp; c->nSurfLast = c->nLessFlat;
   c->lastSet ^= 1;
   c->lo_frameCount++;

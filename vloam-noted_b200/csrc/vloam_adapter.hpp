@@ -113,6 +113,7 @@ public:
     const char* dev = getenv("VLOAM_B200_DEVICE");
     create(p, dev ? atoi(dev) : 0);
   }
+  // explicit parameters, e.g. p.reserved = VLOAM_FLAG_DISTORTION | VLOAM_FLAG_TRANSFORM_TO_END for sweeps that are not motion-compensated
   explicit Engine(const vloam_b200_params& p, int device = 0) { create(p, device); }
   ~Engine() { vloam_b200_destroy(ctx_); }
   Engine(const Engine&) = delete;
@@ -156,7 +157,7 @@ private:
     if (r != VLOAM_OK) throw AdapterError("vloam_b200_create failed (bad scan_line / resolution or no CUDA device): " + std::to_string(r));
   }
   vloam_b200_ctx* ctx_ = nullptr;
-  Sig sig_[7];
+  Sig sig_[8];
   std::vector<float> buf_;
 };
 
@@ -270,7 +271,7 @@ public:
     skip_frame = skip_ != 0;
     if (!skip_frame) {  // "no change if skip_frame"
       if (fresh_) {
-        e_->fetch(VLOAM_CLOUD_CORNER_LAST, laserCloudCornerLast); e_->fetch(VLOAM_CLOUD_SURF_LAST, laserCloudSurfLast); e_->fetch(VLOAM_CLOUD_FULL, laserCloudFullRes);
+        e_->fetch(VLOAM_CLOUD_CORNER_LAST, laserCloudCornerLast); e_->fetch(VLOAM_CLOUD_SURF_LAST, laserCloudSurfLast); e_->fetch(VLOAM_CLOUD_FULL_RES, laserCloudFullRes);
         fresh_ = false;
       }
       laserCloudCornerLast_ = laserCloudCornerLast; laserCloudSurfLast_ = laserCloudSurfLast; laserCloudFullRes_ = laserCloudFullRes;
@@ -328,7 +329,7 @@ public:
     for (int k = 0; k < 3; ++k) if (t[k] != e_->t_wodom[k]) throw AdapterError("input(): t_wodom_curr is not the pose LaserOdometry::output returned");
     if (!skip_frame) {
       e_->expect(VLOAM_CLOUD_CORNER_LAST, laserCloudCornerLast_, "laserCloudCornerLast"); e_->expect(VLOAM_CLOUD_SURF_LAST, laserCloudSurfLast_, "laserCloudSurfLast");
-      e_->expect(VLOAM_CLOUD_FULL, laserCloudFullRes_, "laserCloudFullRes");
+      e_->expect(VLOAM_CLOUD_FULL_RES, laserCloudFullRes_, "laserCloudFullRes");
     } else {
       e_->check(vloam_b200_laser_mapping(e_->ctx(), q_, t_));  // propagates q_wmap_wodom * odometry only
     }

@@ -25,6 +25,9 @@ def lib():
         L.vloam_synth_scan.restype = ctypes.c_int
         L.vloam_synth_scan.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_double,
                                        ctypes.c_double, ctypes.c_double, ctypes.c_int, ctypes.c_double, ctypes.c_void_p, ctypes.c_int]
+        L.vloam_synth_scan_moving.restype = ctypes.c_int
+        L.vloam_synth_scan_moving.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_double,
+                                              ctypes.c_double, ctypes.c_double, ctypes.c_int, ctypes.c_double, ctypes.c_void_p, ctypes.c_int]
         L.vloam_synth_plant.restype = ctypes.c_int
         L.vloam_synth_plant.argtypes = [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_int, ctypes.c_double, ctypes.c_double,
                                         ctypes.c_double, ctypes.c_double, ctypes.c_double, ctypes.c_double, ctypes.c_void_p, ctypes.c_int]
@@ -51,6 +54,20 @@ class World:
         p = np.ascontiguousarray(pose, np.float64)
         n = lib().vloam_synth_scan(self.h, sensor, p.ctypes.data, seed, range_sigma, nan_frac, max_range, order, az0,
                                    out.ctypes.data, cap)
+        assert n >= 0
+        return out[:n].copy()
+
+    def scan_moving(self, sensor, pose_start, pose_end, seed, range_sigma=0.02, nan_frac=0.01, max_range=120.0, order=0, az0=-3.1):
+        """One sweep from a sensor moving from pose_start to pose_end (x,y,z,yaw,pitch,roll) during the sweep, not motion-compensated:
+        azimuth column k of n_az is cast from the pose at fraction k / n_az (translation linear, rotation slerp) -- the order in which
+        ScanRegistration's relTime grows (SR.cpp:183-298) -- and its points are in the sensor frame of that instant.
+        pose_start == pose_end reproduces scan(pose_start) byte for byte."""
+        cap = 300000
+        out = np.empty((cap, 4), np.float32)
+        p0 = np.ascontiguousarray(pose_start, np.float64)
+        p1 = np.ascontiguousarray(pose_end, np.float64)
+        n = lib().vloam_synth_scan_moving(self.h, sensor, p0.ctypes.data, p1.ctypes.data, seed, range_sigma, nan_frac, max_range, order, az0,
+                                          out.ctypes.data, cap)
         assert n >= 0
         return out[:n].copy()
 

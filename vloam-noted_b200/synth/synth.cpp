@@ -111,6 +111,33 @@ void euler_to_R(double yaw, double pitch, double roll, double R[9]) {
   R[6] = -sp;     R[7] = cp * sr;                R[8] = cp * cr;
 }
 
+// ZYX Euler angles -> quaternion {x, y, z, w} of R = Rz(yaw) Ry(pitch) Rx(roll) (the rotation euler_to_R builds)
+void euler_to_q(double yaw, double pitch, double roll, double q[4]) {
+  const double cy = cos(yaw * 0.5), sy = sin(yaw * 0.5), cp = cos(pitch * 0.5), sp = sin(pitch * 0.5), cr = cos(roll * 0.5), sr = sin(roll * 0.5);
+  q[0] = sr * cp * cy - cr * sp * sy; q[1] = cr * sp * cy + sr * cp * sy; q[2] = cr * cp * sy - sr * sp * cy; q[3] = cr * cp * cy + sr * sp * sy;
+}
+void q_to_R(const double q[4], double R[9]) {
+  const double x = q[0], y = q[1], z = q[2], w = q[3];
+  R[0] = 1 - 2 * (y * y + z * z); R[1] = 2 * (x * y - z * w);     R[2] = 2 * (x * z + y * w);
+  R[3] = 2 * (x * y + z * w);     R[4] = 1 - 2 * (x * x + z * z); R[5] = 2 * (y * z - x * w);
+  R[6] = 2 * (x * z - y * w);     R[7] = 2 * (y * z + x * w);     R[8] = 1 - 2 * (x * x + y * y);
+}
+// sensor pose at sweep fraction f in [0, 1] between pose0 and pose1: translation linear, rotation slerp (shortest arc)
+void interp_pose(const double* p0, const double* p1, double f, double o[3], double R[9]) {
+  for (int a = 0; a < 3; ++a) o[a] = p0[a] + f * (p1[a] - p0[a]);
+  double q0[4], q1[4];
+  euler_to_q(p0[3], p0[4], p0[5], q0); euler_to_q(p1[3], p1[4], p1[5], q1);
+  double d = q0[0] * q1[0] + q0[1] * q1[1] + q0[2] * q1[2] + q0[3] * q1[3];
+  if (d < 0) { d = -d; for (int k = 0; k < 4; ++k) q1[k] = -q1[k]; }
+  double s0 = 1 - f, s1 = f;
+  if (d < 1 - 1e-12) { const double th = acos(d), st = sin(th); s0 = sin((1 - f) * th) / st; s1 = sin(f * th) / st; }
+  double q[4], n = 0;
+  for (int k = 0; k < 4; ++k) { q[k] = s0 * q0[k] + s1 * q1[k]; n += q[k] * q[k]; }
+  n = sqrt(n);
+  for (int k = 0; k < 4; ++k) q[k] /= n;
+  q_to_R(q, R);
+}
+
 int beam_table(int sensor, std::vector<double>& elev, int* n_az) {
   elev.clear();
   if (sensor == 0) { for (int i = 0; i < 16; ++i) elev.push_back(-15.0 + 2.0 * i); *n_az = 1800; }
@@ -156,17 +183,23 @@ void* vloam_synth_world_create(uint64_t seed, int kind, double extent) {
 }
 void vloam_synth_world_destroy(void* w) { delete (World*)w; }
 
-// One sweep from pose {x,y,z,yaw,pitch,roll} (world frame).  Writes float32[n][4]
-// (x,y,z,0) in the SENSOR frame; returns n.  order: 0 azimuth-major, 1 ring-major.
-// nan_frac of returns become NaN; returns past max_range are dropped.
-int vloam_synth_scan(void* wv, int sensor, const double* pose, uint64_t seed, double range_sigma, double nan_frac,
+// One sweep; pose1 == nullptr: from the fixed pose {x,y,z,yaw,pitch,roll} (world frame), otherwise azimuth column ia is cast
+// from the pose interpolated between pose0 and pose1 at its emission fraction ia / n_az.
+static int scan_impl(void* wv, int sensor, const double* pose, const double* pose1, uint64_t seed, double range_sigma, double nan_frac,
                      double max_range, int order, double az0, float* out, int cap) {
   const World* w = (const World*)wv;
   std::vector<double> elev; int n_az;
   const int nb = beam_table(sensor, elev, &n_az);
   if (nb < 0) return -1;
   double R[9]; euler_to_R(pose[3], pose[4], pose[5], R);
-  const double o[3] = {pose[0], pose[1], pose[2]};
+  double o[3] = {pose[0], pose[1], pose[2]};
+  // per-column poses of a moving sensor (the columns follow the rotation sense ori = -atan2(y, x) of the emission loop below,
+  // the sense ScanRegistration's relTime assumes, SR.cpp:183-298)
+  std::vector<double> colO, colR;
+  if (pose1) {
+    colO.resize((size_t)n_az * 3); colR.resize((size_t)n_az * 9);
+    for (int ia = 0; ia < n_az; ++ia) interp_pose(pose, pose1, (double)ia / n_az, &colO[(size_t)ia * 3], &colR[(size_t)ia * 9]);
+  }
   Rng rng(seed);
   int n = 0;
   const int outer = order == 0 ? n_az : nb, inner = order == 0 ? nb : n_az;
@@ -177,6 +210,7 @@ int vloam_synth_scan(void* wv, int sensor, const double* pose, uint64_t seed, do
       const double az = -(az0 + 6.283185307179586 * ia / n_az);
       const double el = (elev[ib] + 0.03 * rng.gauss()) * 0.017453292519943295;
       const double ds[3] = {cos(el) * cos(az), cos(el) * sin(az), sin(el)};
+      if (pose1) { memcpy(o, &colO[(size_t)ia * 3], sizeof o); memcpy(R, &colR[(size_t)ia * 9], sizeof R); }
       const double d[3] = {R[0] * ds[0] + R[1] * ds[1] + R[2] * ds[2], R[3] * ds[0] + R[4] * ds[1] + R[5] * ds[2],
                            R[6] * ds[0] + R[7] * ds[1] + R[8] * ds[2]};
       const double u_nan = rng.uni(), noise = rng.gauss();
@@ -190,6 +224,23 @@ int vloam_synth_scan(void* wv, int sensor, const double* pose, uint64_t seed, do
       ++n;
     }
   return n;
+}
+
+// One sweep from pose {x,y,z,yaw,pitch,roll} (world frame).  Writes float32[n][4]
+// (x,y,z,0) in the SENSOR frame; returns n.  order: 0 azimuth-major, 1 ring-major.
+// nan_frac of returns become NaN; returns past max_range are dropped.
+int vloam_synth_scan(void* wv, int sensor, const double* pose, uint64_t seed, double range_sigma, double nan_frac,
+                     double max_range, int order, double az0, float* out, int cap) {
+  return scan_impl(wv, sensor, pose, nullptr, seed, range_sigma, nan_frac, max_range, order, az0, out, cap);
+}
+// The same sweep from a MOVING sensor: azimuth column ia is cast from the pose at fraction ia / n_az between pose_start and
+// pose_end (translation linear, rotation slerp) and its points are written in the sensor frame of that instant -- a sweep that
+// is not motion-compensated.  With the only difference to vloam_synth_scan being those per-column poses, pose_start == pose_end
+// gives exactly vloam_synth_scan(pose_start) (the fixed-pose path is taken then).
+int vloam_synth_scan_moving(void* wv, int sensor, const double* pose_start, const double* pose_end, uint64_t seed, double range_sigma,
+                            double nan_frac, double max_range, int order, double az0, float* out, int cap) {
+  const bool still = memcmp(pose_start, pose_end, 6 * sizeof(double)) == 0;
+  return scan_impl(wv, sensor, pose_start, still ? nullptr : pose_end, seed, range_sigma, nan_frac, max_range, order, az0, out, cap);
 }
 
 // Plant map points on the world's surfaces inside [cx-hw,cx+hw] x [cy-hw,cy+hw] x [zlo,zhi]:
