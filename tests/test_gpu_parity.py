@@ -632,15 +632,15 @@ def test_speculative_submap_equals_inline_build(pkg, op, synth, street):
     frame k used; lm_prepare lets the in-line build run instead when the window moved.  A 28 m drive (the
     centre cube changes at x = 25 m), a mapping_skip_frame = 2 run and a run whose map offset is edited from
     outside so that the window moves two frames later must give bit-identical poses and maps with the
-    speculation switched off (VLOAM_NO_SPECULATION); the long drive is also checked against the oracle."""
+    speculation switched off (VLOAM_NO_GRID); the long drive is also checked against the oracle."""
     import os
     def run(spec, kw, sensor, poses, check_oracle, shift_after=None):
-        if spec: os.environ.pop("VLOAM_NO_SPECULATION", None)
-        else: os.environ["VLOAM_NO_SPECULATION"] = "1"
+        if spec: os.environ.pop("VLOAM_NO_GRID", None)
+        else: os.environ["VLOAM_NO_GRID"] = "1"
         try:
             g = pkg.Context(**kw)
         finally:
-            os.environ.pop("VLOAM_NO_SPECULATION", None)
+            os.environ.pop("VLOAM_NO_GRID", None)
         o = op.Oracle(**kw) if check_oracle else None
         out, centres = [], []
         for k, p in enumerate(poses):

@@ -187,7 +187,6 @@ void vloam_b200_destroy(vloam_b200_ctx* c) {
   if (c->srNext2) { vl_sr_swap(c, *c->srNext2); free_sr_set(c); delete c->srNext2; c->srNext2 = nullptr; }
   cudaStreamDestroy(c->streamSR);
   vl_lm_free(c);
-  vl_scan_free(&c->loScan[0]); vl_scan_free(&c->loScan[1]);
   if (c->streamLO) { cudaStreamSynchronize(c->streamLO); cudaStreamDestroy(c->streamLO); }
   cudaEventDestroy(c->evS2); cudaEventDestroy(c->evLoSolve); cudaEventDestroy(c->evLoNext); if (c->evEnd) cudaEventDestroy(c->evEnd);
   void* singles[] = {c->los, c->losNext, c->evalOut, c->lms, c->lmm, c->cubeC, c->cubeS, c->vScalars, c->loRingTbl, c->loGridCells[0].p, c->loGridCells[1].p,
@@ -197,7 +196,7 @@ void vloam_b200_destroy(vloam_b200_ctx* c) {
                      c->dbgKnnOk[1][1].p};
   for (void* p : singles) vl_dev_free(c, p);
   void* bufs[] = {c->lessSharp[0].p, c->lessSharp[1].p, c->lessSharp[2].p, c->lessFlat[0].p, c->lessFlat[1].p, c->lessFlat[2].p, c->endSharp[0].p, c->endSharp[1].p, c->endSharp[2].p, c->endFlat[0].p, c->endFlat[1].p, c->endFlat[2].p, c->loCornerIdx.p, c->loSurfIdx.p, c->factors.p, c->factorS.p, c->factorValid.p, c->loFactors.p, c->loFactorValid.p, c->evalPartials.p,
-                  c->poolC.p, c->poolS.p, c->stackC.p, c->stackS.p, c->stackCN.p, c->stackSN.p, c->fromMapC.p, c->fromMapS.p, c->knnIdx.p, c->knnD2.p, c->knnOk.p,
+                  c->poolC.p, c->poolS.p, c->stackC.p, c->stackS.p, c->stackCN.p, c->stackSN.p, c->fromMapC.p, c->fromMapS.p, c->knnD2.p, c->knnOk.p,
                   c->vKeys.p, c->vKeys2.p, c->vHead.p, c->vScan.p, c->vScan2.p, c->vOut.p, c->vIn.p, c->regOut.p, c->tailKeys.p, c->staging.p};
   for (void* p : bufs) vl_dev_free(c, p);
   if (c->h_s2flag) cudaFreeHost(c->h_s2flag);

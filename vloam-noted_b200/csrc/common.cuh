@@ -99,9 +99,6 @@ extern thread_local cudaStream_t vl_tls_stream;
 #define VL_STREAM(c) (vl_tls_stream ? vl_tls_stream : (c)->stream)
 struct VlWorker;
 
-// status words of one single-launch scan: tiles x (epoch | status | value) and the tile ticket counter
-struct VlScan { unsigned long long* state = nullptr; int tiles = 0; unsigned epoch = 0; };
-
 struct vloam_b200_ctx {
   vloam_b200_params prm;
   int device;
@@ -204,7 +201,6 @@ struct vloam_b200_ctx {
   // search structures over the "last" clouds, double-buffered: set [lastSet] serves this frame's odometry
   // while the side stream builds set [lastSet ^ 1] from this frame's clouds
   int* loRingTbl;                     // 2 sets x 2 clouds x (144 + 1) ints: ring-value -> first index tables
-  VlScan loScan[2];
   DBuf<int> loGridCells[2], loGridCellOf; DBuf<float4> loGridSorted[2]; bool loGridValid[2]; int loGridMask[2];  // hash of occupied 1.28 m cells per set
   int lastSet;
   DBuf<int> loCornerIdx, loSurfIdx;   // association results (2 / 3 ints per query)
@@ -229,11 +225,11 @@ struct vloam_b200_ctx {
   DBuf<float4> fromMapC, fromMapS;
   int lm_frameCount;
   int lm_optimized;  // host copy: did the last solveMapping run the optimisation (LM.cpp:514)
-  DBuf<int> knnIdx; DBuf<float> knnD2; DBuf<int> knnOk;
+  DBuf<float> knnD2; DBuf<int> knnOk;
   DBuf<float4> knnPts; DBuf<unsigned long long> knnKey;  // the five neighbours themselves (the grid has no stable point ids) and their keys (debug capture)
   DBuf<int> dbgKnnIdx[2][2]; DBuf<float> dbgKnnD2[2][2]; DBuf<int> dbgKnnOk[2][2];
   double dbgLmCost[4];
-  struct GridParams* gridPrm;  // device [2]
+  struct LmDevice* lm;  // the mapping stage's own state (laser_mapping.cu: vl_lm_init)
   // voxel filter scratch
   DBuf<unsigned long long> vKeys, vKeys2; DBuf<int> vHead; DBuf<int> vScan, vScan2;  // two scratch lanes: the corner and surf filters run concurrently
   DBuf<float4> vOut; DBuf<float4> vIn;
@@ -274,14 +270,6 @@ static inline void vl_sr_swap(vloam_b200_ctx* c, SrSet& s) {
   VL_SR_FIELDS(VL_X)
 #undef VL_X
 }
-
-struct GridParams {
-  float ox, oy, oz;   // origin (min corner)
-  float inv;          // 1 / cell
-  int nx, ny, nz;
-  int ncell;
-  int npoints;
-};
 
 // ---- error handling ---------------------------------------------------------
 #define VL_CUDA(call)                                                                     \
@@ -410,12 +398,11 @@ int vl_sr_set_attrs(vloam_b200_ctx* c);
 int vl_sort_set_attrs(vloam_b200_ctx* c);
 int vl_solver_set_attrs(vloam_b200_ctx* c);
 int vl_lo_preload(vloam_b200_ctx* c);
-int vl_lo_lookahead(vloam_b200_ctx* c);
 int vl_lo_lookahead_solve(vloam_b200_ctx* c, bool flush = true, bool waitsIssued = false);   // part 1: queue the next sweep's odometry solve on its own stream (flush: issue the deferred side work first)
 int vl_lo_plan_prebuild(vloam_b200_ctx* c);     // two sweeps ahead: plan the build of the next sweep's search structures as part of this call's side work
 int vl_lo_early_lookahead(vloam_b200_ctx* c, bool* armed);  // ... and queue the next sweep's odometry before this sweep's mapping when its structures are pre-built
 int vl_lo_lookahead_stacks(vloam_b200_ctx* c);  // part 2 (after S2 is recorded): the next sweep's stack filters, if its scan registration is done
-int vl_lo_flush_deferred(vloam_b200_ctx* c);  // queue the deferred side-stream work of the last odometry call (look-ahead scan registration, next search structures)  // queue the NEXT sweep's odometry solve behind this sweep's mapping (no-op unless its scan registration is in flight)
+int vl_lo_flush_deferred(vloam_b200_ctx* c);  // queue the deferred side-stream work of the last odometry call (look-ahead scan registration, next search structures)
 int vl_vg_preload(vloam_b200_ctx* c);
 int vl_lm_preload(vloam_b200_ctx* c);
 int vl_lm_register_full(vloam_b200_ctx* c, const float4* d_in, int n, float4* d_out);
@@ -429,11 +416,6 @@ int vl_lm_export_map(vloam_b200_ctx* c, int which, void* out, long cap, long* by
 int vl_lm_sync_pools(vloam_b200_ctx* c);  // write the in-place grid updates back to the cube pools (no-op when they are current)
 int vl_lm_import_map(vloam_b200_ctx* c, int which, const void* data, long bytes);
 
-// out[0..n] = exclusive scan of in[0..n) in ONE launch (chained scan with look-back, laser_mapping.cu).  `in` and `out`
-// must be 16-byte aligned; d_skip: device flag, non-zero = do nothing.  A VlScan holds the per-tile status words.
-int vl_scan_alloc(VlScan* sc, int n);
-void vl_scan_free(VlScan* sc);
-int vl_scan_exclusive(vloam_b200_ctx* c, const int* in, int n, VlScan* sc, int* out, const int* d_skip = nullptr);
 // sort / voxel primitives (voxel_grid.cu)
 int vl_sort_u64(vloam_b200_ctx* c, unsigned long long* d_keys, int n_pow2);
 // pcl::VoxelGrid of d_in[0..n) -> d_out, count written to *d_count (device int); n is a host bound,

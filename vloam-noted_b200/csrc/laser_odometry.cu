@@ -822,10 +822,6 @@ int vl_lo_lookahead_stacks(vloam_b200_ctx* c) {
   c->loNextValid = true;
   return VLOAM_OK;
 }
-int vl_lo_lookahead(vloam_b200_ctx* c) {
-  VL_TRY(vl_lo_lookahead_solve(c, true));
-  return vl_lo_lookahead_stacks(c);
-}
 
 // The side-stream work a look-ahead replay defers out of the odometry call: the registered next sweep's upload + scan
 // registration (streamSR) and the search structures over this sweep's clouds (stream2).  Thread-agnostic: the helper thread runs it
@@ -931,7 +927,7 @@ int vl_lo_run(vloam_b200_ctx* c, const double* prior_q, const double* prior_t, i
     VL_TRY(vl_lm_enqueue_stacks(c, c->lessSharp[c->cur].p, c->nLessSharp, c->lessFlat[c->cur].p, c->nLessFlat, true));
     stacksQueued = true;
   }
-  // The solve of this sweep was queued behind the previous sweep's mapping (vl_lo_lookahead) into the spare state:
+  // The solve of this sweep was queued behind the previous sweep's mapping (vl_lo_lookahead_solve) into the spare state:
   // adopting it is a pointer swap.  Anything that could make it stale clears loNextValid.
   const bool adoptLO = c->loNextValid && c->srAdopted && !use_prior && early && c->lo_inited && c->loNextSet == set;  // (early: grid valid, both flags set, no capture)
   c->loNextValid = false;
@@ -956,11 +952,7 @@ int vl_lo_run(vloam_b200_ctx* c, const double* prior_q, const double* prior_t, i
   // With the solve adopted, the stacks queued and the mapping stage following in the same call, nothing on the pose
   // chain depends on the search structures of the next "last" clouds: they are queued by the mapping stage right after
   // its own launches (vl_lo_flush_deferred).
-  // (round 1 queued them after the mapping launches to keep the main stream's launch latency low; now the look-ahead odometry of the
-  // NEXT sweep runs beside this sweep's mapping and waits for exactly these structures, while the mapping itself waits for the previous
-  // map update anyway: they are issued at once.  VLOAM_DEFER_LO_GRIDS=1 restores the old order.)
-  static const bool noSide = getenv("VLOAM_NO_SIDE_DEFER") != nullptr;
-  const bool defer = !noSide && adoptLO && stacksQueued && c->inProcessFrame && mapThisFrame;
+  const bool defer = adoptLO && stacksQueued && c->inProcessFrame && mapThisFrame;
   if (defer) c->srDeferred = c->srPendCount > 0;  // ... and so is the next sweep's scan registration: the helper thread issues both while the caller queues the mapping
   else VL_TRY(vl_launch_lookahead(c));  // the next sweep's scan registration, if one is registered, goes to its side stream now
   VL_HOST_MARK(2);

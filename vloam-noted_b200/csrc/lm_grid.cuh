@@ -89,6 +89,29 @@ __device__ __forceinline__ int lg_insert(const LgGrid& g, int cell, const float4
   return e;
 }
 
+// entry key: (valid slot << 32) | voxel key, or | (LG_TAIL | position in the cube) for an unfiltered tail point
+__device__ __forceinline__ unsigned long long lg_key(int slot, unsigned low) { return ((unsigned long long)slot << 32) | low; }
+__device__ __forceinline__ int lg_key_slot(unsigned long long key) { return (int)(key >> 32); }
+__device__ __forceinline__ unsigned lg_key_vox(unsigned long long key) { return (unsigned)key & 0x3fffffffu; }
+
+// Every live entry of both kinds' cells (ncell per kind), one cell per thread of a grid-stride loop: f(entry, key, kind).
+template <typename F>
+__device__ __forceinline__ void lg_for_each_live(const LgGrid& g, int ncell, F f) {
+  for (int cell = blockIdx.x * blockDim.x + threadIdx.x; cell < 2 * ncell; cell += gridDim.x * blockDim.x) {
+    const int2 d = g.dir[cell];
+    const int kind = cell >= ncell;
+    int chunk = d.y;
+    for (int left = d.x; left > 0; left -= LG_C, chunk = left > 0 ? g.next[chunk] : -1) {
+      const int m = min(left, LG_C);
+      for (int i = 0; i < m; ++i) {
+        const int e = chunk * LG_C + i;
+        const unsigned long long key = g.key[e];
+        if (key != LG_DEAD) f(e, key, kind);
+      }
+    }
+  }
+}
+
 // key order == canonical id order; refs < 0 (empty list slot) sort last
 __device__ __forceinline__ bool lg_key_less(const LgGrid& g, int a, int b) {
   if (b < 0) return a >= 0;

@@ -908,9 +908,8 @@ int vl_sr_run(vloam_b200_ctx* c, const float* d_xyz, int n, int stride) {
   // One sweep at a time (this run is on the pose chain's stream): the odometry that follows needs nothing of what comes below --
   // the per-ring voxel filter of the less-flat cloud, ~40 us -- so that tail goes to the side stream behind evSRfeat and the
   // odometry starts at once.  Everything that reads the less-flat cloud or the counts waits for evSR anyway (sync point S1, the
-  // stack filters and search structures issued behind it, the getters).  VLOAM_NO_SR_TAIL_ASIDE=1 keeps it on the chain.
-  static const bool noTailAside = getenv("VLOAM_NO_SR_TAIL_ASIDE") != nullptr;
-  const bool tailAside = !noTailAside && vl_tls_stream == nullptr && !c->prof_name[0] && !vl_debug_capture(c);
+  // stack filters and search structures issued behind it, the getters).
+  const bool tailAside = vl_tls_stream == nullptr && !c->prof_name[0] && !vl_debug_capture(c);
   struct TlsRestore { cudaStream_t prev; bool on; ~TlsRestore() { if (on) vl_tls_stream = prev; } } tlsRestore{vl_tls_stream, tailAside};
   if (tailAside) { VL_CUDA(cudaStreamWaitEvent(c->streamSR, c->evSRfeat, 0)); vl_tls_stream = c->streamSR; }
   const size_t voxSmem = (size_t)SR_VOX_CAP * (sizeof(unsigned long long) + sizeof(float4));
