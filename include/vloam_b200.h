@@ -136,10 +136,47 @@ int vloam_b200_laser_odometry(vloam_b200_ctx* c, const double* prior_q, const do
                               int* skip_frame);
 
 /* LaserMapping::input + solveMapping (LM.cpp:178-209, 212-814), fed from the
- * context's own odometry output as LOM.cpp:149-158 does.  Outputs (may be
+ * context's own odometry output as LOM.cpp:149-158 does, or from the caller's
+ * vloam_b200_laser_mapping_input of this frame (below).  Outputs (may be
  * NULL): the mapped pose q_w_curr/t_w_curr (the high-frequency propagated pose
  * on skipped frames, LM.cpp:197-201). */
 int vloam_b200_laser_mapping(vloam_b200_ctx* c, double* q_w_curr, double* t_w_curr);
+
+/* Stage inputs from the caller.  The reference's LaserOdometry::input (LO.cpp:137-148) and LaserMapping::input
+ * (LM.cpp:178-209) deep-copy whatever they are handed; these four calls do the same, so the stages can run on edited clouds
+ * (moving objects removed), behind another odometry (a VO-fused or wheel / INS pose), on recorded odometry output, or as
+ * separate contexts.
+ *
+ * Points: x, y, z at float offsets 0..2 and the intensity at float offset w_offset of records `stride` floats apart
+ * (4, 3 = packed xyzi; 8, 4 = pcl::PointXYZI as PCL lays it out in memory).  Only those four floats are read; the copy moves
+ * bits, so results are bit-identical to the same points produced on the device.
+ * Copies: a host buffer may be reused as soon as the call returns.  Device buffers (the _device variants) are read on the
+ * context's main stream (vloam_b200_stream) in the order of the context's calls.
+ * Validation: VLOAM_E_INVALID with a message for n < 0, NULL with n > 0, stride < 4, w_offset outside [3, stride - 1], a
+ * NULL pose and skip_frame other than 0 / 1.
+ * No cost without them: a context that never makes these calls runs no extra launch, wait or allocation; their buffers are
+ * reserved by the first call.
+ *
+ * Odometry input: the five ScanRegistration clouds in VLOAM_CLOUD_FULL .. VLOAM_CLOUD_LESS_FLAT order replace this frame's
+ * vloam_b200_scan_registration (call it after begin_frame, before vloam_b200_laser_odometry); get_cloud(0..4) then returns
+ * them.  Ring ids are int(intensity); the clouds need not be ring-major.  Under VLOAM_FLAG_TRANSFORM_TO_END they are moved to
+ * the sweep end like scan-registration output.  The call drops every look-ahead registered or computed with
+ * vloam_b200_prefetch_scan, as a scan_registration call with an unregistered buffer does; results stay bit-identical with or
+ * without the look-ahead. */
+int vloam_b200_laser_odometry_input(vloam_b200_ctx* c, const float* const clouds[5], const int n[5], int stride, int w_offset);
+int vloam_b200_laser_odometry_input_device(vloam_b200_ctx* c, const float* const d_clouds[5], const int n[5], int stride, int w_offset);
+/* Mapping input: laserCloudCornerLast, laserCloudSurfLast, laserCloudFullRes, q_wodom_curr (x,y,z,w), t_wodom_curr and
+ * skip_frame, consumed by exactly one vloam_b200_laser_mapping call of this frame (skip_frame = 1: it returns the
+ * high-frequency pose q_wmap_wodom * q_wodom_curr, LM.cpp:197-201).  An input that no mapping call consumes is dropped by the
+ * next begin_frame; without one, laser_mapping reads the context's own odometry output.  The input never touches the
+ * context's odometry (its "last" clouds, its pose, its frame count, the next frame's skip decision): a context may run its
+ * own scan registration and odometry and still map the caller's clouds.  The clouds are used exactly as given (LaserMapping
+ * applies no TransformToEnd), and vloam_b200_register_full_cloud after that mapping call registers the caller's `full`
+ * cloud. */
+int vloam_b200_laser_mapping_input(vloam_b200_ctx* c, const float* corner, int nc, const float* surf, int ns, const float* full, int nfull,
+                                   int stride, int w_offset, const double* q_wodom, const double* t_wodom, int skip_frame);
+int vloam_b200_laser_mapping_input_device(vloam_b200_ctx* c, const float* d_corner, int nc, const float* d_surf, int ns, const float* d_full,
+                                          int nfull, int stride, int w_offset, const double* q_wodom, const double* t_wodom, int skip_frame);
 
 /* The full-resolution cloud of this sweep registered into the map frame: LaserMapping::publish's loop
  * over laserCloudFullRes with pointAssociateToMap (LM.cpp:901-905; q_w_curr / t_w_curr after

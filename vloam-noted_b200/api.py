@@ -18,6 +18,8 @@ EXPORTS = [
     "vloam_b200_stream", "vloam_b200_kernel_launches", "vloam_b200_set_timing", "vloam_b200_stage_ms", "vloam_b200_debug_get",
     "vloam_b200_debug_set", "vloam_b200_profile_kernel", "vloam_b200_profile_result", "vloam_b200_profile_table", "vloam_b200_profile_timeline", "vloam_b200_register_full_cloud", "vloam_b200_lo_associate", "vloam_b200_voxel_grid", "vloam_b200_evaluate", "vloam_b200_solve", "vloam_b200_fit", "vloam_b200_evaluate_deskew", "vloam_b200_solve_deskew", "vloam_b200_exact_math",
     "vloam_b200_publish_map", "vloam_b200_get_map",
+    "vloam_b200_laser_odometry_input", "vloam_b200_laser_odometry_input_device", "vloam_b200_laser_mapping_input",
+    "vloam_b200_laser_mapping_input_device",
 ]
 
 
@@ -81,6 +83,10 @@ def load_lib(build=False):
     L.vloam_b200_exact_math.argtypes = [vp, vp, vp, ci, vp, vp]
     L.vloam_b200_publish_map.argtypes = [vp]
     L.vloam_b200_get_map.argtypes = [vp, vp, ci]
+    for name in ("vloam_b200_laser_odometry_input", "vloam_b200_laser_odometry_input_device"):
+        getattr(L, name).argtypes = [vp, vp, vp, ci, ci]
+    for name in ("vloam_b200_laser_mapping_input", "vloam_b200_laser_mapping_input_device"):
+        getattr(L, name).argtypes = [vp, vp, ci, vp, ci, vp, ci, ci, ci, vp, vp, ci]
     _lib = L
     return L
 
@@ -105,6 +111,35 @@ def _decode(name, raw):
             return np.frombuffer(raw, np.float32).reshape(-1, 5).copy()
         return np.frombuffer(raw, np.int32).copy()
     return np.frombuffer(raw, np.float32).reshape(-1, 4).copy()
+
+
+def _is_cuda_tensor(a):
+    return hasattr(a, "data_ptr") and getattr(a, "is_cuda", False)
+
+
+def _clouds(clouds):
+    """Caller clouds for the stage inputs: all numpy-like float32[n, stride] (host) or all contiguous float32 torch CUDA tensors
+    [n, stride] (device).  Returns (pointers, counts, stride, device, keep-alive)."""
+    dev = [_is_cuda_tensor(a) for a in clouds]
+    if any(dev) and not all(dev):
+        raise ValueError("stage inputs are either all host arrays or all CUDA tensors")
+    if all(dev):
+        import torch
+        for a in clouds:
+            if a.dtype != torch.float32 or a.dim() != 2 or not a.is_contiguous():
+                raise ValueError("device clouds must be contiguous float32[n, stride] CUDA tensors")
+        torch.cuda.current_stream(clouds[0].device).synchronize()  # the context reads them on its own stream
+        arrs, ptrs = clouds, [a.data_ptr() if a.shape[0] else None for a in clouds]
+    else:
+        arrs = [np.ascontiguousarray(a, np.float32) for a in clouds]
+        for a in arrs:
+            if a.ndim != 2:
+                raise ValueError("clouds must be float32[n, stride]")
+        ptrs = [a.ctypes.data if a.shape[0] else None for a in arrs]
+    strides = {int(a.shape[1]) for a in arrs}
+    if len(strides) != 1:
+        raise ValueError("all clouds of one input call share one stride")
+    return ptrs, [int(a.shape[0]) for a in arrs], strides.pop(), all(dev), arrs
 
 
 class Context:
@@ -192,6 +227,29 @@ class Context:
             qw.ctypes.data if want_pose else None, tw.ctypes.data if want_pose else None,
             ql.ctypes.data if want_pose else None, tl.ctypes.data if want_pose else None, ctypes.byref(skip)))
         return {"q_w_curr": qw, "t_w_curr": tw, "q_last_curr": ql, "t_last_curr": tl, "skip_frame": bool(skip.value)}
+
+    def laser_odometry_input(self, clouds, w_offset=3):
+        """LaserOdometry::input (LO.cpp:137-148): the five ScanRegistration clouds (CLOUD_FULL .. CLOUD_LESS_FLAT order) replace this
+        frame's scan registration.  numpy float32[n, stride] arrays, or float32 CUDA tensors through the _device call; the intensity
+        is column w_offset."""
+        if len(clouds) != 5:
+            raise ValueError("laser_odometry_input takes the five ScanRegistration clouds")
+        ptrs, ns, stride, dev, _keep = _clouds(clouds)
+        pa, na = (ctypes.c_void_p * 5)(*ptrs), (ctypes.c_int * 5)(*ns)
+        fn = self.L.vloam_b200_laser_odometry_input_device if dev else self.L.vloam_b200_laser_odometry_input
+        self._chk(fn(self.h, pa, na, stride, w_offset))
+
+    def laser_mapping_input(self, corner, surf, full, q_wodom, t_wodom, skip_frame=False, w_offset=3):
+        """LaserMapping::input (LM.cpp:178-209): the clouds, odometry pose (q x,y,z,w; t) and skip flag the next laser_mapping call
+        of this frame consumes, instead of the context's own odometry output."""
+        ptrs, ns, stride, dev, _keep = _clouds([corner, surf, full])
+        q = np.ascontiguousarray(q_wodom, np.float64)
+        t = np.ascontiguousarray(t_wodom, np.float64)
+        if q.shape != (4,) or t.shape != (3,):
+            raise ValueError("q_wodom is 4 doubles (x, y, z, w), t_wodom 3")
+        fn = self.L.vloam_b200_laser_mapping_input_device if dev else self.L.vloam_b200_laser_mapping_input
+        self._chk(fn(self.h, ptrs[0], ns[0], ptrs[1], ns[1], ptrs[2], ns[2], stride, w_offset, q.ctypes.data, t.ctypes.data,
+                     1 if skip_frame else 0))
 
     def laser_mapping(self, want_pose=True):
         q, t = np.zeros(4), np.zeros(3)
@@ -327,13 +385,20 @@ class ScanRegistration:
 
 
 class LaserOdometry:
-    """vloam::LaserOdometry (laser_odometry.h:63-87): input is implicit (clouds stay on the device)."""
+    """vloam::LaserOdometry (laser_odometry.h:63-87): by default the input is implicit (the clouds of the context's scan
+    registration stay on the device); input() with clouds copies the caller's instead."""
 
     def __init__(self, ctx):
         self.ctx, self.last = ctx, None
 
     def init(self):
         pass
+
+    def input(self, laserCloud=None, cornerPointsSharp=None, cornerPointsLessSharp=None, surfPointsFlat=None, surfPointsLessFlat=None):
+        """LO.cpp:137-148.  Without clouds nothing is copied (the context's own scan registration is used)."""
+        clouds = (laserCloud, cornerPointsSharp, cornerPointsLessSharp, surfPointsFlat, surfPointsLessFlat)
+        if any(c is not None for c in clouds):
+            self.ctx.laser_odometry_input(clouds)
 
     def solveLO(self, prior_q=None, prior_t=None):
         self.last = self.ctx.laser_odometry(prior_q, prior_t)
@@ -360,8 +425,15 @@ class LaserMapping:
     def reset(self):
         pass
 
-    def input(self, skip_frame):
+    def input(self, skip_frame, laserCloudCornerLast=None, laserCloudSurfLast=None, laserCloudFullRes=None, q_wodom_curr=None,
+              t_wodom_curr=None):
+        """LM.cpp:178-209.  Without clouds and pose the context's own odometry output is mapped; with them (all five) the caller's."""
         self.skip_frame = bool(skip_frame)
+        given = (laserCloudCornerLast, laserCloudSurfLast, laserCloudFullRes, q_wodom_curr, t_wodom_curr)
+        if any(g is not None for g in given):
+            if any(g is None for g in given):
+                raise ValueError("LaserMapping.input takes the three clouds and the odometry pose together")
+            self.ctx.laser_mapping_input(laserCloudCornerLast, laserCloudSurfLast, laserCloudFullRes, q_wodom_curr, t_wodom_curr, skip_frame)
 
     def solveMapping(self):
         """On a skipped frame this only propagates the high-frequency pose (the reference does not call solveMapping then), so the

@@ -189,7 +189,8 @@ void vloam_b200_destroy(vloam_b200_ctx* c) {
   vl_lm_free(c);
   if (c->streamLO) { cudaStreamSynchronize(c->streamLO); cudaStreamDestroy(c->streamLO); }
   cudaEventDestroy(c->evS2); cudaEventDestroy(c->evLoSolve); cudaEventDestroy(c->evLoNext); if (c->evEnd) cudaEventDestroy(c->evEnd);
-  void* singles[] = {c->los, c->losNext, c->evalOut, c->lms, c->lmm, c->cubeC, c->cubeS, c->vScalars, c->loRingTbl, c->loGridCells[0].p, c->loGridCells[1].p,
+  if (c->evIn) cudaEventDestroy(c->evIn);
+  void* singles[] = {c->los, c->losNext, c->miLos, c->evalOut, c->lms, c->lmm, c->cubeC, c->cubeS, c->vScalars, c->loRingTbl, c->loGridCells[0].p, c->loGridCells[1].p,
                      c->loGridCellOf.p, c->loGridSorted[0].p, c->loGridSorted[1].p, c->dbgLoCorner[0].p, c->dbgLoCorner[1].p, c->dbgLoSurf[0].p,
                      c->dbgLoSurf[1].p, c->dbgKnnIdx[0][0].p, c->dbgKnnIdx[0][1].p, c->dbgKnnIdx[1][0].p, c->dbgKnnIdx[1][1].p, c->dbgKnnD2[0][0].p,
                      c->dbgKnnD2[0][1].p, c->dbgKnnD2[1][0].p, c->dbgKnnD2[1][1].p, c->dbgKnnOk[0][0].p, c->dbgKnnOk[0][1].p, c->dbgKnnOk[1][0].p,
@@ -197,7 +198,8 @@ void vloam_b200_destroy(vloam_b200_ctx* c) {
   for (void* p : singles) vl_dev_free(c, p);
   void* bufs[] = {c->lessSharp[0].p, c->lessSharp[1].p, c->lessSharp[2].p, c->lessFlat[0].p, c->lessFlat[1].p, c->lessFlat[2].p, c->endSharp[0].p, c->endSharp[1].p, c->endSharp[2].p, c->endFlat[0].p, c->endFlat[1].p, c->endFlat[2].p, c->loCornerIdx.p, c->loSurfIdx.p, c->factors.p, c->factorS.p, c->factorValid.p, c->loFactors.p, c->loFactorValid.p, c->evalPartials.p,
                   c->poolC.p, c->poolS.p, c->stackC.p, c->stackS.p, c->stackCN.p, c->stackSN.p, c->fromMapC.p, c->fromMapS.p, c->knnD2.p, c->knnOk.p,
-                  c->vKeys.p, c->vKeys2.p, c->vHead.p, c->vScan.p, c->vScan2.p, c->vOut.p, c->vIn.p, c->regOut.p, c->tailKeys.p, c->staging.p};
+                  c->vKeys.p, c->vKeys2.p, c->vHead.p, c->vScan.p, c->vScan2.p, c->vOut.p, c->vIn.p, c->regOut.p, c->tailKeys.p, c->staging.p,
+                  c->inStage.p, c->miCorner.p, c->miSurf.p, c->miFull.p};
   for (void* p : bufs) vl_dev_free(c, p);
   if (c->h_s2flag) cudaFreeHost(c->h_s2flag);
   cudaFreeHost(c->h_los); cudaFreeHost(c->h_lms); cudaFreeHost(c->h_lmm); cudaFreeHost(c->h_vScalars);
@@ -217,6 +219,7 @@ int vloam_b200_begin_frame(vloam_b200_ctx* c) {
   if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
   VL_CUDA(cudaSetDevice(c->device));
   c->lm_reset_pending = true;  // applied by the next solveMapping (the map update of the previous frame may still be reading the list)
+  c->miPending = c->miUsed = false;  // a mapping input the last frame never consumed is dropped
   return VLOAM_OK;
 }
 
@@ -382,16 +385,23 @@ int vloam_b200_laser_odometry(vloam_b200_ctx* c, const double* prior_q, const do
   return VLOAM_OK;
 }
 
+// LaserMapping::input as LOM.cpp:149-158 calls it: the context's own odometry output of this frame
+static VlLmInput own_lm_input(const vloam_b200_ctx* c) {
+  return VlLmInput{c->cornerLastPtr, c->nCornerLast, c->surfLastPtr, c->nSurfLast, c->los, c->skip_frame ? 1 : 0, false};
+}
+
 int vloam_b200_laser_mapping(vloam_b200_ctx* c, double* q_w, double* t_w) {
   if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
-  VL_TRY(vl_lm_run(c));
+  const VlLmInput in = c->miPending ? VlLmInput{c->miCorner.p, c->miNc, c->miSurf.p, c->miNs, c->miLos, c->miSkip ? 1 : 0, true} : own_lm_input(c);
+  c->miUsed = c->miPending; c->miPending = false;
+  VL_TRY(vl_lm_run(c, in));
   if (c->timing) VL_CUDA(cudaEventRecord(c->ev[3], c->stream));
   if (q_w || t_w) {
     VL_CUDA(cudaMemcpyAsync(c->h_lmm, c->lmm, sizeof(LmScalars), cudaMemcpyDeviceToHost, c->stream));
     VL_CUDA(cudaStreamSynchronize(c->stream));
     if (c->h_lmm->overflow) { snprintf(c->err, sizeof c->err, "map pool exhausted"); return VLOAM_E_CAPACITY; }
-    const double* q = c->skip_frame ? c->h_lmm->q_hf : c->h_lmm->pose;
-    const double* t = c->skip_frame ? c->h_lmm->t_hf : c->h_lmm->pose + 4;
+    const double* q = in.skip ? c->h_lmm->q_hf : c->h_lmm->pose;
+    const double* t = in.skip ? c->h_lmm->t_hf : c->h_lmm->pose + 4;
     if (q_w) memcpy(q_w, q, 32);
     if (t_w) memcpy(t_w, t, 24);
   }
@@ -400,15 +410,126 @@ int vloam_b200_laser_mapping(vloam_b200_ctx* c, double* q_w, double* t_w) {
 
 int vloam_b200_register_full_cloud(vloam_b200_ctx* c, float* out, int cap_points) {
   if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
-  VL_TRY(vl_sr_sync_counts(c));
-  const int n = c->nKept;
+  // after a mapping call that consumed a caller input: the caller's laserCloudFullRes, as given (LaserMapping does no TransformToEnd)
+  if (!c->miUsed) VL_TRY(vl_sr_sync_counts(c));
+  const int n = c->miUsed ? c->miNfull : c->nKept;
   if (!out || n == 0) return n;
   if (cap_points < n) { snprintf(c->err, sizeof c->err, "cloud buffer too small (%d < %d)", cap_points, n); return VLOAM_E_CAPACITY; }
   VL_TRY(vl_reserve(c, c->regOut, (size_t)n));
-  VL_TRY(vl_lm_register_full(c, c->cloud.p, n, c->regOut.p));
+  if (c->miUsed) VL_TRY(vl_lm_register_full(c, c->miFull.p, n, c->regOut.p, c->miSkip ? 1 : 0, false));
+  else VL_TRY(vl_lm_register_full(c, c->cloud.p, n, c->regOut.p, c->skip_frame ? 1 : 0, vl_to_end(c)));
   VL_CUDA(cudaMemcpyAsync(out, c->regOut.p, (size_t)n * 16, cudaMemcpyDeviceToHost, c->stream));
   VL_CUDA(cudaStreamSynchronize(c->stream));
   return n;
+}
+
+// ---- stage inputs from the caller (LaserOdometry::input LO.cpp:137-148, LaserMapping::input LM.cpp:178-209) ----------------------
+static int bad_input(vloam_b200_ctx* c, const char* what) {
+  snprintf(c->err, sizeof c->err, "%s", what);
+  return VLOAM_E_INVALID;
+}
+static int check_layout(vloam_b200_ctx* c, int stride, int w_offset) {
+  if (stride < 4) return bad_input(c, "stride must be >= 4 floats (x, y, z, intensity)");
+  if (w_offset < 3 || w_offset > stride - 1) return bad_input(c, "w_offset must lie in [3, stride - 1]");
+  return VLOAM_OK;
+}
+static int check_cloud(vloam_b200_ctx* c, const char* name, const void* p, int n) {
+  if (n < 0 || (n > 0 && !p)) {
+    snprintf(c->err, sizeof c->err, "%s: %s", name, n < 0 ? "negative point count" : "NULL pointer with a non-zero point count");
+    return VLOAM_E_INVALID;
+  }
+  return VLOAM_OK;
+}
+static int stage_inputs_init(vloam_b200_ctx* c, bool mapping) {  // first input call: what every later one reuses
+  if (!c->evIn) VL_CUDA(cudaEventCreateWithFlags(&c->evIn, cudaEventDisableTiming));
+  if (mapping && !c->miLos) {
+    VL_CUDA(cudaMalloc(&c->miLos, sizeof(LoScalars)));
+    __atomic_fetch_add(&c->regrows, 1LL, __ATOMIC_RELAXED);
+  }
+  return VLOAM_OK;
+}
+
+// The five clouds take the place of this frame's scan registration: they are written where vl_sr_run writes (the generation it
+// would advance to), with the device and host counts and the events it records, so the odometry runs unchanged.
+static int odometry_input(vloam_b200_ctx* c, const float* const clouds[5], const int n[5], int stride, int w_offset, bool device) {
+  if (!clouds || !n) return bad_input(c, "clouds and n must not be NULL");
+  VL_TRY(check_layout(c, stride, w_offset));
+  static const char* names[5] = {"laserCloud", "cornerPointsSharp", "cornerPointsLessSharp", "surfPointsFlat", "surfPointsLessFlat"};
+  for (int k = 0; k < 5; ++k) VL_TRY(check_cloud(c, names[k], clouds[k], n[k]));
+  VL_TRY(stage_inputs_init(c, false));
+  if (c->timing) VL_CUDA(cudaEventRecord(c->ev[0], c->stream));
+  vl_drop_lookahead(c);  // as a scan_registration call with an unregistered buffer
+  c->srAdopted = false;
+  // the last scan registration of this set may still have its tail on a side stream (it reads `cloud`) and its counts in flight to
+  // h_srs, which is rewritten below
+  VL_CUDA(cudaEventSynchronize(c->evSR));
+  VL_CUDA(cudaStreamWaitEvent(c->stream, c->evSR, 0));
+  c->sr_counts_valid = false;
+  c->cur = (c->cur + 1) % 3;
+  VL_TRY(vl_reserve(c, c->cloud, (size_t)max(n[0], 1)));
+  VL_TRY(vl_reserve(c, c->sharp, (size_t)max(n[1], 1)));
+  VL_TRY(vl_reserve(c, c->lessSharp[c->cur], (size_t)max(n[2], 1)));
+  VL_TRY(vl_reserve(c, c->flat, (size_t)max(n[3], 1)));
+  VL_TRY(vl_reserve(c, c->lessFlat[c->cur], (size_t)max(n[4], 1)));
+  const VlCloudIn cl[5] = {{clouds[0], n[0], c->cloud.p}, {clouds[1], n[1], c->sharp.p}, {clouds[2], n[2], c->lessSharp[c->cur].p},
+                           {clouds[3], n[3], c->flat.p}, {clouds[4], n[4], c->lessFlat[c->cur].p}};
+  VL_TRY(vl_pack_clouds(c, cl, 5, stride, w_offset, device));
+  SrScalars* h = c->h_srs;
+  memset(h, 0, sizeof *h);
+  h->firstValid = 0; h->lastValid = n[0] - 1; h->count = n[0];
+  h->nSharp = n[1]; h->nLessSharp = n[2]; h->nFlat = n[3]; h->nLessFlat = n[4]; h->nQueries = n[1] + n[3];
+  VL_CUDA(cudaMemcpyAsync(c->srs, h, sizeof(SrScalars), cudaMemcpyHostToDevice, c->stream));
+  VL_CUDA(cudaEventRecord(c->evSRfeat, c->stream));
+  VL_CUDA(cudaEventRecord(c->evSR, c->stream));
+  c->n_in = n[0] + n[1] + n[2] + n[3] + n[4]; c->stride = 4;
+  c->nKept = n[0]; c->nSharp = n[1]; c->nLessSharp = n[2]; c->nFlat = n[3]; c->nLessFlat = n[4];
+  c->sr_counts_valid = true;
+  if (c->timing) VL_CUDA(cudaEventRecord(c->ev[1], c->stream));
+  return VLOAM_OK;
+}
+int vloam_b200_laser_odometry_input(vloam_b200_ctx* c, const float* const clouds[5], const int n[5], int stride, int w_offset) {
+  if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
+  return odometry_input(c, clouds, n, stride, w_offset, false);
+}
+int vloam_b200_laser_odometry_input_device(vloam_b200_ctx* c, const float* const d_clouds[5], const int n[5], int stride, int w_offset) {
+  if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
+  return odometry_input(c, d_clouds, n, stride, w_offset, true);
+}
+
+// Copied into context-owned buffers and a pose block of their own: nothing of the odometry state is touched.
+static int mapping_input(vloam_b200_ctx* c, const float* corner, int nc, const float* surf, int ns, const float* full, int nfull, int stride,
+                         int w_offset, const double* q_wodom, const double* t_wodom, int skip_frame, bool device) {
+  VL_TRY(check_layout(c, stride, w_offset));
+  VL_TRY(check_cloud(c, "laserCloudCornerLast", corner, nc));
+  VL_TRY(check_cloud(c, "laserCloudSurfLast", surf, ns));
+  VL_TRY(check_cloud(c, "laserCloudFullRes", full, nfull));
+  if (!q_wodom || !t_wodom) return bad_input(c, "q_wodom and t_wodom must not be NULL");
+  if (skip_frame != 0 && skip_frame != 1) return bad_input(c, "skip_frame must be 0 or 1");
+  VL_TRY(stage_inputs_init(c, true));
+  // (the buffers were last read by the previous frame's stack filters and register_full_cloud, both ordered before this main-stream point)
+  VL_TRY(vl_reserve(c, c->miCorner, (size_t)max(nc, 1)));
+  VL_TRY(vl_reserve(c, c->miSurf, (size_t)max(ns, 1)));
+  VL_TRY(vl_reserve(c, c->miFull, (size_t)max(nfull, 1)));
+  const VlCloudIn cl[3] = {{corner, nc, c->miCorner.p}, {surf, ns, c->miSurf.p}, {full, nfull, c->miFull.p}};
+  VL_TRY(vl_pack_clouds(c, cl, 3, stride, w_offset, device));
+  LoScalars h;
+  memset(&h, 0, sizeof h);
+  h.para_q[3] = 1.0;
+  memcpy(h.q_w, q_wodom, 32); memcpy(h.t_w, t_wodom, 24);
+  VL_CUDA(cudaMemcpyAsync(c->miLos, &h, sizeof h, cudaMemcpyHostToDevice, c->stream));  // (pageable: staged before the call returns)
+  c->miNc = nc; c->miNs = ns; c->miNfull = nfull; c->miSkip = skip_frame != 0;
+  c->miPending = true;
+  return VLOAM_OK;
+}
+int vloam_b200_laser_mapping_input(vloam_b200_ctx* c, const float* corner, int nc, const float* surf, int ns, const float* full, int nfull,
+                                   int stride, int w_offset, const double* q_wodom, const double* t_wodom, int skip_frame) {
+  if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
+  return mapping_input(c, corner, nc, surf, ns, full, nfull, stride, w_offset, q_wodom, t_wodom, skip_frame, false);
+}
+int vloam_b200_laser_mapping_input_device(vloam_b200_ctx* c, const float* d_corner, int nc, const float* d_surf, int ns, const float* d_full,
+                                          int nfull, int stride, int w_offset, const double* q_wodom, const double* t_wodom, int skip_frame) {
+  if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
+  return mapping_input(c, d_corner, nc, d_surf, ns, d_full, nfull, stride, w_offset, q_wodom, t_wodom, skip_frame, true);
 }
 
 static int process_common(vloam_b200_ctx* c, double* pose_out) {
@@ -419,7 +540,7 @@ static int process_common(vloam_b200_ctx* c, double* pose_out) {
   if (rlo != VLOAM_OK) return rlo;
   if (pose_out) {
     c->s2Done = false;
-    VL_TRY(vl_lm_run(c));
+    VL_TRY(vl_lm_run(c, own_lm_input(c)));
     if (c->timing) VL_CUDA(cudaEventRecord(c->ev[3], c->stream));
     if (!c->s2Done) {  // (mapping skipped on this frame) -- otherwise sync point S2 already brought both structs over
       VL_CUDA(cudaMemcpyAsync(c->h_los, c->los, sizeof(LoScalars), cudaMemcpyDeviceToHost, c->stream));

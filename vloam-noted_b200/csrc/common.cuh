@@ -238,6 +238,16 @@ struct vloam_b200_ctx {
   int* h_vScalars;
   // refilter scratch
   DBuf<unsigned long long> tailKeys; DBuf<float4> staging;
+  // caller-supplied stage inputs (vloam_b200_laser_odometry_input / vloam_b200_laser_mapping_input, stage_inputs.cu); everything here
+  // is reserved by the first input call, a context that never makes one holds none of it
+  DBuf<float> inStage;                  // host clouds with stride != 4 or w_offset != 3, uploaded as they are, before vl_pack_xyzi
+  DBuf<float4> miCorner, miSurf, miFull;  // LaserMapping::input's laserCloudCornerLast / laserCloudSurfLast / laserCloudFullRes
+  LoScalars* miLos;                     // device: the caller's q_wodom_curr / t_wodom_curr in q_w / t_w (never c->los)
+  cudaEvent_t evIn;                     // the caller's clouds are on the device (the stack filters of the side streams wait on it)
+  int miNc, miNs, miNfull;
+  bool miPending;                       // a mapping input waits for the next vloam_b200_laser_mapping call of this frame
+  bool miUsed;                          // the mapping call of this frame consumed one (register_full_cloud and the pose follow it)
+  bool miSkip;                          // its skip_frame
   // per-kernel timing (vloam_b200_profile_kernel): CUDA events around the launches of one named kernel
   char prof_name[64];                 // kernel to time, or "*" for every launch
   cudaEvent_t prof_ev[VL_PROF_MAX][2];
@@ -383,8 +393,18 @@ int vl_sr_exact_math(vloam_b200_ctx* c, const float* d_y, const float* d_x, int 
 int vl_lo_run(vloam_b200_ctx* c, const double* prior_q, const double* prior_t, int use_prior);
 int vl_lo_associate_only(vloam_b200_ctx* c, const double* x, int* corner_idx, int* surf_idx);
 int vl_lo_build_last(vloam_b200_ctx* c, int set, const float4* corner, int nc, const float4* surf, int ns);
-int vl_lm_run(vloam_b200_ctx* c);
-int vl_lm_enqueue_stacks(vloam_b200_ctx* c, const float4* corner, int nc, const float4* surf, int ns, bool early = false);
+// What one solveMapping reads (LaserMapping::input, LM.cpp:178-209): the context's own odometry output, or the caller's
+// (vloam_b200_laser_mapping_input).  los: device block whose q_w / t_w are q_wodom_curr / t_wodom_curr.
+struct VlLmInput {
+  const float4* corner; int nc;
+  const float4* surf; int ns;
+  const LoScalars* los;
+  int skip;
+  bool caller;  // the clouds are the caller's: filter them into the stacks here, superseding any filtered from the context's own
+};
+int vl_lm_run(vloam_b200_ctx* c, const VlLmInput& in);
+// early: see laser_mapping.cu; ownClouds: the clouds are this sweep's odometry output (under VLOAM_FLAG_TRANSFORM_TO_END the filters wait for evEnd)
+int vl_lm_enqueue_stacks(vloam_b200_ctx* c, const float4* corner, int nc, const float4* surf, int ns, bool early = false, bool ownClouds = true);
 int vl_lm_enqueue_stacks_next(vloam_b200_ctx* c, const float4* corner, int nc, const float4* surf, int ns);  // into the spare stack buffers (helper thread)
 int vl_lm_adopt_stacks_next(vloam_b200_ctx* c);  // make the spare stack buffers current
 int vl_lm_publish_map(vloam_b200_ctx* c);         // queue the assembly of laserCloudMap (LM.cpp:884-899) on the publication stream
@@ -405,7 +425,11 @@ int vl_lo_lookahead_stacks(vloam_b200_ctx* c);  // part 2 (after S2 is recorded)
 int vl_lo_flush_deferred(vloam_b200_ctx* c);  // queue the deferred side-stream work of the last odometry call (look-ahead scan registration, next search structures)
 int vl_vg_preload(vloam_b200_ctx* c);
 int vl_lm_preload(vloam_b200_ctx* c);
-int vl_lm_register_full(vloam_b200_ctx* c, const float4* d_in, int n, float4* d_out);
+int vl_lm_register_full(vloam_b200_ctx* c, const float4* d_in, int n, float4* d_out, int skip, bool toEnd);
+// stage_inputs.cu: up to VL_PACK_MAX caller clouds of (stride, w_offset) float records into float4 buffers, on the main stream
+#define VL_PACK_MAX 5
+struct VlCloudIn { const float* src; int n; float4* dst; };
+int vl_pack_clouds(vloam_b200_ctx* c, const VlCloudIn* clouds, int k, int stride, int w_offset, bool device);
 int vl_lm_fit_sets(vloam_b200_ctx* c, const float* d_near, int n, int kind, int* d_ok, double* d_prm);  // vloam_b200_fit
 int vl_lm_join(vloam_b200_ctx* c);      // wait until the helper thread has issued the pending map update; returns its status
 int vl_lm_submit_task(vloam_b200_ctx* c, int (*fn)(vloam_b200_ctx*));  // hand a launch-issuing task to the helper thread (joins the previous one first)

@@ -1791,9 +1791,12 @@ static int lm_issue_stacks(vloam_b200_ctx* c, const float4* corner, int nc, cons
   if (!toNext) c->stacksReady = true;
   return VLOAM_OK;
 }
-int vl_lm_enqueue_stacks(vloam_b200_ctx* c, const float4* corner, int nc, const float4* surf, int ns, bool early) {
+int vl_lm_enqueue_stacks(vloam_b200_ctx* c, const float4* corner, int nc, const float4* surf, int ns, bool early, bool ownClouds) {
   VL_TRY(vl_lm_join(c));  // evKeys of the previous frame's update must have been recorded before it is waited on
-  if (vl_to_end(c)) {  // the clouds are this sweep's end clouds (LO.cpp:537-556): filter them behind its TransformToEnd
+  if (!ownClouds) {  // the caller's clouds (vloam_b200_laser_mapping_input): behind their upload, and behind any filter of this sweep's own
+    VL_CUDA(cudaStreamWaitEvent(c->stream2, c->evIn, 0));
+    VL_CUDA(cudaStreamWaitEvent(c->stream4, c->evIn, 0));
+  } else if (vl_to_end(c)) {  // the clouds are this sweep's end clouds (LO.cpp:537-556): filter them behind its TransformToEnd
     VL_CUDA(cudaStreamWaitEvent(c->stream2, c->evEnd, 0));
     VL_CUDA(cudaStreamWaitEvent(c->stream4, c->evEnd, 0));
   }
@@ -2013,19 +2016,20 @@ static int lm_sync_s2(vloam_b200_ctx* c, bool capture, bool* lookaheadDone, bool
 // The in-place path: the grid describes this sweep's sub-map unless lm_prepare_fast finds the window moved or the grid dirty.  The
 // passes and the in-place map update are queued, then the host waits at S2 and updates its bounds.  *fellBack: lm_prepare_fast raised
 // needSlow -- nothing of this sweep's mapping was applied (every kernel returned at once) and the caller repeats it on the pool path.
-static int lm_run_in_place(vloam_b200_ctx* c, LmDevice* d, int nqBound, int resetValid, bool inlineUpdate, bool* fellBack) {
+static int lm_run_in_place(vloam_b200_ctx* c, LmDevice* d, const LoScalars* lo, int nqBound, int resetValid, bool inlineUpdate, bool* fellBack) {
   *fellBack = false;
   bool lookaheadDone = false;
   // stacks filtered a sweep ago (look-ahead): the counts are set by lm_prepare_fast itself, one launch fewer on the pose chain
   const bool countsSet = c->stacksAdopted;
+  // the odometry state S2 hands to the host (h_los) is always the context's own, also when `lo` is the caller's pose
   const LoScalars* const losNow = c->los;  // (read before the helper thread may swap the odometry states)
   if (countsSet) {
     VL_CUDA(cudaStreamWaitEvent(c->stream, c->evStacks, 0));
     VL_CUDA(cudaStreamWaitEvent(c->stream, c->evStacksC, 0));
-    VL_LAUNCH(lm_prepare_fast, 1, 256, 0, c->lmm, c->los, d->work, d->grid.hdr, 0, resetValid, (const int*)(d->dQ + 2 * c->stackSel),
+    VL_LAUNCH(lm_prepare_fast, 1, 256, 0, c->lmm, lo, d->work, d->grid.hdr, 0, resetValid, (const int*)(d->dQ + 2 * c->stackSel),
               (const int*)(d->dQ + 2 * c->stackSel + 1), (const int*)d->grid.top);
   } else {
-    VL_LAUNCH(lm_prepare_fast, 1, 256, 0, c->lmm, c->los, d->work, d->grid.hdr, 0, resetValid, (const int*)nullptr, (const int*)nullptr, (const int*)nullptr);
+    VL_LAUNCH(lm_prepare_fast, 1, 256, 0, c->lmm, lo, d->work, d->grid.hdr, 0, resetValid, (const int*)nullptr, (const int*)nullptr, (const int*)nullptr);
   }
   if (c->timing) VL_CUDA(cudaEventRecord(c->evx[0], c->stream));
   VL_HOST_MARK(8);
@@ -2173,14 +2177,15 @@ static int lm_pool_update(vloam_b200_ctx* c, LmDevice* d, const LmPoolUpdate& u)
 
 // The pool path (round 1's): cube tables, sorted pools; the grid is rebuilt for the window lm_prepare finds.  lookaheadDone: the
 // in-place path fell back after its sync point S2 had already queued the next sweep's odometry.
-static int lm_run_pool(vloam_b200_ctx* c, LmDevice* d, int nqBound, int resetValid, bool capture, bool inlineUpdate, bool lookaheadDone) {
+static int lm_run_pool(vloam_b200_ctx* c, LmDevice* d, const LoScalars* lo, int nqBound, int resetValid, bool capture, bool inlineUpdate,
+                       bool lookaheadDone) {
   VL_CUDA(cudaStreamWaitEvent(c->stream, c->evAux, 0));  // (the previous sweep's raw appends outside the window edit the cube tables)
   // a map publication queued since the last update: lm_prepare rolls the cube tables it reads, and this stream's evPose orders the
   // update, the speculative rebuild and the appends (stream3, streamAux) behind it as well
   VL_CUDA(cudaStreamWaitEvent(c->stream, d->evPub, 0));
   if (d->poolsStale) VL_TRY(lm_materialize(c, d));  // the in-place updates since the last pool-path sweep, written back first (main stream)
   d->paths[1]++;
-  VL_LAUNCH(lm_prepare, 1, 1024, 0, c->lmm, c->los, c->cubeC, c->cubeS, d->work, 0, resetValid, d->subReal);
+  VL_LAUNCH(lm_prepare, 1, 1024, 0, c->lmm, lo, c->cubeC, c->cubeS, d->work, 0, resetValid, d->subReal);
   const long long totalBound = d->hMapUpperC + d->hMapUpperS;
   if (d->gridEnabled) VL_TRY(lm_reserve_merge(c, d, LG_NEWVOX_MAX, LG_NEWVOX_MAX, totalBound, false));
   VL_TRY(lg_rebuild_launch(c, d, d->subReal, totalBound));
@@ -2211,30 +2216,32 @@ static int lm_run_pool(vloam_b200_ctx* c, LmDevice* d, int nqBound, int resetVal
   return VLOAM_OK;
 }
 
-int vl_lm_run(vloam_b200_ctx* c) {
+int vl_lm_run(vloam_b200_ctx* c, const VlLmInput& in) {
   LmDevice* d = c->lm;
   VL_HOST_MARK(3);
   VL_TRY(vl_lm_join(c));  // the previous frame's map update has been issued (evMap recorded, host bounds updated)
   VL_HOST_MARK(4);
-  const int skip = c->skip_frame ? 1 : 0;
   const int resetValid = c->lm_reset_pending ? 1 : 0;
   c->lm_reset_pending = false;
   VL_CUDA(cudaStreamWaitEvent(c->stream, c->evMap, 0));  // the previous frame's map update (stream3) must be complete
   // ... its raw appends to cubes OUTSIDE the window (streamAux) touch pool segments only: nothing of the in-place path reads them
   // (a single CTA that takes 20-60 us when the sensor nears a window edge: it used to sit on the next sweep's pose chain);
   // the pool path waits for them before it reads the cube tables.
-  if (skip) {  // LM.cpp:197-201: only the high-frequency pose is propagated
-    VL_LAUNCH(lm_prepare_fast, 1, 256, 0, c->lmm, c->los, d->work, d->grid.hdr, 1, resetValid, (const int*)nullptr, (const int*)nullptr, (const int*)nullptr);
+  if (in.skip) {  // LM.cpp:197-201: only the high-frequency pose is propagated
+    if (in.caller) c->stacksReady = false;  // (stacks this sweep's odometry may have filtered are not used)
+    VL_LAUNCH(lm_prepare_fast, 1, 256, 0, c->lmm, in.los, d->work, d->grid.hdr, 1, resetValid, (const int*)nullptr, (const int*)nullptr, (const int*)nullptr);
     VL_TRY(vl_lo_flush_deferred(c)); VL_CUDA(cudaGetLastError());
     return VLOAM_OK;
   }
-  if (!c->stacksReady) {  // laser_mapping called without this frame's laser_odometry having queued them
+  if (in.caller) {  // filtered again from the caller's clouds into the pair the update reads, on the same side streams as any first filter
+    VL_TRY(vl_lm_enqueue_stacks(c, in.corner, in.nc, in.surf, in.ns, false, false));
+  } else if (!c->stacksReady) {  // laser_mapping called without this frame's laser_odometry having queued them
     VL_CUDA(cudaStreamSynchronize(c->stream));
-    VL_TRY(vl_lm_enqueue_stacks(c, c->cornerLastPtr, c->nCornerLast, c->surfLastPtr, c->nSurfLast));
+    VL_TRY(vl_lm_enqueue_stacks(c, in.corner, in.nc, in.surf, in.ns));
   }
   c->stacksReady = false;
   const bool capture = vl_debug_capture(c);
-  const int nqBound = max(c->nCornerLast + c->nSurfLast, 1);  // a voxel filter never grows a cloud
+  const int nqBound = max(in.nc + in.ns, 1);  // a voxel filter never grows a cloud
   VL_TRY(vl_reserve(c, c->knnPts, (size_t)nqBound * 5));
   VL_TRY(vl_reserve(c, c->knnD2, (size_t)nqBound * 5));
   VL_TRY(vl_reserve(c, c->knnOk, (size_t)nqBound));
@@ -2243,10 +2250,10 @@ int vl_lm_run(vloam_b200_ctx* c) {
   const bool inlineUpdate = d->noWorker || capture || c->prof_name[0];  // profiling and debug snapshots serialise everything
   bool fellBack = false;
   if (d->gridEnabled && d->gridValid && !capture && d->gridTopUpper + 2LL * nqBound <= d->grid.cap && d->newVoxUpper + nqBound <= LG_NEWVOX_MAX) {
-    VL_TRY(lm_run_in_place(c, d, nqBound, resetValid, inlineUpdate, &fellBack));
+    VL_TRY(lm_run_in_place(c, d, in.los, nqBound, resetValid, inlineUpdate, &fellBack));
     if (!fellBack) return VLOAM_OK;
   }
-  return lm_run_pool(c, d, nqBound, resetValid, capture, inlineUpdate, fellBack);
+  return lm_run_pool(c, d, in.los, nqBound, resetValid, capture, inlineUpdate, fellBack);
 }
 
 // LM.cpp:901-905 (LaserMapping::publish): laserCloudFullRes through pointAssociateToMap.  lo != nullptr
@@ -2269,11 +2276,11 @@ __global__ void __launch_bounds__(256) lm_register_full(const float4* __restrict
   }
 }
 
-int vl_lm_register_full(vloam_b200_ctx* c, const float4* d_in, int n, float4* d_out) {
+int vl_lm_register_full(vloam_b200_ctx* c, const float4* d_in, int n, float4* d_out, int skip, bool toEnd) {
   VL_BYTES(32.0 * n);
   // (c->los is this sweep's odometry state: a look-ahead solve of the next sweep writes the spare state, losNext)
-  VL_LAUNCH(lm_register_full, c->num_sms * 4, 256, 0, d_in, n, c->lmm, c->skip_frame ? 1 : 0, d_out,
-            vl_to_end(c) ? (const double*)c->los->para_q : (const double*)nullptr, vl_distortion(c) ? 1 : 0);
+  VL_LAUNCH(lm_register_full, c->num_sms * 4, 256, 0, d_in, n, c->lmm, skip, d_out, toEnd ? (const double*)c->los->para_q : (const double*)nullptr,
+            vl_distortion(c) ? 1 : 0);
   VL_CUDA(cudaGetLastError());
   return VLOAM_OK;
 }

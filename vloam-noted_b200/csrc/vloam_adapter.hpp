@@ -20,14 +20,25 @@
 // LO.cpp:45-54, LM.cpp:44-45, 99-102, 125-128) through vloam::adapter_param_source(), an injectable getter that defaults
 // to ros::param::get; a missing parameter aborts like ROS_BREAK() does (AdapterError).  VLOAM_B200_DEVICE selects the GPU.
 //
-// Data flow: the feature clouds never leave the device inside the pipeline; output() copies them out because the
-// reference's callers (and publish()) expect PCL clouds, and input() ASSERTS that the clouds handed in are the ones the
-// previous stage's output() produced from this context (size + first / last point) instead of uploading them again.
-// `adapter_options().fetch_clouds = false` skips the copies (poses only).
+// Data flow: inside one Engine the feature clouds never leave the device; output() copies them out because the reference's
+// callers (and publish()) expect PCL clouds.  input() then has three cases:
+//   - its stage's predecessor never ran in this Engine (a stage constructed on its own, with a private Engine from init()):
+//     the clouds and pose handed in are uploaded (vloam_b200_laser_odometry_input / vloam_b200_laser_mapping_input), as the
+//     reference's input() deep-copies them (LO.cpp:137-148, LM.cpp:178-209);
+//   - the shared Engine, `adapter_options().caller_clouds = true`: the clouds are compared in full with a private copy of
+//     what output() produced, and the pose with the one it returned; when they are equal the device copy is kept, otherwise
+//     the edited input is uploaded (feature clouds with moving objects removed, the mapping stage behind another odometry);
+//   - the shared Engine by default: input() ASSERTS that the clouds are the ones output() produced (size + first / last
+//     point) and throws on an edited copy, without keeping a copy of its own.
+// Clouds are passed to the C ABI as PCL lays them out in memory (stride sizeof(PointType) / 4 floats, intensity at
+// offsetof(PointType, intensity)): no host repack for the 16-byte stand-in or real PCL's 32-byte PointXYZI.
+// `adapter_options().fetch_clouds = false` skips the copies (poses only); the stages then keep the device path.
 //
 // publish(): the VloamTF writes are done; ROS topic / tf broadcast plumbing (SR.cpp:516-564, LO.cpp:587-611, 621-657,
 // LM.cpp:816-833, 862-920) stays with the caller -- the poses and clouds it would publish are the ones output() returns.
 #pragma once
+#include <stddef.h>
+#include <string.h>
 #include <functional>
 #include <memory>
 #include <stdexcept>
@@ -72,7 +83,10 @@ inline double adapter_param(const char* name) {
   if (!adapter_param_source().get(name, v)) throw AdapterError(std::string("missing ROS parameter '") + name + "' (the reference calls ROS_BREAK here)");
   return v;
 }
-struct AdapterOptions { bool fetch_clouds = true; };
+struct AdapterOptions {
+  bool fetch_clouds = true;    // output() copies the clouds to the host
+  bool caller_clouds = false;  // input() in a shared Engine accepts edited clouds / another odometry pose (uploads them)
+};
 inline AdapterOptions& adapter_options() { static AdapterOptions o; return o; }
 
 // Eigen's Quaterniond * Vector3d (uv = 2 u x v; v + w uv + u x uv), as the device code evaluates it.  Used only by
@@ -121,16 +135,20 @@ public:
   vloam_b200_ctx* ctx() const { return ctx_; }
   void check(int r) const { if (r < 0) throw AdapterError(vloam_b200_last_error(ctx_)); }
 
-  // device cloud `which` -> *out (allocated when null); remembers its signature for the input() assertions
+  // device cloud `which` -> *out (allocated when null); remembers its signature for the input() assertions, and under
+  // caller_clouds the cloud itself
   void fetch(int which, CloudPtr& out) {
     if (!out) out = CloudPtr(new Cloud());
     const int n = vloam_b200_get_cloud(ctx_, which, nullptr, 0);
     check(n);
+    if (which <= VLOAM_CLOUD_LESS_FLAT) produced_sr = true;
     Sig& s = sig_[which];
     s.n = (size_t)n; s.valid = true;
+    copy_[which].clear();
     if (!adapter_options().fetch_clouds) { out->points.clear(); s.valid = false; return; }
     buf_.resize((size_t)n * 4);
     if (n) check(vloam_b200_get_cloud(ctx_, which, buf_.data(), n));
+    if (adapter_options().caller_clouds) copy_[which] = buf_;
     out->points.resize(n);
     for (int i = 0; i < n; ++i) { PointType p; p.x = buf_[i * 4]; p.y = buf_[i * 4 + 1]; p.z = buf_[i * 4 + 2]; p.intensity = buf_[i * 4 + 3]; out->points[i] = p; }
     out->width = (unsigned)n; out->height = 1; out->is_dense = true;
@@ -149,8 +167,26 @@ public:
     if (!same) throw AdapterError(std::string("input(): ") + what + " is not the cloud the previous stage's output() returned; the CUDA path keeps the clouds on "
                                   "the device and cannot take edited copies (use vloam_b200_debug_set for state injection)");
   }
+  // caller_clouds: is `in` bit for bit the cloud output() produced?  (false when it was not fetched: the clouds are uploaded)
+  bool same(int which, const CloudPtr& in) const {
+    const std::vector<float>& c = copy_[which];
+    if (!sig_[which].valid || !in || in->points.size() * 4 != c.size()) return false;
+    for (size_t i = 0; i < in->points.size(); ++i) {
+      const PointType& p = in->points[i];
+      const float v[4] = {p.x, p.y, p.z, p.intensity};
+      if (memcmp(v, &c[i * 4], sizeof v) != 0) return false;
+    }
+    return true;
+  }
   int skip_from_device = 0;  // skip_frame as LaserOdometry::output computed it (LO.cpp:668-678)
   double q_wodom[4] = {0, 0, 0, 1}, t_wodom[3] = {0, 0, 0};
+  // the predecessor of a stage ran in this Engine: ScanRegistration::output fetched its clouds (also with fetch_clouds = false,
+  // when they stay on the device) / LaserOdometry::solveLO ran.  A stage whose predecessor never ran here uploads its input.
+  bool produced_sr = false, produced_lo = false;
+  // PCL memory as the C ABI reads it
+  static const float* points(const CloudPtr& c) { return c && !c->points.empty() ? reinterpret_cast<const float*>(c->points.data()) : nullptr; }
+  static int count(const CloudPtr& c) { return c ? (int)c->points.size() : 0; }
+  static const int kStride = (int)(sizeof(PointType) / sizeof(float)), kWOffset = (int)(offsetof(PointType, intensity) / sizeof(float));
 private:
   void create(const vloam_b200_params& p, int device) {
     const int r = vloam_b200_create(&p, device, &ctx_);
@@ -159,6 +195,7 @@ private:
   vloam_b200_ctx* ctx_ = nullptr;
   Sig sig_[8];
   std::vector<float> buf_;
+  std::vector<float> copy_[8];  // caller_clouds: what fetch() copied out, xyzi
 };
 
 // ---- scan_registration.h:64-81 -------------------------------------------------------------------------------------
@@ -231,11 +268,22 @@ public:
     laserCloudCornerLast = CloudPtr(new pcl::PointCloud<PointType>()); laserCloudSurfLast = CloudPtr(new pcl::PointCloud<PointType>());
     laserCloudFullRes = CloudPtr(new pcl::PointCloud<PointType>());
   }
-  // LO.cpp:137-148 deep-copies the five clouds; here they already live on the device: the arguments are checked to be
-  // ScanRegistration::output's clouds of this sweep.
+  // LO.cpp:137-148 deep-copies the five clouds.  In a shared Engine they already live on the device: by default the arguments
+  // are checked to be ScanRegistration::output's clouds of this sweep; under caller_clouds an edited set is uploaded.  A stage
+  // whose ScanRegistration never ran in its Engine uploads them.
   void input(const CloudPtr& laserCloud_, const CloudPtr& cornerPointsSharp_, const CloudPtr& cornerPointsLessSharp_, const CloudPtr& surfPointsFlat_,
              const CloudPtr& surfPointsLessFlat_) {
     need();
+    const CloudPtr* in[5] = {&laserCloud_, &cornerPointsSharp_, &cornerPointsLessSharp_, &surfPointsFlat_, &surfPointsLessFlat_};
+    bool upload = !e_->produced_sr;
+    if (!upload && adapter_options().caller_clouds)
+      for (int w = VLOAM_CLOUD_FULL; w <= VLOAM_CLOUD_LESS_FLAT; ++w) upload = upload || !e_->same(w, *in[w]);
+    if (upload) {
+      const float* p[5]; int n[5];
+      for (int w = 0; w < 5; ++w) { p[w] = Engine::points(*in[w]); n[w] = Engine::count(*in[w]); }
+      e_->check(vloam_b200_laser_odometry_input(e_->ctx(), p, n, Engine::kStride, Engine::kWOffset));
+      return;
+    }
     e_->expect(VLOAM_CLOUD_FULL, laserCloud_, "laserCloud"); e_->expect(VLOAM_CLOUD_SHARP, cornerPointsSharp_, "cornerPointsSharp");
     e_->expect(VLOAM_CLOUD_LESS_SHARP, cornerPointsLessSharp_, "cornerPointsLessSharp"); e_->expect(VLOAM_CLOUD_FLAT, surfPointsFlat_, "surfPointsFlat");
     e_->expect(VLOAM_CLOUD_LESS_FLAT, surfPointsLessFlat_, "surfPointsLessFlat");
@@ -250,6 +298,7 @@ public:
       pq[0] = r.x(); pq[1] = r.y(); pq[2] = r.z(); pq[3] = r.w(); pt[0] = o.x(); pt[1] = o.y(); pt[2] = o.z();
     }
     e_->check(vloam_b200_laser_odometry(e_->ctx(), pq, pt, prior ? 1 : 0, qw_, tw_, ql_, tl_, &skip_));
+    e_->produced_lo = true;
     e_->skip_from_device = skip_;
     for (int k = 0; k < 4; ++k) e_->q_wodom[k] = qw_[k];
     for (int k = 0; k < 3; ++k) e_->t_wodom[k] = tw_[k];
@@ -316,15 +365,30 @@ public:
     if (!e_) e_ = std::make_shared<Engine>();
   }
   void reset() { need(); e_->check(vloam_b200_begin_frame(e_->ctx())); }  // LM.cpp:132-136
-  // LM.cpp:178-209.  The three clouds must be LaserOdometry::output's (they are on the device already); the odometry
-  // pose handed in must be the one LaserOdometry::output returned (the device reads it from the shared context); on a
-  // skipped frame this call computes the high-frequency pose (LM.cpp:197-201), as solveMapping is not called then.
+  // LM.cpp:178-209.  In a shared Engine by default the three clouds must be LaserOdometry::output's (they are on the device
+  // already) and the odometry pose the one it returned (the device reads it from the shared context); under caller_clouds
+  // anything else is uploaded, and a stage whose LaserOdometry never ran in its Engine always uploads (the reference deep-copies
+  // both).  On a skipped frame this call computes the high-frequency pose (LM.cpp:197-201), as solveMapping is not called then.
   void input(const CloudPtr& laserCloudCornerLast_, const CloudPtr& laserCloudSurfLast_, const CloudPtr& laserCloudFullRes_, const Eigen::Quaterniond& q_wodom_curr_,
              const Eigen::Vector3d& t_wodom_curr_, const bool& skip_frame_) {
     need();
     skip_frame = skip_frame_;
-    if ((e_->skip_from_device != 0) != skip_frame) throw AdapterError("input(): skip_frame differs from the one LaserOdometry::output returned");
     const double q[4] = {q_wodom_curr_.x(), q_wodom_curr_.y(), q_wodom_curr_.z(), q_wodom_curr_.w()}, t[3] = {t_wodom_curr_.x(), t_wodom_curr_.y(), t_wodom_curr_.z()};
+    bool upload = !e_->produced_lo;
+    if (!upload && adapter_options().caller_clouds) {
+      upload = (e_->skip_from_device != 0) != skip_frame || memcmp(q, e_->q_wodom, sizeof q) != 0 || memcmp(t, e_->t_wodom, sizeof t) != 0;
+      if (!skip_frame)
+        upload = upload || !e_->same(VLOAM_CLOUD_CORNER_LAST, laserCloudCornerLast_) || !e_->same(VLOAM_CLOUD_SURF_LAST, laserCloudSurfLast_) ||
+                 !e_->same(VLOAM_CLOUD_FULL_RES, laserCloudFullRes_);
+    }
+    if (upload) {
+      e_->check(vloam_b200_laser_mapping_input(e_->ctx(), Engine::points(laserCloudCornerLast_), Engine::count(laserCloudCornerLast_),
+                                               Engine::points(laserCloudSurfLast_), Engine::count(laserCloudSurfLast_), Engine::points(laserCloudFullRes_),
+                                               Engine::count(laserCloudFullRes_), Engine::kStride, Engine::kWOffset, q, t, skip_frame ? 1 : 0));
+      if (skip_frame) e_->check(vloam_b200_laser_mapping(e_->ctx(), q_, t_));  // consumes the input: the high-frequency pose
+      return;
+    }
+    if ((e_->skip_from_device != 0) != skip_frame) throw AdapterError("input(): skip_frame differs from the one LaserOdometry::output returned");
     for (int k = 0; k < 4; ++k) if (q[k] != e_->q_wodom[k]) throw AdapterError("input(): q_wodom_curr is not the pose LaserOdometry::output returned");
     for (int k = 0; k < 3; ++k) if (t[k] != e_->t_wodom[k]) throw AdapterError("input(): t_wodom_curr is not the pose LaserOdometry::output returned");
     if (!skip_frame) {
