@@ -195,6 +195,40 @@ int vloam_b200_publish_map(vloam_b200_ctx* c);
  * publish_map before get_map replaces the first. */
 int vloam_b200_get_map(vloam_b200_ctx* c, float* out_xyzi, int cap_points);
 
+/* Prior maps: start from a map built earlier -- to continue mapping it in a later session, or to localize in it with the map held
+ * fixed.  No reference counterpart (LaserMapping always starts empty, LM.h:75-78); a context that never makes these calls runs no
+ * extra launch, wait or allocation, and their buffers are reserved by the first call.
+ *
+ * load_map replaces the context's map, both kinds, with world-frame (map-frame) clouds: `corner` for laserCloudCornerArray, `surf` for
+ * laserCloudSurfArray, as (stride, w_offset) float records like the stage inputs above (host pointers; device pointers for the _device
+ * variant, read on the context's main stream).  Each point goes to its cube by the insert formula (LM.cpp:747-756) at the context's
+ * current window centre (laserCloudCen*); points outside the 21x21x11 grid (LM.cpp:758-761) and points with a non-finite x, y or z
+ * are dropped, and dropped[2] (may be NULL) receives how many per kind.  Every non-empty cube is then pcl::VoxelGrid-filtered at
+ * line_res / plane_res over its points in input order (LM.cpp:795-808): one centroid per occupied voxel, f32 sums in input order,
+ * ascending voxel order.  Poses, odometry state, frame counts and the window centre are unchanged.  The call waits for the helper
+ * thread, the map update in flight and a pending publish_map (whose get_map still returns the old map); the next mapped sweep
+ * rebuilds its search structures.  Errors: VLOAM_E_INVALID as for the stage inputs, VLOAM_E_CAPACITY above 2097151 points of a kind;
+ * on any error the map is unchanged.  Empty clouds clear the map.
+ * A published map round-trips: load_map(get_map_kind(0), get_map_kind(1)) at the window centre it was published with gives back
+ * the same cubes. */
+int vloam_b200_load_map(vloam_b200_ctx* c, const float* corner, int nc, const float* surf, int ns, int stride, int w_offset,
+                        long long dropped[2]);
+int vloam_b200_load_map_device(vloam_b200_ctx* c, const float* d_corner, int nc, const float* d_surf, int ns, int stride, int w_offset,
+                               long long dropped[2]);
+/* The odometry-to-map transform q_wmap_wodom (x,y,z,w) / t_wmap_wodom the mapping stage keeps (transformUpdate, LM.cpp:147-151): it
+ * forms the next initial guess (LM.cpp:206-207) and the skipped-frame pose (LM.cpp:197-201), i.e. where the sensor starts in a
+ * loaded map.  Ordered on the device behind the last mapping; takes effect at the next laser_mapping.  VLOAM_E_INVALID for NULL or
+ * non-finite values. */
+int vloam_b200_set_map_pose(vloam_b200_ctx* c, const double q_wmap_wodom[4], const double t_wmap_wodom[3]);
+/* enabled = 0: later mapped sweeps localize against the map without changing it -- LM.cpp:741-808 (insert, re-filter, raw appends
+ * to cubes outside the window) is skipped; the solve, transformUpdate, register_full_cloud, publish_map, skipped frames and the
+ * look-ahead are as before, and the window still rolls (LM.cpp:252-444), clearing the cubes that leave the grid.  enabled = 1
+ * (the default) resumes normal updates on the current map. */
+int vloam_b200_set_map_update(vloam_b200_ctx* c, int enabled);
+/* The corner (which = 0) or surf (1) points of the last publish_map, in cube order: the get_map cloud without the other kind's
+ * cubes.  Same waits and errors as get_map; VLOAM_E_INVALID for another `which`. */
+int vloam_b200_get_map_kind(vloam_b200_ctx* c, int which, float* out_xyzi, int cap_points);
+
 /* MAIN.cpp:143-144, 186-190 in one call: begin_frame, scan_registration,
  * laser_odometry, laser_mapping.  pose_out (may be NULL): 14 doubles
  * {odom q[4], odom t[3], mapped q[4], mapped t[3]}.  On a mapped frame the call

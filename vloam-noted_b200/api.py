@@ -20,6 +20,7 @@ EXPORTS = [
     "vloam_b200_publish_map", "vloam_b200_get_map",
     "vloam_b200_laser_odometry_input", "vloam_b200_laser_odometry_input_device", "vloam_b200_laser_mapping_input",
     "vloam_b200_laser_mapping_input_device",
+    "vloam_b200_load_map", "vloam_b200_load_map_device", "vloam_b200_set_map_pose", "vloam_b200_set_map_update", "vloam_b200_get_map_kind",
 ]
 
 
@@ -87,6 +88,11 @@ def load_lib(build=False):
         getattr(L, name).argtypes = [vp, vp, vp, ci, ci]
     for name in ("vloam_b200_laser_mapping_input", "vloam_b200_laser_mapping_input_device"):
         getattr(L, name).argtypes = [vp, vp, ci, vp, ci, vp, ci, ci, ci, vp, vp, ci]
+    for name in ("vloam_b200_load_map", "vloam_b200_load_map_device"):
+        getattr(L, name).argtypes = [vp, vp, ci, vp, ci, ci, ci, vp]
+    L.vloam_b200_set_map_pose.argtypes = [vp, vp, vp]
+    L.vloam_b200_set_map_update.argtypes = [vp, ci]
+    L.vloam_b200_get_map_kind.argtypes = [vp, ci, vp, ci]
     _lib = L
     return L
 
@@ -215,6 +221,37 @@ class Context:
         if n:
             n = self._chk(self.L.vloam_b200_get_map(self.h, out.ctypes.data, n))
         return out[:n]
+
+    def get_map_kind(self, which):
+        """The corner (0) or surf (1) points of the last publish_map, in cube order: float32[n, 4] (the get_map cloud without the
+        other kind's cubes, so load_map(get_map_kind(0), get_map_kind(1)) restores the published map)."""
+        n = self._chk(self.L.vloam_b200_get_map_kind(self.h, which, None, 0))
+        out = np.empty((n, 4), np.float32)
+        if n:
+            n = self._chk(self.L.vloam_b200_get_map_kind(self.h, which, out.ctypes.data, n))
+        return out[:n]
+
+    def load_map(self, corner, surf, w_offset=3):
+        """Replace the map with world-frame clouds (numpy float32[n, stride], or float32 CUDA tensors): binned into the cubes at the
+        current window centre (LM.cpp:747-761) and VoxelGrid-filtered per cube (LM.cpp:795-808).  Returns the points dropped
+        (outside the cube grid or non-finite) per kind, int64[2]."""
+        ptrs, ns, stride, dev, _keep = _clouds([corner, surf])
+        dropped = np.zeros(2, np.int64)
+        fn = self.L.vloam_b200_load_map_device if dev else self.L.vloam_b200_load_map
+        self._chk(fn(self.h, ptrs[0], ns[0], ptrs[1], ns[1], stride, w_offset, dropped.ctypes.data))
+        return dropped
+
+    def set_map_pose(self, q_wmap_wodom, t_wmap_wodom):
+        """The odometry-to-map transform (q x,y,z,w; t) the next laser_mapping starts from (LM.cpp:147-151, 206-207)."""
+        q = np.ascontiguousarray(q_wmap_wodom, np.float64)
+        t = np.ascontiguousarray(t_wmap_wodom, np.float64)
+        if q.shape != (4,) or t.shape != (3,):
+            raise ValueError("q_wmap_wodom is 4 doubles (x, y, z, w), t_wmap_wodom 3")
+        self._chk(self.L.vloam_b200_set_map_pose(self.h, q.ctypes.data, t.ctypes.data))
+
+    def set_map_update(self, enabled):
+        """False: localize against the map without changing it (LM.cpp:741-808 skipped); True (default) resumes mapping."""
+        self._chk(self.L.vloam_b200_set_map_update(self.h, 1 if enabled else 0))
 
     def laser_odometry(self, prior_q=None, prior_t=None, want_pose=True):
         qw, tw, ql, tl = np.zeros(4), np.zeros(3), np.zeros(4), np.zeros(3)
@@ -453,6 +490,19 @@ class LaserMapping:
             self._published_at = n
             return True
         return False
+
+    def load_map(self, corner, surf, w_offset=3):
+        """Start from a prior map (Context.load_map); returns the dropped points per kind."""
+        return self.ctx.load_map(corner, surf, w_offset)
+
+    def set_map_pose(self, q_wmap_wodom, t_wmap_wodom):
+        self.ctx.set_map_pose(q_wmap_wodom, t_wmap_wodom)
+
+    def set_map_update(self, enabled):
+        self.ctx.set_map_update(enabled)
+
+    def get_map_kind(self, which):
+        return self.ctx.get_map_kind(which)
 
 
 class LidarOdometryMapping:

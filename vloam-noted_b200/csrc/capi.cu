@@ -1,5 +1,6 @@
 // capi.cu -- the C ABI of include/vloam_b200.h on top of the stage files.
 #include <stdlib.h>
+#include <cmath>
 #include <string>
 #include <vector>
 #include "common.cuh"
@@ -530,6 +531,43 @@ int vloam_b200_laser_mapping_input_device(vloam_b200_ctx* c, const float* d_corn
                                           int nfull, int stride, int w_offset, const double* q_wodom, const double* t_wodom, int skip_frame) {
   if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
   return mapping_input(c, d_corner, nc, d_surf, ns, d_full, nfull, stride, w_offset, q_wodom, t_wodom, skip_frame, true);
+}
+
+// ---- prior maps -------------------------------------------------------------------------------------------------------------------
+static int load_map(vloam_b200_ctx* c, const float* corner, int nc, const float* surf, int ns, int stride, int w_offset, long long dropped[2],
+                    bool device) {
+  VL_TRY(check_layout(c, stride, w_offset));
+  VL_TRY(check_cloud(c, "corner", corner, nc));
+  VL_TRY(check_cloud(c, "surf", surf, ns));
+  VL_TRY(stage_inputs_init(c, false));
+  return vl_lm_load_map(c, corner, nc, surf, ns, stride, w_offset, device, dropped);
+}
+int vloam_b200_load_map(vloam_b200_ctx* c, const float* corner, int nc, const float* surf, int ns, int stride, int w_offset, long long dropped[2]) {
+  if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
+  return load_map(c, corner, nc, surf, ns, stride, w_offset, dropped, false);
+}
+int vloam_b200_load_map_device(vloam_b200_ctx* c, const float* d_corner, int nc, const float* d_surf, int ns, int stride, int w_offset,
+                               long long dropped[2]) {
+  if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
+  return load_map(c, d_corner, nc, d_surf, ns, stride, w_offset, dropped, true);
+}
+int vloam_b200_set_map_pose(vloam_b200_ctx* c, const double q_wmap_wodom[4], const double t_wmap_wodom[3]) {
+  if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
+  if (!q_wmap_wodom || !t_wmap_wodom) return bad_input(c, "set_map_pose: q and t must not be NULL");
+  for (int k = 0; k < 7; ++k)
+    if (!std::isfinite(k < 4 ? q_wmap_wodom[k] : t_wmap_wodom[k - 4])) return bad_input(c, "set_map_pose: non-finite value");
+  return vl_lm_set_map_pose(c, q_wmap_wodom, t_wmap_wodom);
+}
+int vloam_b200_set_map_update(vloam_b200_ctx* c, int enabled) {
+  if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
+  vl_lm_set_map_update(c, enabled != 0);
+  return VLOAM_OK;
+}
+int vloam_b200_get_map_kind(vloam_b200_ctx* c, int which, float* out_xyzi, int cap_points) {
+  if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
+  if (which != 0 && which != 1) return bad_input(c, "get_map_kind: which must be 0 (corner) or 1 (surf)");
+  if (cap_points < 0) return VLOAM_E_INVALID;
+  return vl_lm_get_map_kind(c, which, out_xyzi, cap_points);
 }
 
 static int process_common(vloam_b200_ctx* c, double* pose_out) {

@@ -439,6 +439,12 @@ void vl_lm_shutdown(vloam_b200_ctx* c);  // stop the helper thread
 int vl_lm_export_map(vloam_b200_ctx* c, int which, void* out, long cap, long* bytes);
 int vl_lm_sync_pools(vloam_b200_ctx* c);  // write the in-place grid updates back to the cube pools (no-op when they are current)
 int vl_lm_import_map(vloam_b200_ctx* c, int which, const void* data, long bytes);
+// prior maps (vloam_b200_load_map, set_map_pose, set_map_update, get_map_kind)
+int vl_lm_load_map(vloam_b200_ctx* c, const float* corner, int nc, const float* surf, int ns, int stride, int w_offset, bool device,
+                   long long dropped[2]);
+int vl_lm_set_map_pose(vloam_b200_ctx* c, const double q[4], const double t[3]);
+void vl_lm_set_map_update(vloam_b200_ctx* c, bool enabled);
+int vl_lm_get_map_kind(vloam_b200_ctx* c, int which, float* out, int cap_points);
 
 // sort / voxel primitives (voxel_grid.cu)
 int vl_sort_u64(vloam_b200_ctx* c, unsigned long long* d_keys, int n_pow2);

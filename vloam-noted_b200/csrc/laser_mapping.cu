@@ -1673,6 +1673,13 @@ struct LmDevice {  // extra device state owned by this file
   DBuf<float4> pubOut;               // the published cloud
   bool pubDone;                      // something was published since create
   long long pubNewCap, pubOutCap;    // bounds the last assembly was sized for (checked by vl_lm_get_map)
+  // ---- prior maps (vloam_b200_load_map / set_map_update / get_map_kind); the buffers are reserved by the first call
+  bool mapUpdate;                    // LM.cpp:741-808 runs on mapped sweeps (vloam_b200_set_map_update; default on)
+  DBuf<float4> ldIn[2];              // the caller's corner / surf clouds, packed
+  DBuf<unsigned long long> ldKeys;   // (cube | voxel | input index) keys of both kinds
+  DBuf<int> ldInt;                   // LD_SCALARS scalars | per-cube output offsets of both kinds | per-tile run heads of both kinds
+  DBuf<int> pubKindOff;              // get_map_kind: output offset of every cube's segment of one kind (+ total)
+  DBuf<float4> pubKind;              // ... and the cloud
 };
 
 // chunk pool of the grid: P points occupy at most min(P, cells) + P / LG_C chunks (every cell ends in one partly filled chunk)
@@ -1717,7 +1724,7 @@ int vl_lm_init(vloam_b200_ctx* c) {
   VL_CUDA(cudaMemset(d->pubInt, 0, sizeof(int) * MP_INTS));
   d->gridEnabled = getenv("VLOAM_NO_GRID") == nullptr;
   d->noWorker = getenv("VLOAM_NO_WORKER") != nullptr;
-  d->gridValid = false; d->poolsStale = false; d->gridTopUpper = 0; d->newVoxUpper = 0; d->builtCount = 0;
+  d->gridValid = false; d->poolsStale = false; d->gridTopUpper = 0; d->newVoxUpper = 0; d->builtCount = 0; d->mapUpdate = true;
   VL_CUDA(cudaFuncSetAttribute(rf_seg_sort, cudaFuncAttributeMaxDynamicSharedMemorySize, RF_SEG_CAP * 8));
   d->hMapUpperC = d->hMapUpperS = 0;
   // Map pools: bump allocation with doubling per cube; when a pool is half full it is doubled (copy) at sync point
@@ -1750,7 +1757,8 @@ void vl_lm_free(vloam_b200_ctx* c) {  // everything vl_lm_init and this file's r
   if (d->evPub) cudaEventDestroy(d->evPub);
   void* dev[] = {d->work, d->dQ, d->subReal, d->subSpec, d->newPts.p, d->newCube.p, d->unmatched.p, d->grid.dir, d->grid.top, d->grid.hdr,
                  d->grid.pts, d->grid.key, d->grid.next, d->grid.posOf, d->muKey.p, d->muInt.p, d->knnIds.p,
-                 d->pubWork, d->pubInt, d->pubKeys.p, d->pubEnt.p, d->pubOut.p};
+                 d->pubWork, d->pubInt, d->pubKeys.p, d->pubEnt.p, d->pubOut.p, d->ldIn[0].p, d->ldIn[1].p, d->ldKeys.p, d->ldInt.p,
+                 d->pubKindOff.p, d->pubKind.p};
   for (void* p : dev) vl_dev_free(c, p);
   delete d;
   c->lm = nullptr;
@@ -2062,9 +2070,21 @@ static int lm_run_in_place(vloam_b200_ctx* c, LmDevice* d, const LoScalars* lo, 
     VL_TRY(vl_lo_lookahead_solve(c));
     lookaheadDone = true;
   }
-  VL_TRY(lm_pool_headroom(c, 0, 0, nqBound, nqBound));  // (points outside the window are appended raw to their cubes' pool segments: room for them
-                                                        // is checked BEFORE the append is queued, with the bound, against the pool top of the last S2)
-  {
+  // (points outside the window are appended raw to their cubes' pool segments: room for them is checked BEFORE the append is queued,
+  // with the bound, against the pool top of the last S2)
+  if (d->mapUpdate) VL_TRY(lm_pool_headroom(c, 0, 0, nqBound, nqBound));
+  if (!d->mapUpdate) {  // frozen map: no insert, no re-filter, no raw append -- the update's events are recorded behind the pose all the same
+    vl_tls_stream = c->stream3;
+    struct Restore { ~Restore() { vl_tls_stream = nullptr; } } restore;
+    VL_CUDA(cudaStreamWaitEvent(c->stream3, c->evAux, 0));  // (a previous sweep's raw appends: evAux keeps covering them)
+    VL_CUDA(cudaStreamWaitEvent(c->stream3, c->evPose, 0));
+    VL_CUDA(cudaEventRecord(c->evKeys, c->stream3));
+    VL_CUDA(cudaEventRecord(c->evKeysSel[c->stackSel], c->stream3));
+    VL_CUDA(cudaEventRecord(c->evUpd, c->stream3));
+    VL_CUDA(cudaEventRecord(c->evAux, c->stream3));
+    VL_CUDA(cudaEventRecord(c->evMap, c->stream3));
+    if (c->timing) VL_CUDA(cudaEventRecord(c->evx[7], c->stream3));
+  } else {
     const int nq = nqBound;
     const float4* const stackCp = c->stackC.p; const float4* const stackSp = c->stackS.p;
     vl_tls_stream = c->stream3;
@@ -2111,14 +2131,16 @@ static int lm_run_in_place(vloam_b200_ctx* c, LmDevice* d, const LoScalars* lo, 
     d->baseC = d->hMapUpperC; d->baseS = d->hMapUpperS; d->outBaseC = c->h_lmm->outsideC; d->outBaseS = c->h_lmm->outsideS;
   }
   c->lm_optimized = c->h_lmm->optimized;
-  d->gridTopUpper = (long long)c->h_lmm->gridTop + nq;  // chunks in use before this update + at most one new chunk per new voxel
-  // map size after this update <= size at the build + voxels created in the grid + raw appends outside the window (device counts
-  // at this S2: everything up to the previous update) + this sweep's points.  (Adding Qc + Qs per sweep drifts by ~15k points a
-  // sweep -- most of them merge into existing voxels -- and made the next window move regrow the grid and the merge buffers.)
-  d->hMapUpperC = d->baseC + (c->h_lmm->gridCountC - d->builtCountC) + (c->h_lmm->outsideC - d->outBaseC) + Qc;
-  d->hMapUpperS = d->baseS + ((c->h_lmm->gridCount - c->h_lmm->gridCountC) - (d->builtCount - d->builtCountC)) + (c->h_lmm->outsideS - d->outBaseS) + Qs;
-  d->newVoxUpper = (long long)c->h_lmm->gridCount - d->builtCount + nq;  // voxels created so far (device count at S2) + at most nq by this update
-  if (nq > 0) d->poolsStale = true;
+  if (d->mapUpdate) {  // (a frozen map grows no bound)
+    d->gridTopUpper = (long long)c->h_lmm->gridTop + nq;  // chunks in use before this update + at most one new chunk per new voxel
+    // map size after this update <= size at the build + voxels created in the grid + raw appends outside the window (device counts
+    // at this S2: everything up to the previous update) + this sweep's points.  (Adding Qc + Qs per sweep drifts by ~15k points a
+    // sweep -- most of them merge into existing voxels -- and made the next window move regrow the grid and the merge buffers.)
+    d->hMapUpperC = d->baseC + (c->h_lmm->gridCountC - d->builtCountC) + (c->h_lmm->outsideC - d->outBaseC) + Qc;
+    d->hMapUpperS = d->baseS + ((c->h_lmm->gridCount - c->h_lmm->gridCountC) - (d->builtCount - d->builtCountC)) + (c->h_lmm->outsideS - d->outBaseS) + Qs;
+    d->newVoxUpper = (long long)c->h_lmm->gridCount - d->builtCount + nq;  // voxels created so far (device count at S2) + at most nq by this update
+    if (nq > 0) d->poolsStale = true;
+  }
   d->paths[0]++;
   c->lm_frameCount++;
   VL_HOST_MARK(7);
@@ -2133,6 +2155,7 @@ struct LmPoolUpdate {
   long long totalC, totalS;           // points in all cubes before the update
   const float4* stackC; const float4* stackS; int stackSel;
   bool rebuildAfter;                  // rebuild the grid behind the update (in-place path next sweep)
+  bool update;                        // LmDevice::mapUpdate when the sweep was mapped
 };
 
 // ---- map update (LM.cpp:741-808) of the pool path on stream3: the caller reads the pose, and the next frame's scan registration +
@@ -2142,7 +2165,10 @@ static int lm_pool_update(vloam_b200_ctx* c, LmDevice* d, const LmPoolUpdate& u)
   struct Restore { ~Restore() { vl_tls_stream = nullptr; } } restore;
   VL_CUDA(cudaStreamWaitEvent(c->stream3, c->evPose, 0));
   const int nq = u.Qc + u.Qs, nKeys = u.tailTotal + nq;
-  if (nKeys > 0) {
+  if (!u.update) {  // frozen map: no insert, no re-filter, no raw append (the window roll of lm_prepare still cleared what left the grid)
+    VL_CUDA(cudaEventRecord(c->evKeys, c->stream3));
+    VL_CUDA(cudaEventRecord(c->evKeysSel[u.stackSel], c->stream3));
+  } else if (nKeys > 0) {
     VL_TRY(lm_reserve_merge(c, d, nKeys, max(nq, 1), (long long)u.Mc + u.Ms));
     VL_LAUNCH(rf_keys, vl_div_up(nKeys, 256), 256, 0, c->lmm, d->work, c->prm, c->cubeC, c->cubeS, c->poolC.p, c->poolS.p, u.stackC, u.stackS,
               d->newPts.p, d->newCube.p, c->tailKeys.p, nKeys);
@@ -2162,7 +2188,7 @@ static int lm_pool_update(vloam_b200_ctx* c, LmDevice* d, const LmPoolUpdate& u)
   }
   VL_CUDA(cudaEventRecord(c->evAux, c->streamAux));
   // the map after this frame's update holds at most the points it held before plus this frame's inserts
-  d->hMapUpperC = u.totalC + u.Qc; d->hMapUpperS = u.totalS + u.Qs;
+  d->hMapUpperC = u.totalC + (u.update ? u.Qc : 0); d->hMapUpperS = u.totalS + (u.update ? u.Qs : 0);
   // ---- the grid of the NEXT sweep: rebuilt here, behind the update on its side stream, for the window this sweep used (a cube
   // is 50 m wide, so the next sweep almost always uses the same one and runs the in-place path; lm_prepare_fast checks).
   // Debug snapshots keep the pool path every sweep.
@@ -2205,7 +2231,7 @@ static int lm_run_pool(vloam_b200_ctx* c, LmDevice* d, const LoScalars* lo, int 
   VL_TRY(lm_pool_headroom(c, h->totalC, h->totalS, h->Qc, h->Qs));
   c->lm_optimized = h->optimized;
   const LmPoolUpdate u = {h->tailC + h->tailS, h->Qc, h->Qs, h->Mc, h->Ms, h->totalC, h->totalS, c->stackC.p, c->stackS.p, c->stackSel,
-                          d->gridEnabled && !capture};
+                          d->gridEnabled && !capture, d->mapUpdate};
   d->gridValid = false;
   c->lm_frameCount++;
   // otherwise the helper thread issues the update while the caller returns with its pose (whoever needs the map next joins it first: vl_lm_join)
@@ -2314,14 +2340,26 @@ int vl_lm_export_map(vloam_b200_ctx* c, int which, void* out, long cap, long* by
   return VLOAM_OK;
 }
 
+// The map is replaced from outside (a debug import, vloam_b200_load_map): the helper thread has issued the last update and the last
+// publication has finished reading the old map; the grid is rebuilt by the next mapped sweep (pool path), the pools are no longer
+// behind it, and the host bounds restart from the new contents (the caller sets hMapUpper*).
+static int lm_map_replaced(vloam_b200_ctx* c) {
+  LmDevice* d = c->lm;
+  VL_TRY(vl_lm_join(c));
+  VL_TRY(vl_lm_pub_sync(c));
+  d->gridValid = false; d->poolsStale = false;
+  d->newVoxUpper = 0; d->gridTopUpper = 0;
+  return VLOAM_OK;
+}
+
 int vl_lm_import_map(vloam_b200_ctx* c, int which, const void* data, long bytes) {
   LmDevice* d = c->lm;
-  d->gridValid = false;  // the map behind the grid is replaced
   if (bytes < (long)VL_CUBE_NUM * 4) { snprintf(c->err, sizeof c->err, "map blob too short"); return VLOAM_E_INVALID; }
   const int* counts = (const int*)data;
   long long total = 0;
   for (int i = 0; i < VL_CUBE_NUM; ++i) total += counts[i];
   if (bytes != (long)VL_CUBE_NUM * 4 + total * 16) { snprintf(c->err, sizeof c->err, "map blob size mismatch"); return VLOAM_E_INVALID; }
+  VL_TRY(lm_map_replaced(c));
   DBuf<float4>& pool = which ? c->poolS : c->poolC;
   // fresh layout: every cube gets 25 % head room (at least 256 points)
   MapCubeTable h;
@@ -2430,6 +2468,258 @@ int vl_lm_pub_sync(vloam_b200_ctx* c) {
   LmDevice* d = c->lm;
   if (d && d->pubStream) VL_CUDA(cudaStreamSynchronize(d->pubStream));
   return VLOAM_OK;
+}
+
+// ---- vloam_b200_load_map: world-frame clouds -> the cube map -----------------------------------------------------------------------
+// Every point goes to its cube by the insert formula (LM.cpp:747-761, lm_cube_of) at the context's current laserCloudCen*; every
+// non-empty cube is then pcl::VoxelGrid-filtered (LM.cpp:795-808) over its points in input order.  One device-wide sort of the keys
+//   [63:51] cube | [50:21] voxel (lm_vox_key: ascending == pcl's linear voxel index) | [20:0] input index
+// buckets the points by cube, orders each cube by voxel and keeps input order inside a voxel -- the tie order of SURVEY Appendix B --
+// so that a dense cube of ~100k points is sorted by the multi-CTA kernels like any other (no per-segment single-CTA sort).
+#define LD_IDX_BITS 21
+#define LD_CUBE_SHIFT 51
+#define LD_NO_KEY (~0ull)
+#define LD_TILE 256
+#define LD_SCALARS 8  // ldInt[0..7]: {points, pool top} of corner, of surf, dropped corner, dropped surf
+__device__ __forceinline__ unsigned long long ld_run(unsigned long long key) { return key >> LD_IDX_BITS; }  // (cube, voxel)
+__device__ __forceinline__ bool ld_head(const unsigned long long* keys, int i, unsigned long long key) {
+  return key != LD_NO_KEY && (i == 0 || ld_run(keys[i - 1]) != ld_run(key));
+}
+
+// finite check, cube (LM.cpp:747-756) and inside-grid check (LM.cpp:758-761), voxel key; dropped points are counted per kind
+__global__ void __launch_bounds__(256) ld_keys(const float4* __restrict__ in, int n, int P, int kind, const LmScalars* __restrict__ s,
+                                               vloam_b200_params prm, unsigned long long* __restrict__ keys, int* __restrict__ dropped) {
+  VL_PDL_WAIT();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  unsigned long long key = LD_NO_KEY;
+  bool drop = false;
+  if (i < n) {
+    const float4 p = in[i];
+    drop = true;
+    // (|v| < 1e9: the int conversion of lm_cube_of cannot overflow; such a point is outside any window anyway)
+    if (fabsf(p.x) < 1e9f && fabsf(p.y) < 1e9f && fabsf(p.z) < 1e9f) {
+      const int ci = lm_cube_of(p.x, s->cenW), cj = lm_cube_of(p.y, s->cenH), ck = lm_cube_of(p.z, s->cenD);
+      if (ci >= 0 && ci < VL_CUBE_W && cj >= 0 && cj < VL_CUBE_H && ck >= 0 && ck < VL_CUBE_D) {
+        const unsigned vk = lm_vox_key(p, lm_leaf_inv(prm, kind), ci, cj, ck, s->cenW, s->cenH, s->cenD);
+        const int cb = ci + VL_CUBE_W * cj + VL_CUBE_W * VL_CUBE_H * ck;
+        key = ((unsigned long long)cb << LD_CUBE_SHIFT) | ((unsigned long long)vk << LD_IDX_BITS) | (unsigned long long)i;
+        drop = false;
+      }
+    }
+  }
+  if (i < P) keys[i] = key;
+  const unsigned b = __ballot_sync(0xffffffffu, drop);
+  if ((threadIdx.x & 31) == 0 && b) atomicAdd(dropped + kind, __popc(b));
+}
+
+// run heads (one per occupied voxel) per tile of LD_TILE sorted keys, and per cube (the cube table's count, zeroed before)
+__global__ void __launch_bounds__(LD_TILE) ld_heads(const unsigned long long* __restrict__ keys, int P, MapCubeTable* __restrict__ t,
+                                                    int* __restrict__ tileCnt) {
+  VL_PDL_WAIT();
+  __shared__ int ws[LD_TILE / 32];
+  const int i = blockIdx.x * LD_TILE + threadIdx.x;
+  const unsigned long long key = i < P ? keys[i] : LD_NO_KEY;
+  const bool head = ld_head(keys, i, key);
+  const int cb = head ? (int)(key >> LD_CUBE_SHIFT) : -1;
+  const unsigned same = __match_any_sync(0xffffffffu, cb);  // heads of a warp nearly always share their cube: one atomic per cube
+  if (head && (__ffs(same) - 1) == (int)(threadIdx.x & 31)) atomicAdd(&t->count[cb], __popc(same));
+  const unsigned bal = __ballot_sync(0xffffffffu, head);
+  if ((threadIdx.x & 31) == 0) ws[threadIdx.x >> 5] = __popc(bal);
+  __syncthreads();
+  if (threadIdx.x == 0) { int sum = 0; for (int w = 0; w < LD_TILE / 32; ++w) sum += ws[w]; tileCnt[blockIdx.x] = sum; }
+}
+
+// tile offsets (in place), and the pool layout of a fresh import: every cube count + count / 4 + 256 points of room (as
+// vl_lm_import_map), sorted = count; output offset of every cube's first centroid, pool top, totals
+__global__ void __launch_bounds__(1024) ld_layout(int* __restrict__ tileCnt, int nTiles, MapCubeTable* __restrict__ t, int* __restrict__ cubeOff,
+                                                  LmScalars* __restrict__ s, int kind, int* __restrict__ tot) {
+  VL_PDL_WAIT();
+  __shared__ int ws[32];
+  int carry = 0;  // the same value in every thread
+  for (int base = 0; base < nTiles; base += 1024) {
+    const int b = base + threadIdx.x;
+    const int own = b < nTiles ? tileCnt[b] : 0;
+    int sum = 0;
+    const int ex = vl_block_excl_scan<1024>(own, ws, &sum);
+    if (b < nTiles) tileCnt[b] = carry + ex;
+    carry += sum;
+  }
+  constexpr int PER = (VL_CUBE_NUM + 1023) / 1024;
+  const int c0 = threadIdx.x * PER;
+  int cnt[PER], cap[PER], ownN = 0, ownCap = 0;
+#pragma unroll
+  for (int k = 0; k < PER; ++k) {
+    cnt[k] = c0 + k < VL_CUBE_NUM ? t->count[c0 + k] : 0;
+    cap[k] = cnt[k] ? cnt[k] + cnt[k] / 4 + 256 : 0;
+    ownN += cnt[k]; ownCap += cap[k];
+  }
+  int totN = 0, totCap = 0;
+  int runN = vl_block_excl_scan<1024>(ownN, ws, &totN);
+  int runC = vl_block_excl_scan<1024>(ownCap, ws, &totCap);
+#pragma unroll
+  for (int k = 0; k < PER; ++k) {
+    const int cb = c0 + k;
+    if (cb >= VL_CUBE_NUM) continue;
+    cubeOff[cb] = runN; t->start[cb] = cap[k] ? runC : 0; t->cap[cb] = cap[k]; t->sorted[cb] = cnt[k];
+    runN += cnt[k]; runC += cap[k];
+  }
+  if (threadIdx.x == 0) {
+    tot[2 * kind] = totN; tot[2 * kind + 1] = totCap;
+    if (kind) s->poolTopS = totCap; else s->poolTopC = totCap;
+  }
+}
+
+// one thread per run head: the voxel's points in input order, f32 sums, one division (rf_fold / rf_centroid), to its place in the pool
+__global__ void __launch_bounds__(LD_TILE) ld_fold(const float4* __restrict__ in, const unsigned long long* __restrict__ keys, int P,
+                                                   const int* __restrict__ tileOff, const int* __restrict__ cubeOff,
+                                                   const MapCubeTable* __restrict__ t, float4* __restrict__ pool) {
+  VL_PDL_WAIT();
+  __shared__ int ws[LD_TILE / 32];
+  const int i = blockIdx.x * LD_TILE + threadIdx.x;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const unsigned long long key = i < P ? keys[i] : LD_NO_KEY;
+  const bool head = ld_head(keys, i, key);
+  const unsigned bal = __ballot_sync(0xffffffffu, head);
+  if (lane == 0) ws[warp] = __popc(bal);
+  __syncthreads();
+  if (!head) return;
+  int before = 0;
+  for (int w = 0; w < warp; ++w) before += ws[w];
+  const unsigned long long run = ld_run(key);
+  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+  int cnt = 0;
+  for (int q = i; q < P && ld_run(keys[q]) == run; ++q) { acc = rf_fold(acc, in[(int)(keys[q] & ((1ull << LD_IDX_BITS) - 1))]); ++cnt; }
+  const int cb = (int)(key >> LD_CUBE_SHIFT);
+  const int rank = tileOff[blockIdx.x] + before + __popc(bal & ((1u << lane) - 1u));
+  pool[t->start[cb] + rank - cubeOff[cb]] = rf_centroid(acc, cnt);
+}
+
+int vl_lm_load_map(vloam_b200_ctx* c, const float* corner, int nc, const float* surf, int ns, int stride, int w_offset, bool device,
+                   long long dropped[2]) {
+  LmDevice* d = c->lm;
+  if (nc >= (1 << LD_IDX_BITS) || ns >= (1 << LD_IDX_BITS)) {
+    snprintf(c->err, sizeof c->err, "load_map: at most %d points per kind", (1 << LD_IDX_BITS) - 1);
+    return VLOAM_E_CAPACITY;
+  }
+  VL_TRY(lm_map_replaced(c));
+  // the last map update and its raw appends (stream3, streamAux) edit the tables and pools rewritten below
+  VL_CUDA(cudaStreamWaitEvent(c->stream, c->evMap, 0));
+  VL_CUDA(cudaStreamWaitEvent(c->stream, c->evAux, 0));
+  const int n[2] = {nc, ns};
+  int P[2], nTiles[2];
+  for (int k = 0; k < 2; ++k) {
+    P[k] = 0;
+    if (n[k] > 0) { P[k] = 2; while (P[k] < n[k]) P[k] <<= 1; }
+    nTiles[k] = vl_div_up(P[k], LD_TILE);
+    VL_TRY(vl_reserve(c, d->ldIn[k], (size_t)max(n[k], 1)));
+  }
+  VL_TRY(vl_reserve(c, d->ldKeys, (size_t)max(P[0] + P[1], 1)));
+  VL_TRY(vl_reserve(c, d->ldInt, (size_t)LD_SCALARS + 2 * VL_CUBE_NUM + nTiles[0] + nTiles[1]));
+  const VlCloudIn cl[2] = {{corner, nc, d->ldIn[0].p}, {surf, ns, d->ldIn[1].p}};
+  VL_TRY(vl_pack_clouds(c, cl, 2, stride, w_offset, device));
+  int* tot = d->ldInt.p;
+  int* cubeOff[2] = {tot + LD_SCALARS, tot + LD_SCALARS + VL_CUBE_NUM};
+  int* tiles[2] = {tot + LD_SCALARS + 2 * VL_CUBE_NUM, tot + LD_SCALARS + 2 * VL_CUBE_NUM + nTiles[0]};
+  unsigned long long* keys[2] = {d->ldKeys.p, d->ldKeys.p + P[0]};
+  MapCubeTable* tab[2] = {c->cubeC, c->cubeS};
+  VL_CUDA(cudaMemsetAsync(tot, 0, LD_SCALARS * sizeof(int), c->stream));
+  for (int k = 0; k < 2; ++k) {
+    VL_CUDA(cudaMemsetAsync(tab[k], 0, sizeof(MapCubeTable), c->stream));
+    if (n[k] > 0) {
+      VL_BYTES(24.0 * P[k]);
+      VL_LAUNCH(ld_keys, vl_div_up(P[k], 256), 256, 0, (const float4*)d->ldIn[k].p, n[k], P[k], k, (const LmScalars*)c->lmm, c->prm, keys[k], tot + 4);
+      VL_TRY(vl_sort_u64(c, keys[k], P[k]));
+      VL_LAUNCH(ld_heads, nTiles[k], LD_TILE, 0, (const unsigned long long*)keys[k], P[k], tab[k], tiles[k]);
+    }
+    VL_LAUNCH(ld_layout, 1, 1024, 0, tiles[k], nTiles[k], tab[k], cubeOff[k], c->lmm, k, tot);
+  }
+  int h[LD_SCALARS];
+  VL_CUDA(cudaMemcpyAsync(h, tot, sizeof h, cudaMemcpyDeviceToHost, c->stream));
+  VL_CUDA(cudaStreamSynchronize(c->stream));
+  for (int k = 0; k < 2; ++k) {
+    DBuf<float4>& pool = k ? c->poolS : c->poolC;
+    if ((size_t)h[2 * k + 1] * 2 > pool.cap) VL_TRY(vl_reserve(c, pool, (size_t)h[2 * k + 1] * 2));  // (contents are replaced below)
+    if (n[k] > 0) {
+      VL_BYTES(32.0 * P[k]);
+      VL_LAUNCH(ld_fold, nTiles[k], LD_TILE, 0, (const float4*)d->ldIn[k].p, (const unsigned long long*)keys[k], P[k], (const int*)tiles[k],
+                (const int*)cubeOff[k], (const MapCubeTable*)tab[k], pool.p);
+    }
+  }
+  // whatever reads the map next on another stream (a publication, the next update) waits for these
+  VL_CUDA(cudaEventRecord(c->evMap, c->stream));
+  VL_CUDA(cudaEventRecord(c->evAux, c->stream));
+  VL_CUDA(cudaGetLastError());
+  d->hMapUpperC = h[0]; d->hMapUpperS = h[2];
+  c->h_lmm->poolTopC = h[1]; c->h_lmm->poolTopS = h[3];
+  if (dropped) { dropped[0] = h[4]; dropped[1] = h[5]; }
+  return VLOAM_OK;
+}
+
+// vloam_b200_set_map_pose: q_wmap_wodom / t_wmap_wodom (LM.cpp:147-151) on the main stream, behind the last transformUpdate
+struct LmMapPose { double q[4], t[3]; };
+__global__ void lm_set_map_pose(LmScalars* __restrict__ s, LmMapPose p) {
+  VL_PDL_WAIT();
+  for (int k = 0; k < 4; ++k) s->q_wmap_wodom[k] = p.q[k];
+  for (int k = 0; k < 3; ++k) s->t_wmap_wodom[k] = p.t[k];
+}
+int vl_lm_set_map_pose(vloam_b200_ctx* c, const double q[4], const double t[3]) {
+  VL_TRY(vl_lm_join(c));
+  LmMapPose p;
+  memcpy(p.q, q, sizeof p.q); memcpy(p.t, t, sizeof p.t);
+  VL_LAUNCH(lm_set_map_pose, 1, 1, 0, c->lmm, p);
+  VL_CUDA(cudaGetLastError());
+  return VLOAM_OK;
+}
+
+void vl_lm_set_map_update(vloam_b200_ctx* c, bool enabled) { c->lm->mapUpdate = enabled; }
+
+// vloam_b200_get_map_kind: the segments of one kind of the published cloud (pubInt: segment q = 2 cube + kind), in cube order
+__global__ void __launch_bounds__(1024) mp_kind_layout(const int* __restrict__ pub, int kind, int* __restrict__ off) {
+  VL_PDL_WAIT();
+  __shared__ int ws[32];
+  constexpr int PER = (VL_CUBE_NUM + 1023) / 1024;
+  const int c0 = threadIdx.x * PER;
+  int cnt[PER], own = 0;
+#pragma unroll
+  for (int k = 0; k < PER; ++k) {
+    const int q = 2 * (c0 + k) + kind;
+    cnt[k] = c0 + k < VL_CUBE_NUM ? pub[q + 1] - pub[q] : 0;
+    own += cnt[k];
+  }
+  int tot = 0;
+  int run = vl_block_excl_scan<1024>(own, ws, &tot);
+#pragma unroll
+  for (int k = 0; k < PER; ++k) if (c0 + k < VL_CUBE_NUM) { off[c0 + k] = run; run += cnt[k]; }
+  if (threadIdx.x == 0) off[VL_CUBE_NUM] = tot;
+}
+__global__ void __launch_bounds__(256) mp_kind_copy(const int* __restrict__ pub, const int* __restrict__ off, int kind, const float4* __restrict__ cloud,
+                                                    float4* __restrict__ out) {
+  VL_PDL_WAIT();
+  const int total = off[VL_CUBE_NUM];
+  for (int g = blockIdx.x * blockDim.x + threadIdx.x; g < total; g += gridDim.x * blockDim.x) {
+    int lo = 0, hi = VL_CUBE_NUM;
+    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (off[mid] <= g) lo = mid; else hi = mid; }
+    out[g] = cloud[pub[2 * lo + kind] + (g - off[lo])];
+  }
+}
+int vl_lm_get_map_kind(vloam_b200_ctx* c, int which, float* out, int cap_points) {
+  LmDevice* d = c->lm;
+  const int n = vl_lm_get_map(c, nullptr, 0);  // waits for the publication; its errors
+  if (n < 0) return n;
+  VL_TRY(vl_reserve(c, d->pubKindOff, (size_t)VL_CUBE_NUM + 1));
+  VL_LAUNCH(mp_kind_layout, 1, 1024, 0, (const int*)d->pubInt, which, d->pubKindOff.p);
+  int m = 0;
+  VL_CUDA(cudaMemcpyAsync(&m, d->pubKindOff.p + VL_CUBE_NUM, sizeof m, cudaMemcpyDeviceToHost, c->stream));
+  VL_CUDA(cudaStreamSynchronize(c->stream));
+  if (!out || m == 0) return m;
+  if (cap_points < m) { snprintf(c->err, sizeof c->err, "map buffer too small (%d < %d)", cap_points, m); return VLOAM_E_CAPACITY; }
+  VL_TRY(vl_reserve(c, d->pubKind, (size_t)m));
+  VL_BYTES(32.0 * m);
+  VL_LAUNCH(mp_kind_copy, min(vl_div_up(m, 256), c->num_sms * 8), 256, 0, (const int*)d->pubInt, (const int*)d->pubKindOff.p, which,
+            (const float4*)d->pubOut.p, d->pubKind.p);
+  VL_CUDA(cudaMemcpyAsync(out, d->pubKind.p, (size_t)m * 16, cudaMemcpyDeviceToHost, c->stream));
+  VL_CUDA(cudaStreamSynchronize(c->stream));
+  return m;
 }
 
 void vl_lm_paths(vloam_b200_ctx* c, long long out[2]) { const LmDevice* d = c->lm; out[0] = d->paths[0]; out[1] = d->paths[1]; }

@@ -44,6 +44,7 @@
 #include <stdexcept>
 #include <stdlib.h>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include <pcl/point_cloud.h>
@@ -424,6 +425,41 @@ public:
     for (int i = 0; i < n; ++i) { PointType p; p.x = buf[i * 4]; p.y = buf[i * 4 + 1]; p.z = buf[i * 4 + 2]; p.intensity = buf[i * 4 + 3]; out->points[i] = p; }
     return true;
   }
+  // adapter-only: the two kinds of the latest published laserCloudMap (vloam_b200_get_map_kind), in the form loadMap takes back;
+  // false before the first publication
+  bool laserCloudMap(CloudPtr& corner, CloudPtr& surf) {
+    need();
+    if (publishedAt_ == 0) return false;
+    CloudPtr* outs[2] = {&corner, &surf};
+    for (int k = 0; k < 2; ++k) {
+      const int n = vloam_b200_get_map_kind(e_->ctx(), k, nullptr, 0);
+      e_->check(n);
+      std::vector<float> buf((size_t)n * 4);
+      if (n) e_->check(vloam_b200_get_map_kind(e_->ctx(), k, buf.data(), n));
+      CloudPtr& out = *outs[k];
+      if (!out) out = CloudPtr(new pcl::PointCloud<PointType>());
+      out->points.resize(n);
+      for (int i = 0; i < n; ++i) { PointType p; p.x = buf[i * 4]; p.y = buf[i * 4 + 1]; p.z = buf[i * 4 + 2]; p.intensity = buf[i * 4 + 3]; out->points[i] = p; }
+    }
+    return true;
+  }
+  // adapter-only prior maps (no reference counterpart): replace the map with world-frame clouds (PCL memory passed as it is laid
+  // out); returns the points dropped per kind (outside the cube grid or non-finite)
+  std::pair<long long, long long> loadMap(const CloudPtr& corner, const CloudPtr& surf) {
+    need();
+    long long dropped[2] = {0, 0};
+    e_->check(vloam_b200_load_map(e_->ctx(), Engine::points(corner), Engine::count(corner), Engine::points(surf), Engine::count(surf), Engine::kStride,
+                                  Engine::kWOffset, dropped));
+    return std::make_pair(dropped[0], dropped[1]);
+  }
+  // where the sensor starts in a loaded map: q_wmap_wodom / t_wmap_wodom (LM.cpp:147-151), used from the next solveMapping on
+  void setMapPose(const Eigen::Quaterniond& q_wmap_wodom, const Eigen::Vector3d& t_wmap_wodom) {
+    need();
+    const double q[4] = {q_wmap_wodom.x(), q_wmap_wodom.y(), q_wmap_wodom.z(), q_wmap_wodom.w()}, t[3] = {t_wmap_wodom.x(), t_wmap_wodom.y(), t_wmap_wodom.z()};
+    e_->check(vloam_b200_set_map_pose(e_->ctx(), q, t));
+  }
+  // false: localize against the map without changing it (LM.cpp:741-808 skipped); true (default) maps again
+  void setMapUpdate(bool enabled) { need(); e_->check(vloam_b200_set_map_update(e_->ctx(), enabled ? 1 : 0)); }
   int mappedFrames() const { return frameCount; }
   void output() {}                   // declared in LM.h:93, never defined in the reference
   void output(Eigen::Quaterniond& q_w_curr, Eigen::Vector3d& t_w_curr) const {  // adapter-only accessor of the mapped pose
