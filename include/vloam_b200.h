@@ -229,6 +229,60 @@ int vloam_b200_set_map_update(vloam_b200_ctx* c, int enabled);
  * cubes.  Same waits and errors as get_map; VLOAM_E_INVALID for another `which`. */
 int vloam_b200_get_map_kind(vloam_b200_ctx* c, int which, float* out_xyzi, int cap_points);
 
+/* Relocalization: find the sensor in a loaded map without an initial guess -- after a restart inside a saved map, say.  No reference
+ * counterpart.  Call order: load_map, set_map_update(c, 0), one process_frame (its mapped pose is meaningless: the map pose is still the
+ * identity), relocalize with apply = 1, then keep calling process_frame; sweeps registered ahead with prefetch_scan stay valid.
+ *
+ * The search is exact over its discretisation (branch and bound over translation on the device; the scores are integers):
+ *   Query points: the VoxelGrid-filtered stacks of the last mapped sweep (lm.cornerStack then lm.surfStack, in that sweep's sensor
+ *   frame -- its end frame under VLOAM_FLAG_TRANSFORM_TO_END), the ones with (x*x + y*y) + z*z <= max_range^2 (double) in that order,
+ *   every k-th of the n kept with k = ceil(n / max_points), each as u = R_c p in double.  R_c is Eigen's toRotationMatrix of q_c / |q_c|.
+ *   Grid: cells of size r = resolution; N = floor(half_xy / r), Nz = floor(half_z / r); Gx = Gy = 2 (ceil(max_range / r) + N + 1),
+ *   Gz = 2 (ceil(max |u_z| / r) + Nz + 1); origin o = t_c - r (G / 2) (integer G / 2).  A cell is occupied when a point of either
+ *   kind of the map falls in it: floor((m - o) / r) in double.
+ *   Candidates (j, iz, iy, ix), iz in [-Nz, Nz], iy and ix in [-N, N]: R = Rz(theta_j) R_c (roll and pitch of the centre are kept),
+ *   t = t_c + r (ix, iy, iz).  Yaw step d = yaw_step_deg (degrees), or r / max_range radians when it is 0.  half_yaw_deg = 180: j in
+ *   [0, ceil(2 pi / d - 1e-9)), theta_j = j d; otherwise J = floor(half_yaw_deg pi / 180 / d + 1e-9), j in [-J, J].  Linear index
+ *   ((j' nZ + iz') S + iy') S + ix' with every coordinate counted from its lowest value, S = 2N + 1, nZ = 2Nz + 1.
+ *   Score: the number of query points whose cell floor(((c u_x - s u_y) + t_c.x - o_x) / r), ... (c, s = cos, sin theta_j; z:
+ *   floor((u_z + t_c.z - o_z) / r)) moved by (ix, iy, iz) is occupied (outside the grid: not).  best: the highest score, ties to the
+ *   lowest index; runner-up: the same outside {max(|dx|, |dy|) < exclusion_m and |d theta| < exclusion_deg} around best (yaw distance
+ *   taken around the circle when half_yaw_deg = 180).  found: best score >= min_score * n_points.
+ * With apply and found, q/t_wmap_wodom (vloam_b200_set_map_pose's field) is set by transformUpdate (LM.cpp:147-151) from the found pose
+ * and the odometry pose the last mapped sweep was mapped with; the next laser_mapping starts from there (LM.cpp:206-207) and its solve
+ * refines the last half cell and half yaw step.  Nothing else changes: no map edit, no lm.pose write, no window move.
+ * The call drains the context (vloam_b200_synchronize) and blocks until the result is on the host.  Errors: VLOAM_E_INVALID for NULL
+ * pointers, non-finite or negative values, resolution / max_range / max_points <= 0, half_yaw_deg > 180, no mapped sweep since create or
+ * the last load_map (or a skipped sweep last), an empty map and no query point within max_range; VLOAM_E_CAPACITY above 2^31 - 1
+ * candidates or grid cells, or 16383 translation steps per side.  A context that never calls it makes no extra launch, wait or
+ * allocation. */
+typedef struct vloam_b200_reloc_params {
+  double q_c[4], t_c[3];  /* centre pose T_map_sensor (q x,y,z,w): the caller's rough guess; default identity */
+  double half_xy;         /* m, default 20 */
+  double half_z;          /* m, default 1 */
+  double half_yaw_deg;    /* 180 (default) = every heading */
+  double resolution;      /* m: occupancy cell and translation step, default 1 */
+  double yaw_step_deg;    /* 0 (default) = resolution / max_range radians */
+  double max_range;       /* m, default 60 */
+  double min_score;       /* fraction of the query points for `found`, default 0.3 */
+  double exclusion_m;     /* runner-up exclusion zone, default 3 m ... */
+  double exclusion_deg;   /* ... and 10 degrees */
+  int max_points;         /* default 2048 */
+  int apply;              /* default 1: set q/t_wmap_wodom when found */
+} vloam_b200_reloc_params;
+typedef struct vloam_b200_reloc_result {
+  double q[4], t[3];                 /* best pose T_map_sensor */
+  double runner_q[4], runner_t[3];   /* runner-up pose (zeros when every candidate lies in the exclusion zone) */
+  long long index, runner_index;     /* linear candidate indices (-1: no runner-up) */
+  long long candidates;              /* size of the search space */
+  long long nodes;                   /* bounds and scores evaluated by both searches */
+  int score, runner_score;           /* query points on occupied cells (runner_score -1: none) */
+  int n_points;                      /* query points */
+  int found;
+} vloam_b200_reloc_result;
+void vloam_b200_default_reloc_params(vloam_b200_reloc_params* p);
+int vloam_b200_relocalize(vloam_b200_ctx* c, const vloam_b200_reloc_params* p, vloam_b200_reloc_result* result);
+
 /* MAIN.cpp:143-144, 186-190 in one call: begin_frame, scan_registration,
  * laser_odometry, laser_mapping.  pose_out (may be NULL): 14 doubles
  * {odom q[4], odom t[3], mapped q[4], mapped t[3]}.  On a mapped frame the call
@@ -267,6 +321,9 @@ int vloam_b200_profile_timeline(vloam_b200_ctx* c, char* buf, int cap);
  * lm.surfStack lm.cornerFromMap lm.surfFromMap lm.validInd lm.cornerMap
  * lm.surfMap lm.knn.{cidx,sidx,cd2,sd2,cok,sok}{0,1} lm.costs lo.costs
  * lm.paths (int64 {in-place, pool-path} mapped sweeps since create);
+ * of the last relocalize: rl.points (float64 u xyz per query point), rl.occ (float64 origin[3], int64 dims[3], then the level-0
+ * occupancy bytes, x fastest), rl.yaw (float64 cos, sin per yaw), rl.levels (int64 frontier nodes kept per level [2][16], then the
+ * nodes evaluated per pass [2]), rl.ms (float32 device ms {search, occupancy + pyramid});
  * set: lo.last lo.pose lm.pose lm.state lm.cornerMap lm.surfMap. */
 long vloam_b200_debug_get(vloam_b200_ctx* c, const char* name, void* out, long cap_bytes);
 int vloam_b200_debug_set(vloam_b200_ctx* c, const char* name, const void* data, long bytes);

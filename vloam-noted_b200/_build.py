@@ -7,7 +7,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libvloam_b200.so")
 SYNTH_LIB = os.path.join(HERE, "libvloam_synth.so")
-CU_SOURCES = ["scan_registration.cu", "voxel_grid.cu", "laser_odometry.cu", "laser_mapping.cu", "lm_solver.cu", "stage_inputs.cu", "capi.cu"]
+CU_SOURCES = ["scan_registration.cu", "voxel_grid.cu", "laser_odometry.cu", "laser_mapping.cu", "lm_solver.cu", "stage_inputs.cu", "relocalize.cu", "capi.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -21,6 +21,7 @@ EXPORTS = [
     "vloam_b200_laser_odometry_input", "vloam_b200_laser_odometry_input_device", "vloam_b200_laser_mapping_input",
     "vloam_b200_laser_mapping_input_device",
     "vloam_b200_load_map", "vloam_b200_load_map_device", "vloam_b200_set_map_pose", "vloam_b200_set_map_update", "vloam_b200_get_map_kind",
+    "vloam_b200_default_reloc_params", "vloam_b200_relocalize",
 ]
 
 
@@ -28,6 +29,25 @@ class Params(ctypes.Structure):
     """vloam_b200_params: the ROS parameters of the three init() functions."""
     _fields_ = [("n_scans", ctypes.c_int), ("minimum_range", ctypes.c_float), ("line_res", ctypes.c_float),
                 ("plane_res", ctypes.c_float), ("mapping_skip_frame", ctypes.c_int), ("reserved", ctypes.c_int)]
+
+
+class RelocParams(ctypes.Structure):
+    """vloam_b200_reloc_params: the search of vloam_b200_relocalize (include/vloam_b200.h)."""
+    _fields_ = [("q_c", ctypes.c_double * 4), ("t_c", ctypes.c_double * 3)] + [
+        (n, ctypes.c_double) for n in ("half_xy", "half_z", "half_yaw_deg", "resolution", "yaw_step_deg", "max_range", "min_score",
+                                       "exclusion_m", "exclusion_deg")] + [("max_points", ctypes.c_int), ("apply", ctypes.c_int)]
+
+
+class RelocResult(ctypes.Structure):
+    """vloam_b200_reloc_result.  q / t: the best pose T_map_sensor (q x,y,z,w); runner_q / runner_t / runner_score: the best candidate
+    outside the exclusion zone (runner_score -1: none); index / runner_index: linear candidate indices."""
+    _fields_ = [("q", ctypes.c_double * 4), ("t", ctypes.c_double * 3), ("runner_q", ctypes.c_double * 4), ("runner_t", ctypes.c_double * 3),
+                ("index", ctypes.c_longlong), ("runner_index", ctypes.c_longlong), ("candidates", ctypes.c_longlong), ("nodes", ctypes.c_longlong),
+                ("score", ctypes.c_int), ("runner_score", ctypes.c_int), ("n_points", ctypes.c_int), ("found", ctypes.c_int)]
+
+    def __repr__(self):
+        return "RelocResult(found=%d, score=%d/%d, t=%s, runner_score=%d, candidates=%d, nodes=%d)" % (
+            self.found, self.score, self.n_points, np.round(list(self.t), 3), self.runner_score, self.candidates, self.nodes)
 
 
 class VloamError(RuntimeError):
@@ -93,6 +113,8 @@ def load_lib(build=False):
     L.vloam_b200_set_map_pose.argtypes = [vp, vp, vp]
     L.vloam_b200_set_map_update.argtypes = [vp, ci]
     L.vloam_b200_get_map_kind.argtypes = [vp, ci, vp, ci]
+    L.vloam_b200_default_reloc_params.argtypes = [ctypes.POINTER(RelocParams)]
+    L.vloam_b200_relocalize.argtypes = [vp, ctypes.POINTER(RelocParams), ctypes.POINTER(RelocResult)]
     _lib = L
     return L
 
@@ -102,7 +124,16 @@ def _decode(name, raw):
         return raw
     dt = {"sr.curvature": np.float32, "sr.label": np.int32, "sr.scanStartInd": np.int32, "sr.scanEndInd": np.int32,
           "lo.pose": np.float64, "lm.pose": np.float64, "lm.state": np.int32, "lm.validInd": np.int32,
-          "lo.costs": np.float64, "lm.costs": np.float64, "alloc.count": np.int64, "lm.paths": np.int64}
+          "lo.costs": np.float64, "lm.costs": np.float64, "alloc.count": np.int64, "lm.paths": np.int64, "rl.levels": np.int64,
+          "rl.ms": np.float32}
+    if name == "rl.points":
+        return np.frombuffer(raw, np.float64).reshape(-1, 3).copy()
+    if name == "rl.yaw":
+        return np.frombuffer(raw, np.float64).reshape(-1, 2).copy()
+    if name == "rl.occ":  # (origin float64[3], dims int64[3], level-0 occupancy uint8[Gz, Gy, Gx])
+        o = np.frombuffer(raw[:24], np.float64).copy()
+        dims = np.frombuffer(raw[24:48], np.int64).copy()
+        return o, dims, np.frombuffer(raw[48:], np.uint8).reshape(dims[2], dims[1], dims[0]).copy()
     if name in dt:
         return np.frombuffer(raw, dt[name]).copy()
     if name.startswith("lo.assoc.corner"):
@@ -252,6 +283,27 @@ class Context:
     def set_map_update(self, enabled):
         """False: localize against the map without changing it (LM.cpp:741-808 skipped); True (default) resumes mapping."""
         self._chk(self.L.vloam_b200_set_map_update(self.h, 1 if enabled else 0))
+
+    def relocalize(self, q, t, **options):
+        """Find the last mapped sweep in the loaded map around the rough pose (q x,y,z,w; t) without needing it to be close: an exact
+        search over yaw and translation (vloam_b200_relocalize).  options: the fields of vloam_b200_reloc_params (half_xy, half_z,
+        half_yaw_deg, resolution, yaw_step_deg, max_range, min_score, exclusion_m, exclusion_deg, max_points, apply).  With apply
+        (default) and a found pose the next laser_mapping starts from it.  Returns a RelocResult."""
+        p = RelocParams()
+        self.L.vloam_b200_default_reloc_params(ctypes.byref(p))
+        q = np.asarray(q, np.float64)
+        t = np.asarray(t, np.float64)
+        if q.shape != (4,) or t.shape != (3,):
+            raise ValueError("q is 4 doubles (x, y, z, w), t 3")
+        p.q_c[:] = list(q)
+        p.t_c[:] = list(t)
+        for k, v in options.items():
+            if k not in dict(RelocParams._fields_) or k in ("q_c", "t_c"):
+                raise TypeError("unknown relocalize option %r" % k)
+            setattr(p, k, int(v) if k in ("max_points", "apply") else float(v))
+        res = RelocResult()
+        self._chk(self.L.vloam_b200_relocalize(self.h, ctypes.byref(p), ctypes.byref(res)))
+        return res
 
     def laser_odometry(self, prior_q=None, prior_t=None, want_pose=True):
         qw, tw, ql, tl = np.zeros(4), np.zeros(3), np.zeros(4), np.zeros(3)
@@ -500,6 +552,10 @@ class LaserMapping:
 
     def set_map_update(self, enabled):
         self.ctx.set_map_update(enabled)
+
+    def relocalize(self, q, t, **options):
+        """Find the last mapped sweep in the loaded map without an initial guess (Context.relocalize)."""
+        return self.ctx.relocalize(q, t, **options)
 
     def get_map_kind(self, which):
         return self.ctx.get_map_kind(which)

@@ -188,6 +188,7 @@ void vloam_b200_destroy(vloam_b200_ctx* c) {
   if (c->srNext2) { vl_sr_swap(c, *c->srNext2); free_sr_set(c); delete c->srNext2; c->srNext2 = nullptr; }
   cudaStreamDestroy(c->streamSR);
   vl_lm_free(c);
+  vl_rl_free(c);
   if (c->streamLO) { cudaStreamSynchronize(c->streamLO); cudaStreamDestroy(c->streamLO); }
   cudaEventDestroy(c->evS2); cudaEventDestroy(c->evLoSolve); cudaEventDestroy(c->evLoNext); if (c->evEnd) cudaEventDestroy(c->evEnd);
   if (c->evIn) cudaEventDestroy(c->evIn);
@@ -570,6 +571,33 @@ int vloam_b200_get_map_kind(vloam_b200_ctx* c, int which, float* out_xyzi, int c
   return vl_lm_get_map_kind(c, which, out_xyzi, cap_points);
 }
 
+// ---- relocalization --------------------------------------------------------------------------------------------------------------
+void vloam_b200_default_reloc_params(vloam_b200_reloc_params* p) {
+  if (!p) return;
+  memset(p, 0, sizeof *p);
+  p->q_c[3] = 1.0;
+  p->half_xy = 20.0; p->half_z = 1.0; p->half_yaw_deg = 180.0; p->resolution = 1.0; p->yaw_step_deg = 0.0; p->max_range = 60.0;
+  p->min_score = 0.3; p->exclusion_m = 3.0; p->exclusion_deg = 10.0; p->max_points = 2048; p->apply = 1;
+}
+int vloam_b200_relocalize(vloam_b200_ctx* c, const vloam_b200_reloc_params* p, vloam_b200_reloc_result* result) {
+  if (!c) return VLOAM_E_INVALID;  // ABI boundary: a null context is the caller's error, not a crash
+  if (!p || !result) return bad_input(c, "relocalize: params and result must not be NULL");
+  const double* q_c = p->q_c;
+  const double* t_c = p->t_c;
+  for (int k = 0; k < 7; ++k)
+    if (!std::isfinite(k < 4 ? q_c[k] : t_c[k - 4])) return bad_input(c, "relocalize: non-finite centre pose");
+  if (!(q_c[0] * q_c[0] + q_c[1] * q_c[1] + q_c[2] * q_c[2] + q_c[3] * q_c[3] > 0.0)) return bad_input(c, "relocalize: zero quaternion");
+  const double nonneg[] = {p->half_xy, p->half_z, p->half_yaw_deg, p->yaw_step_deg, p->min_score, p->exclusion_m, p->exclusion_deg};
+  for (double v : nonneg)
+    if (!std::isfinite(v) || v < 0.0) return bad_input(c, "relocalize: half-widths, yaw step, min_score and exclusion must be finite and >= 0");
+  if (!std::isfinite(p->resolution) || !(p->resolution > 0.0) || !std::isfinite(p->max_range) || !(p->max_range > 0.0) || p->max_points < 1)
+    return bad_input(c, "relocalize: resolution, max_range and max_points must be finite and > 0");
+  if (p->half_yaw_deg > 180.0) return bad_input(c, "relocalize: half_yaw_deg above 180");
+  memset(result, 0, sizeof *result);
+  VL_TRY(vloam_b200_synchronize(c));  // the last sweep's map update, stacks and look-ahead work are complete
+  return vl_rl_run(c, *p, q_c, t_c, result);
+}
+
 static int process_common(vloam_b200_ctx* c, double* pose_out) {
   VL_HOST_MARK(1);
   c->inProcessFrame = true;
@@ -814,6 +842,7 @@ long vloam_b200_debug_get(vloam_b200_ctx* c, const char* name, void* out, long c
     const int v[4] = {c->h_lmm->gridTop, c->h_lmm->gridCount, c->h_lmm->gridDead, c->h_lmm->gridDirty};
     return put_host(v, sizeof v, out, cap);
   }
+  if (n.rfind("rl.", 0) == 0) return vl_rl_debug(c, name, out, cap);
   if (n == "alloc.count") { const long long v = c->regrows; return put_host(&v, sizeof v, out, cap); }  // device buffer (re)allocations so far
   if (n == "lm.paths") { long long v[2]; vl_lm_paths(c, v); return put_host(v, sizeof v, out, cap); }  // mapped sweeps since create: {in-place, pool path}
   if (n == "lo.costs") return put_host(c->dbgLoCost, sizeof c->dbgLoCost, out, cap);

@@ -248,6 +248,9 @@ struct vloam_b200_ctx {
   bool miPending;                       // a mapping input waits for the next vloam_b200_laser_mapping call of this frame
   bool miUsed;                          // the mapping call of this frame consumed one (register_full_cloud and the pose follow it)
   bool miSkip;                          // its skip_frame
+  // vloam_b200_relocalize (relocalize.cu): its state is created by the first call
+  struct RlState* rl;
+  bool rlReady;                         // the last laser_mapping call mapped a sweep, and no map was loaded since (its stacks are the query)
   // per-kernel timing (vloam_b200_profile_kernel): CUDA events around the launches of one named kernel
   char prof_name[64];                 // kernel to time, or "*" for every launch
   cudaEvent_t prof_ev[VL_PROF_MAX][2];
@@ -445,6 +448,10 @@ int vl_lm_load_map(vloam_b200_ctx* c, const float* corner, int nc, const float* 
 int vl_lm_set_map_pose(vloam_b200_ctx* c, const double q[4], const double t[3]);
 void vl_lm_set_map_update(vloam_b200_ctx* c, bool enabled);
 int vl_lm_get_map_kind(vloam_b200_ctx* c, int which, float* out, int cap_points);
+// relocalization (relocalize.cu): vloam_b200_relocalize on a drained context, its debug getters (rl.*) and its state
+int vl_rl_run(vloam_b200_ctx* c, const vloam_b200_reloc_params& p, const double q_c[4], const double t_c[3], vloam_b200_reloc_result* res);
+long vl_rl_debug(vloam_b200_ctx* c, const char* name, void* out, long cap);
+void vl_rl_free(vloam_b200_ctx* c);
 
 // sort / voxel primitives (voxel_grid.cu)
 int vl_sort_u64(vloam_b200_ctx* c, unsigned long long* d_keys, int n_pow2);
@@ -488,6 +495,17 @@ __device__ __forceinline__ void vl_qmul(const double a[4], const double b[4], do
   const double y = aw * by + ay * bw + az * bx - ax * bz;
   const double z = aw * bz + az * bw + ax * by - ay * bx;
   o[0] = x; o[1] = y; o[2] = z; o[3] = w;
+}
+// transformUpdate (LM.cpp:147-151): q_wmap_wodom = q_w_curr * q_wodom_curr.inverse() (Eigen's conjugate / squaredNorm),
+// t_wmap_wodom = t_w_curr - q_wmap_wodom * t_wodom_curr; pose = {q_w_curr, t_w_curr}
+__device__ __forceinline__ void vl_transform_update(const double pose[7], const double q_wodom[4], const double t_wodom[3], double q_out[4], double t_out[3]) {
+  const double* q = q_wodom;
+  const double n2 = q[0] * q[0] + q[1] * q[1] + q[2] * q[2] + q[3] * q[3];
+  const double qi[4] = {-q[0] / n2, -q[1] / n2, -q[2] / n2, q[3] / n2};
+  vl_qmul(pose, qi, q_out);
+  double r[3];
+  vl_qrot(q_out, t_wodom[0], t_wodom[1], t_wodom[2], r);
+  for (int k = 0; k < 3; ++k) t_out[k] = pose[4 + k] - r[k];
 }
 // Eigen::Quaterniond::Identity().slerp(t, q) (Eigen/src/Geometry/Quaternion.h), used by TransformToStart and the odometry
 // functors when DISTORTION is on (LO.cpp:163, LF.hpp:29-33, 86-90): d = w; |d| >= 1 - eps -> (1 - t) I + t q, else

@@ -776,15 +776,7 @@ __global__ void lm_transform_update(LmScalars* s, const LgHeader* __restrict__ g
   // LM.cpp:147-151
   if (threadIdx.x == 0) {
     if (gh) { s->gridTop = *gridTop; s->gridDirty = gh->dirty; s->gridDead = gh->dead; s->gridCount = gh->count[0] + gh->count[1]; s->gridCountC = gh->count[0]; }
-    if (!s->needSlow) {  // (needSlow: the sweep is repeated on the pool path: leave the state untouched)
-      const double* q = s->q_wodom;
-      const double n2 = q[0] * q[0] + q[1] * q[1] + q[2] * q[2] + q[3] * q[3];
-      const double qi[4] = {-q[0] / n2, -q[1] / n2, -q[2] / n2, q[3] / n2};
-      vl_qmul(s->pose, qi, s->q_wmap_wodom);
-      double r[3];
-      vl_qrot(s->q_wmap_wodom, s->t_wodom[0], s->t_wodom[1], s->t_wodom[2], r);
-      for (int k = 0; k < 3; ++k) s->t_wmap_wodom[k] = s->pose[4 + k] - r[k];
-    }
+    if (!s->needSlow) vl_transform_update(s->pose, s->q_wodom, s->t_wodom, s->q_wmap_wodom, s->t_wmap_wodom);  // (needSlow: the sweep is repeated on the pool path: leave the state untouched)
   }
   if (!hostLmm) return;
   __syncwarp();
@@ -2254,6 +2246,7 @@ int vl_lm_run(vloam_b200_ctx* c, const VlLmInput& in) {
   // (a single CTA that takes 20-60 us when the sensor nears a window edge: it used to sit on the next sweep's pose chain);
   // the pool path waits for them before it reads the cube tables.
   if (in.skip) {  // LM.cpp:197-201: only the high-frequency pose is propagated
+    c->rlReady = false;
     if (in.caller) c->stacksReady = false;  // (stacks this sweep's odometry may have filtered are not used)
     VL_LAUNCH(lm_prepare_fast, 1, 256, 0, c->lmm, in.los, d->work, d->grid.hdr, 1, resetValid, (const int*)nullptr, (const int*)nullptr, (const int*)nullptr);
     VL_TRY(vl_lo_flush_deferred(c)); VL_CUDA(cudaGetLastError());
@@ -2275,6 +2268,7 @@ int vl_lm_run(vloam_b200_ctx* c, const VlLmInput& in) {
   VL_TRY(vl_reserve(c, c->factorValid, (size_t)nqBound));
   const bool inlineUpdate = d->noWorker || capture || c->prof_name[0];  // profiling and debug snapshots serialise everything
   bool fellBack = false;
+  c->rlReady = true;
   if (d->gridEnabled && d->gridValid && !capture && d->gridTopUpper + 2LL * nqBound <= d->grid.cap && d->newVoxUpper + nqBound <= LG_NEWVOX_MAX) {
     VL_TRY(lm_run_in_place(c, d, in.los, nqBound, resetValid, inlineUpdate, &fellBack));
     if (!fellBack) return VLOAM_OK;
@@ -2349,6 +2343,7 @@ static int lm_map_replaced(vloam_b200_ctx* c) {
   VL_TRY(vl_lm_pub_sync(c));
   d->gridValid = false; d->poolsStale = false;
   d->newVoxUpper = 0; d->gridTopUpper = 0;
+  c->rlReady = false;  // (the stacks belong to a sweep mapped in the old map)
   return VLOAM_OK;
 }
 

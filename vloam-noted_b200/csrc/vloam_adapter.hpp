@@ -460,6 +460,28 @@ public:
   }
   // false: localize against the map without changing it (LM.cpp:741-808 skipped); true (default) maps again
   void setMapUpdate(bool enabled) { need(); e_->check(vloam_b200_set_map_update(e_->ctx(), enabled ? 1 : 0)); }
+  // adapter-only relocalization (vloam_b200_relocalize): find the last mapped sweep in the loaded map around the rough pose
+  // T_map_sensor = (q_c, t_c) without needing it to be close; with options.apply and a found pose the next solveMapping starts there
+  struct RelocOptions {
+    double half_xy = 20.0, half_z = 1.0, half_yaw_deg = 180.0, resolution = 1.0, yaw_step_deg = 0.0, max_range = 60.0, min_score = 0.3;
+    double exclusion_m = 3.0, exclusion_deg = 10.0;
+    int max_points = 2048;
+    bool apply = true;
+  };
+  vloam_b200_reloc_result relocalize(const Eigen::Quaterniond& q_c, const Eigen::Vector3d& t_c) { return relocalize(q_c, t_c, RelocOptions()); }
+  vloam_b200_reloc_result relocalize(const Eigen::Quaterniond& q_c, const Eigen::Vector3d& t_c, const RelocOptions& o) {
+    need();
+    vloam_b200_reloc_params p;
+    vloam_b200_default_reloc_params(&p);
+    p.q_c[0] = q_c.x(); p.q_c[1] = q_c.y(); p.q_c[2] = q_c.z(); p.q_c[3] = q_c.w();
+    p.t_c[0] = t_c.x(); p.t_c[1] = t_c.y(); p.t_c[2] = t_c.z();
+    p.half_xy = o.half_xy; p.half_z = o.half_z; p.half_yaw_deg = o.half_yaw_deg; p.resolution = o.resolution; p.yaw_step_deg = o.yaw_step_deg;
+    p.max_range = o.max_range; p.min_score = o.min_score; p.exclusion_m = o.exclusion_m; p.exclusion_deg = o.exclusion_deg;
+    p.max_points = o.max_points; p.apply = o.apply ? 1 : 0;
+    vloam_b200_reloc_result r;
+    e_->check(vloam_b200_relocalize(e_->ctx(), &p, &r));
+    return r;
+  }
   int mappedFrames() const { return frameCount; }
   void output() {}                   // declared in LM.h:93, never defined in the reference
   void output(Eigen::Quaterniond& q_w_curr, Eigen::Vector3d& t_w_curr) const {  // adapter-only accessor of the mapped pose
